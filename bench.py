@@ -16,6 +16,13 @@ resident in HBM; `e2e` times the same call sequence with HOST (pinned) buffers: 
 the transfer of the matrix into host memory are inside the timed region. The CPU baseline / reference arm run the
 UNMODIFIED reference compiled into oracle/_ref (or, if that .so is absent, the oracle port) on a bounded sample of the
 same workload, and the GPU path is checked against that very run (`parity_vs_reference`).
+
+--steps K sets the number of timed steps of the headline (device-resident), end-to-end, whole-genome and reference
+regions. The side measurements reported next to them have fixed counts: the tensor kernel alone (2 steps), the eigen-solver
+(3 runs), EM (one call) and the C++ shim driver (2 steps). --dump-outputs DIR writes, after the timed steps, the
+similarity matrix the timed path computed in its last step as DIR/*.npy (float64; a fixed sample of its rows when the
+whole matrix exceeds 32 MB). The inputs are generated from fixed seeds, so two builds run with the same arguments can be
+compared output for output. The bench writes nothing into the source tree (which may be read-only).
 """
 from __future__ import annotations
 
@@ -32,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree
 
 # ---- workload: BASELINE.json configs[2] (headline) ---------------------------------------------------------------
 WORKLOAD = dict(
@@ -199,6 +207,37 @@ def reference_threads():
         return max(1, os.cpu_count() or 1)
 
 
+DUMP_MATRIX_BYTES = 32 << 20
+
+
+def dump_matrix(out_dir, M):
+    """The N x N similarity matrix as DIR/similarity_matrix_rows.npy (float64): all of its rows when they fit in
+    DUMP_MATRIX_BYTES, else a sample of rows drawn with a fixed seed (the same rows for the same N), whose indices are
+    DIR/similarity_matrix_row_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = M.shape[0]
+    k = min(n, max(1, DUMP_MATRIX_BYTES // (8 * n)))
+    rows = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    np.save(os.path.join(out_dir, "similarity_matrix_rows.npy"), np.ascontiguousarray(M[rows], dtype=np.float64))
+    np.save(os.path.join(out_dir, "similarity_matrix_row_index.npy"), rows.astype(np.float64))
+
+
+def host_matrix(rig, counts, epi, lik, normalization):
+    """The matrix of the planes in `counts`: the epilogue the timed steps ran on them, once more, into host memory.
+    Rank 0 gets it, the other ranks None."""
+    if rig.world == 1:
+        return counts.finalize(*lik, normalization)
+    from secedo_b200 import dist as sdist
+    shared = sdist.SharedHostMatrix(rig.ctx, counts.num_cells)
+    epi.run(*lik, normalization, out_ptr=shared.dev_ptr, same_stream=True)
+    rig.ctx.synchronize()
+    rig.barrier()
+    M = shared.array.copy() if rig.rank == 0 else None
+    rig.barrier()
+    shared.close()
+    return M
+
+
 def metric_name():
     w = WORKLOAD
     return "similarity-matrix significant loci/s (%dK cells, %gx)" % (w["n_cells"] // 1000, w["coverage"])
@@ -217,9 +256,13 @@ def main_reference(args):
     p = cpu_sample()
     times, loci, kind = [], 0, "reference"
     for i in range(args.warmup + args.steps):
-        s, loci, kind = run_reference_step(p, threads)
+        last = i == args.warmup + args.steps - 1
+        r = run_reference_step(p, threads, want_matrix=bool(args.dump_outputs) and last)
+        s, loci, kind = r[:3]
         if i >= args.warmup:
             times.append(s)
+    if args.dump_outputs:
+        dump_matrix(args.dump_outputs, r[3])
     total = sum(times)
     value = loci * len(times) / total
     sample = (f"{CPU_SAMPLE_LOCI} pre-filter loci ({loci} significant, {p.n_entries} pileup entries) of the workload per "
@@ -359,6 +402,15 @@ class Rig:
 PHASES = ("ms_link", "ms_first_order", "ms_stage", "ms_gemm", "ms_multi", "gemm_launches")
 
 
+def synth_sub_batch(ctx, rank, b):
+    """sub-batch b of rank `rank` of the workload, generated in HBM from its own seed"""
+    w = WORKLOAD
+    return ctx.synth_pileup(w["n_cells"], w["coverage"], w["n_chr"], w["loci_per_chr"], n_clones=w["n_clones"],
+                            frac_somatic=w["frac_somatic"], frac_germline=w["frac_germline"], theta=w["theta"],
+                            spacing=w["spacing"], p_multi=w["p_multi"], p_mate=w["p_mate"],
+                            p_mate_mismatch=w["p_mate_mismatch"], seed=1000 + 64 * rank + b)
+
+
 def main_ours(args):
     from secedo_b200 import dist as sdist
     from secedo_b200.pileup import Pileup
@@ -371,14 +423,7 @@ def main_ours(args):
     threads = reference_threads()  # the num_threads of BOTH arms (selects the reference's tail cutoff)
     ident = np.arange(N, dtype=np.uint32)
     lik = (w["L"], w["eps"], w["h"], w["theta"])
-
-    def synth(seed):
-        return ctx.synth_pileup(N, w["coverage"], w["n_chr"], w["loci_per_chr"], n_clones=w["n_clones"],
-                                frac_somatic=w["frac_somatic"], frac_germline=w["frac_germline"], theta=w["theta"],
-                                spacing=w["spacing"], p_multi=w["p_multi"], p_mate=w["p_mate"],
-                                p_mate_mismatch=w["p_mate_mismatch"], seed=seed)
-
-    raw_dev = [synth(1000 + 64 * rank + b) for b in range(SUB)]
+    raw_dev = [synth_sub_batch(ctx, rank, b) for b in range(SUB)]
     dims = [r.dims() for r in raw_dev]
     n_chr = dims[0][0]
     P, E = sum(d[1] for d in dims), sum(d[2] for d in dims)
@@ -490,6 +535,12 @@ def main_ours(args):
     # ---- device-resident input ------------------------------------------------------------------------
     l2_0 = ctx2.launch_count() if ctx2 else 0
     ms_dev, acc, launches, clocks = rig.timed(step_resident, args.steps, args.warmup, finish=finish_prev)
+    if args.dump_outputs:  # now: the steps below overwrite the planes of the last timed step
+        k = (pipe["i"] - 1) % len(counts_ab)
+        M = host_matrix(rig, counts_ab[k], epi_ab[k], lik, w["normalization"])
+        if rank == 0:
+            dump_matrix(args.dump_outputs, M)
+        del M
     if ctx2:  # warm-up launches of the second context are not part of the timed region
         launches += (ctx2.launch_count() - l2_0) * args.steps // (args.steps + args.warmup)
     sig_local = acc["sig_loci"] // args.steps
@@ -566,7 +617,7 @@ def main_ours(args):
     if world == 1:
         # second result buffer: the matrix of step s travels to the host (own stream) while step s + 1 is computed
         out_bufs = [torch.empty((N, N), dtype=torch.float64).pin_memory().numpy() for _ in range(2)]
-    e2e_steps = max(1, min(args.steps, int(os.environ.get("SECEDO_BENCH_E2E_STEPS", 10))))
+    e2e_steps = args.steps
     E2E_WARMUP = 2
     # uploads run up to LOOKAHEAD chromosomes ahead of the kernels, but never across the warm-up / timed boundary nor past
     # the last step: every timed step's H2D bytes are copied inside the timed region
@@ -730,11 +781,16 @@ def main_ours(args):
         if not args.skip_extras and world == 1:
             try:
                 import subprocess
+                import tempfile
                 import __graft_entry__ as ge
-                exe = ge.build_shim_bench()
-                env = dict(os.environ, SECEDO_B200_DEVICES=str(rig.local_rank))
-                r = subprocess.run([exe, str(N), str(w["coverage"]), "4", str(int(os.environ.get("SECEDO_BENCH_SHIM_LOCI", 8192))),
-                                    str(threads), "2"], capture_output=True, text=True, timeout=600, env=env)
+                with tempfile.TemporaryDirectory() as tmp:
+                    # the driver build() left next to the library if it is fresh, else one compiled outside the tree
+                    # (which may be read-only)
+                    exe = ge.build_shim_bench(tmp)
+                    env = dict(os.environ, SECEDO_B200_DEVICES=str(rig.local_rank))
+                    r = subprocess.run([exe, str(N), str(w["coverage"]), "4",
+                                        str(int(os.environ.get("SECEDO_BENCH_SHIM_LOCI", 8192))), str(threads), "2"],
+                                       capture_output=True, text=True, timeout=600, env=env)
                 e2e_shim = json.loads(r.stdout.strip().splitlines()[-1]) if r.returncode == 0 else {"error": (r.stderr or r.stdout)[-300:]}
             except Exception as ex:  # noqa: BLE001
                 e2e_shim = {"error": str(ex)[-300:]}
@@ -916,13 +972,13 @@ def main_genome(args):
         finish(st)
         return st
 
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, args.warmup
     if resident:
         ms, acc, launches, clocks = rig.timed(genome_resident, steps, warmup)
         how = "whole share resident in HBM; barrier + events around the whole genome, max over ranks"
     else:
-        # one pass (after a one-call warm-up): every batch of segments is generated, then timed on its own
-        steps, warmup = 1, 0
+        # `steps` passes (after a one-call warm-up): every batch of segments is generated, then timed on its own
+        warmup = 0
         st = {"sig_loci": 0, "ms_gemm": 0.0, "gemm_launches": 0}
         parts = generate(calls[0])
         counts.zero()
@@ -935,34 +991,41 @@ def main_genome(args):
             th.start()
         rig.barrier()
         launches0 = ctx.launch_count()
-        counts.zero()
-        ms_local = 0.0
-        for call in calls:
-            parts = generate(call)
-            torch.cuda.synchronize()
+        ms = 0.0
+        for _ in range(steps):
+            counts.zero()
+            ms_local = 0.0
+            for call in calls:
+                parts = generate(call)
+                torch.cuda.synchronize()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record(stream)
+                accumulate_call(call, parts, st)
+                # this batch's tensor kernel (on its own stream) belongs to this batch's timed region: wait for it, so that
+                # it does not run hidden under the untimed generation of the next batch
+                ms_left, n_left = ctx.tensor_times()
+                st["ms_gemm"] += ms_left
+                st["gemm_launches"] += n_left
+                e1.record(stream)
+                e1.synchronize()
+                ms_local += e0.elapsed_time(e1)
+                parts.free()
+            rig.barrier()  # the slowest rank's accumulation ends here
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(stream)
-            accumulate_call(call, parts, st)
-            # this batch's tensor kernel (on its own stream) belongs to this batch's timed region: wait for it, so that it
-            # does not run hidden under the untimed generation of the next batch
-            ms_left, n_left = ctx.tensor_times()
-            st["ms_gemm"] += ms_left
-            st["gemm_launches"] += n_left
+            finish(st)
             e1.record(stream)
-            e1.synchronize()
-            ms_local += e0.elapsed_time(e1)
-            parts.free()
-        rig.barrier()  # the slowest rank's accumulation ends here
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream)
-        finish(st)
-        e1.record(stream)
-        torch.cuda.synchronize()
-        ms = rig.max_over_ranks(ms_local) + rig.max_over_ranks(e0.elapsed_time(e1))
+            torch.cuda.synchronize()
+            ms += rig.max_over_ranks(ms_local) + rig.max_over_ranks(e0.elapsed_time(e1))
         stop.set()
         acc, launches, clocks = st, ctx.launch_count() - launches0, summarize_clocks(lines)
         how = ("share larger than HBM: every batch of 4 segments generated in front of its own timed region; time = max over "
-               "ranks of the summed per-batch device times + the epilogue")
+               "ranks of the summed per-batch device times + the epilogue, summed over the steps")
+    if args.dump_outputs:
+        M = host_matrix(rig, counts, epi, lik, w["normalization"])
+        if rank == 0:
+            dump_matrix(args.dump_outputs, M)
+        del M
     sig_local = acc["sig_loci"] // steps
     sig_total = rig.sum_over_ranks(sig_local)
     ok = None
@@ -1007,7 +1070,10 @@ if __name__ == "__main__":
     ap.add_argument("--path", default="auto", choices=["auto", "scatter", "gemm"])
     ap.add_argument("--workload", default="cfg3", choices=["cfg3", "cfg3-genome", "cfg5"])
     ap.add_argument("--skip-extras", action="store_true", help="skip the spectral / EM side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the similarity matrix of the last timed step to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     select_workload(a.workload)
     if a.workload == "cfg5":
         a.skip_extras = True  # the eigen-solver / EM side measurements belong to the headline workload
