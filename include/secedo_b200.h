@@ -110,11 +110,11 @@ uint64_t sgpu_launch_count(const sgpu_ctx *ctx);
 int sgpu_tensor_times(sgpu_ctx *ctx, float *ms, uint64_t *launches);
 /* Scheduling knobs of a context (their defaults come from the environment variables of the same meaning, read by sgpu_init;
  * the results never depend on them). Waits for the context's work first. Names:
- *   "async_gemm"     1: the first-order tensor kernel runs on its own stream beside the next batch (SECEDO_B200_ASYNC_GEMM)
- *   "late_gemm"      1: ... and is issued behind the next batch's dense read-linking kernel (SECEDO_B200_GEMM_LATE)
- *   "gemm_stages"    4, 5, 6: operand ring of the tensor kernel (SECEDO_B200_GEMM_STAGES)
- *   "prefer_shared"  0 never, 1 always, 2 around the co-run window: device-wide cudaFuncCachePreferShared (SECEDO_B200_PREFER_SHARED)
- *   "win_smem_kb"    shared memory a read-linking CTA may use, 0 = all (SECEDO_B200_WIN_SMEM_KB) */
+ *   "async_gemm"     1: the first-order tensor kernel runs on its own stream beside the next batch and is issued behind the
+ *                    next batch's dense read-linking kernel (SECEDO_B200_ASYNC_GEMM)
+ *   "prefer_shared"  1: device-wide cudaFuncCachePreferShared around the window in which kernels run beside a deferred
+ *                    tensor kernel, 0: never switched; other values fail with SGPU_E_ARG (SECEDO_B200_PREFER_SHARED;
+ *                    default: on when async_gemm is on at sgpu_init) */
 int sgpu_set_option(sgpu_ctx *ctx, const char *name, int value);
 
 /* ---- pileup staging (replaces the host vector<vector<PosData>>) --------------------------- */

@@ -1,6 +1,6 @@
 """One device-resident hot-path step of the bench workload per iteration (filter -> accumulate -> finalize), nothing else:
 the command that the ncu captures of the hot-path kernels wrap.   python profiles/hot_step.py [iterations]
-Env knobs of the library (SECEDO_B200_TILE_BAND, SECEDO_B200_L2_PROMO, ...) apply."""
+Env knobs of the library (SECEDO_B200_ASYNC_GEMM, SECEDO_B200_PREFER_SHARED, ...) apply."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

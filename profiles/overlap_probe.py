@@ -1,6 +1,6 @@
 """Device-resident hot-path steps of the bench workload (4 sub-batches -> one matrix per step), nothing else: A/B probe for
-the library's env knobs that are read at context creation (SECEDO_B200_ASYNC_GEMM, SECEDO_B200_GEMM_STAGES,
-SECEDO_B200_WIN_SMEM_KB, ...).   python profiles/overlap_probe.py [steps] [warmup] [label]
+the library's env knobs that are read at context creation (SECEDO_B200_ASYNC_GEMM, SECEDO_B200_PREFER_SHARED,
+...).   python profiles/overlap_probe.py [steps] [warmup] [label]
 Prints one JSON line: ms per step (host clock around synchronised regions), per-phase device times, tensor kernel average,
 and a checksum of the count planes of the last step (must not depend on the knobs)."""
 import json, os, sys, time

@@ -64,8 +64,8 @@ class Context:
         return int(self._lib.sgpu_launch_count(self._h))
 
     def set_option(self, name: str, value: int) -> None:
-        """Scheduling knobs (``async_gemm``, ``late_gemm``, ``gemm_stages``, ``prefer_shared``, ``win_smem_kb``): see
-        ``sgpu_set_option`` in include/secedo_b200.h. Results never depend on them."""
+        """Scheduling knobs (``async_gemm`` 0 / 1, ``prefer_shared`` 0 / 1): see ``sgpu_set_option`` in
+        include/secedo_b200.h. Results never depend on them."""
         self.check(self._lib.sgpu_set_option(self._h, name.encode(), int(value)))
 
     def tensor_times(self):

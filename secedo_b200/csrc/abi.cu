@@ -321,24 +321,10 @@ int sgpu_init(int device, sgpu_ctx **out) {
         SGPU_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->tensor_stream, cudaStreamNonBlocking, greatest));
         const char *as = getenv("SECEDO_B200_ASYNC_GEMM");
         ctx->async_gemm = !(as && as[0] == '0');
-        const char *lg = getenv("SECEDO_B200_GEMM_LATE");
-        ctx->late_gemm = !(lg && lg[0] == '0');
-        const char *fp = getenv("SECEDO_B200_GEMM_FLUSH_AT");
-        ctx->flush_point = fp ? std::min(2, std::max(0, atoi(fp))) : 0;
         // kernels only run beside the tensor kernel while the device-wide cache preference is PreferShared (sgpu_ctx::prefer_shared,
-        // profiles/coresidency_probe.cu): 2 = switched on and off around the window in which that can happen
+        // profiles/coresidency_probe.cu): switched on and off around the window in which that can happen
         const char *ps = getenv("SECEDO_B200_PREFER_SHARED");
-        ctx->prefer_shared = ps ? atoi(ps) : (ctx->async_gemm ? 2 : 0);
-        if (ctx->prefer_shared == 1) {
-            SGPU_TRY(sgpu_cache_preference(ctx, true));
-        }
-        // operand ring of the CTA-pair kernel: 6 stages fill the SM; 5 leave 64 KB per SM to the kernels beside it
-        const char *gs = getenv("SECEDO_B200_GEMM_STAGES");
-        ctx->gemm_stages = gs ? static_cast<uint32_t>(std::min(6, std::max(4, atoi(gs)))) : (ctx->async_gemm ? 5u : 6u);
-        const char *ws = getenv("SECEDO_B200_WIN_SMEM_KB");
-        // read linking: a geometry that fits beside the tensor kernel (60 KB: one CTA per SM, a denser table) was slower than
-        // letting link_window wait for the whole SM (profiles/r2_overlap_probes.txt), so no limit by default
-        ctx->win_smem_limit = ws ? static_cast<uint32_t>(std::max(16, atoi(ws))) * 1024u : 0u;
+        ctx->prefer_shared = ps ? ps[0] != '0' : ctx->async_gemm;
     }
     return SGPU_OK;
 }
@@ -430,7 +416,7 @@ int sgpu_synchronize(sgpu_ctx *ctx) {
 } // extern "C"
 
 int sgpu_cache_preference(sgpu_ctx *ctx, bool shared) {
-    if (ctx->prefer_shared == 0 || (ctx->prefer_shared == 1 && !shared) || ctx->cache_pref_now == (shared ? 1 : 0)) {
+    if (!ctx->prefer_shared || ctx->cache_pref_now == (shared ? 1 : 0)) {
         return SGPU_OK;
     }
     SGPU_CUDA(ctx, cudaDeviceSetCacheConfig(shared ? cudaFuncCachePreferShared : cudaFuncCachePreferNone));
@@ -463,27 +449,15 @@ int sgpu_set_option(sgpu_ctx *ctx, const char *name, int value) {
     const std::string n(name);
     if (n == "async_gemm") {
         ctx->async_gemm = value != 0;
-    } else if (n == "late_gemm") {
-        ctx->late_gemm = value != 0;
-    } else if (n == "gemm_stages") {
-        if (value < 4 || value > 6) {
-            return sgpu_fail(ctx, SGPU_E_ARG, "gemm_stages must be 4, 5 or 6");
-        }
-        ctx->gemm_stages = static_cast<uint32_t>(value);
     } else if (n == "prefer_shared") {
-        if (value < 0 || value > 2) {
-            return sgpu_fail(ctx, SGPU_E_ARG, "prefer_shared must be 0, 1 or 2");
+        if (value != 0 && value != 1) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "prefer_shared must be 0 or 1");
         }
         if (ctx->cache_pref_now == 1) { // back to the default split before the mode changes
             SGPU_CUDA(ctx, cudaDeviceSetCacheConfig(cudaFuncCachePreferNone));
             ctx->cache_pref_now = 0;
         }
-        ctx->prefer_shared = value;
-        if (value == 1) {
-            SGPU_TRY(sgpu_cache_preference(ctx, true));
-        }
-    } else if (n == "win_smem_kb") {
-        ctx->win_smem_limit = value > 0 ? static_cast<uint32_t>(std::max(16, value)) * 1024u : 0u;
+        ctx->prefer_shared = value == 1;
     } else {
         return sgpu_fail(ctx, SGPU_E_ARG, "sgpu_set_option: unknown option '%s'", name);
     }

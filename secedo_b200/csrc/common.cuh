@@ -52,24 +52,20 @@ struct sgpu_ctx {
         cudaEvent_t t0 = nullptr, t1 = nullptr; // around the kernel, on the stream it was launched on
     };
     std::deque<TensorJob> tensor_jobs;
-    void *pending_gemm = nullptr;        // gemm.cu: prepared launch of the last deferred tensor kernel, not issued yet
-    bool late_gemm = true;               // issue it behind the next batch's link_window kernel (SECEDO_B200_GEMM_LATE=0: at once)
-    int flush_point = 0;                 // where exactly (SECEDO_B200_GEMM_FLUSH_AT): 0 behind link_window, 1 behind the
-                                         // special-entry chain, 2 behind the partition kernel
+    void *pending_gemm = nullptr;        // gemm.cu: prepared launch of the last deferred tensor kernel, issued behind the next
+                                         // batch's link_window kernel (sgpu_tensor_flush)
     std::vector<cudaEvent_t> event_pool; // recycled timing events
     // Kernels only share an SM with the tensor kernel while the DEVICE-WIDE cache preference is cudaFuncCachePreferShared: a
     // kernel with 16 KB of static shared memory otherwise waited for the whole tensor kernel, and neither the carve-out
     // attribute nor cudaFuncSetCacheConfig of that kernel changed it (profiles/coresidency_probe.cu, r2_coresidency.txt,
-    // r2_overlap_probes.txt). The preference costs the kernels that run alone ~4 % (less L1), so by default (2) it is only
-    // in force from the launch of a deferred tensor kernel to the launch of the next batch's link_window kernel (which
-    // never fits beside it). 0: never, 1: always, 2: toggled.
-    int prefer_shared = 0;
+    // r2_overlap_probes.txt). The preference costs the kernels that run alone ~4 % (less L1), so it is only in force from
+    // the launch of a deferred tensor kernel to the launch of the next batch's link_window kernel (which never fits beside
+    // it). false: never switched (the host application keeps its own preference).
+    bool prefer_shared = false;
     int cache_pref_now = -1;             // what this context last set (-1: nothing yet)
-    uint32_t gemm_stages = 6;            // operand ring of syrk2_kernel (SECEDO_B200_GEMM_STAGES = 4, 5, 6)
-    uint32_t win_smem_limit = 0;         // reads.cu: shared memory a link_window CTA may use (0 = default)
     // gemm.cu: rasterised list of upper-triangle output tiles for tile_cache_cells cells (device memory)
     void *tile_cache = nullptr;
-    uint32_t tile_cache_n = 0, tile_cache_cells = 0, tile_cache_bm = 0;
+    uint32_t tile_cache_n = 0, tile_cache_cells = 0;
     // epilogue.cu: F / G coefficients of the last likelihood parameters, tile list of the last matrix size
     bool ft_valid = false;
     double ft_eps = 0, ft_h = 0, ft_theta = 0, ft_f10 = 0, ft_f01 = 0, ft_g2[3] = { 0, 0, 0 }, ft_g3[4] = { 0, 0, 0, 0 };

@@ -14,15 +14,13 @@
 //   stage_tile_kernel    per (k-block of 32 loci, stripe): base counts in a shared-memory tile -> Hadamard planes,
 //                        written as finished K-major operand rows U[chunk][cell][k-block][plane][32 loci]
 //                        (one 128-byte row per cell and k-block); tail k-blocks hold Z and -Z (S = C C^T - Z Z^T)
-//   syrk2_kernel<stages> persistent CTA pairs (cluster of 2, tcgen05 cta_group::2, 256 x 256 tiles): warp 0 of both
-//                        CTAs = TMA producer (cp.async.bulk.tensor.3d, 128B swizzle, mbarrier ring of 4 / 5 / 6
-//                        stages), warp 1 of the leader = tcgen05.mma.kind::i8 issuer (M=256, N=256, K=32;
+//   syrk2_kernel         persistent CTA pairs (cluster of 2, tcgen05 cta_group::2, 256 x 256 tiles): warp 0 of both
+//                        CTAs = TMA producer (cp.async.bulk.tensor.3d, 128B swizzle, mbarrier ring of 5 stages),
+//                        warp 1 of the leader = tcgen05.mma.kind::i8 issuer (M=256, N=256, K=32;
 //                        accumulators Q = 4S - T and T in TMEM, 2 x 256 columns per CTA), warps 2-5 = epilogue
 //                        (tcgen05.ld, S = (Q+T)/4, D = T - S, vector stores / load-add-store into the int32 planes,
 //                        RED.ADD for edge and split tiles, upper triangle only); the pairs start the n-th tile
 //                        together (wave counter) so that a wave shares its operand slabs through L2
-//   syrk_kernel          the same on single CTAs (128 x 256 tiles, 4 stages): devices with an odd SM count,
-//                        SECEDO_B200_GEMM_PAIRS=0
 // Only output tiles that intersect the upper triangle are computed; the K range of a panel is split across CTAs for
 // the tiles that do not fill a whole round of the grid.
 //
@@ -40,21 +38,13 @@
 
 namespace {
 
-constexpr int BM = 128;            // rows (cells) of an output tile = UMMA M
+constexpr int BM = 128;            // rows (cells) of an output tile held by one CTA of a pair
 constexpr int BN = 256;            // columns (cells) of an output tile = UMMA N
 constexpr int KB_BYTES = 128;      // bytes of K per stage and row: 32 loci x 4 planes
 constexpr int LOCI_PER_KB = 32;
-constexpr int STAGES = 4;
 constexpr int A_BYTES = BM * KB_BYTES;  // 16 KB
-constexpr int B_BYTES = BN * KB_BYTES;  // 32 KB
-constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */;
 constexpr int GEMM_THREADS = 192;  // 6 warps
 constexpr uint32_t TMEM_COLS = 512;
-#ifndef SGPU_PREFETCH_KB
-#define SGPU_PREFETCH_KB 0
-#endif
-constexpr uint32_t PREFETCH_KB = SGPU_PREFETCH_KB; // k-blocks an L2 prefetch runs ahead of the TMA loads; 0 = off (measured: 12 ahead doubles the kernel time, the TMA unit serialises the prefetches with the loads)
 
 // Panel layout. One 128-byte row per (cell, k-block of 32 loci). The rows of CK consecutive k-blocks
 // form a chunk [chunk][cell][k-block in chunk]: the ~1 200 loci that are staged concurrently then touch
@@ -526,12 +516,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void *p) { return static_cast
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     asm volatile(
             "{\n\t"
@@ -544,17 +528,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
             "}" ::"r"(bar),
             "r"(parity)
             : "memory");
-}
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int32_t c0, int32_t c1, int32_t c2) {
-    asm volatile(
-            "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-            "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-            : "memory");
-}
-// bring a box into L2 without touching shared memory (hides DRAM latency the 4-stage ring cannot cover)
-__device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap *map, int32_t c0, int32_t c1, int32_t c2) {
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(map), "r"(c0), "r"(c1), "r"(c2)
-                 : "memory");
 }
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
@@ -577,22 +550,6 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
     d |= static_cast<uint64_t>(2) << 61;                      // SWIZZLE_128B
     return d;
 }
-// instruction descriptor, kind::i8: D = S32, A = B = signed 8 bit, both K-major, N = 256, M = 128
-constexpr uint32_t IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((BN >> 3) << 17) | ((BM >> 4) << 24);
-
-__device__ __forceinline__ void umma_i8(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
-    asm volatile(
-            "{\n\t"
-            ".reg .pred p;\n\t"
-            "setp.ne.b32 p, %4, 0;\n\t"
-            "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t"
-            "}" ::"r"(d_tmem),
-            "l"(a_desc), "l"(b_desc), "r"(IDESC), "r"(accumulate)
-            : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
     asm volatile(
             "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -606,15 +563,15 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
 }
 
 struct WorkItem {
-    uint32_t rb, cb;   // row block (x128), column block (x256)
+    uint32_t rb, cb;   // row block (x256), column block (x256)
     uint32_t k0, k1;   // k-block range
     uint32_t partial;  // 1: the tile's K range is shared with other CTAs -> atomics only
 };
 
 // Work list of one launch: the first n_full items are whole tiles (all k-blocks), n_full a multiple of
-// the grid so that every CTA owns the same number of them; the remaining tiles are cut into `splits`
+// the number of pairs so that every pair owns the same number of them; the remaining tiles are cut into `splits`
 // K ranges each, so that the last round keeps every SM busy for 1/splits of a tile instead of leaving
-// most of them idle for a whole tile (1 055 tiles on 148 SMs = 7.13 rounds).
+// most of them idle for a whole tile (528 tiles on 74 pairs = 7.13 rounds).
 struct WorkList {
     const uint2 *tiles; // (row block, column block), rasterised for L2 reuse
     uint32_t n_full;    // tiles processed whole
@@ -625,7 +582,7 @@ struct WorkList {
     uint32_t ck_shift;  // log2(k-blocks per chunk of the panel layout)
     uint32_t kb_neg0;   // k-blocks >= kb_neg0 hold tail reads only: their B operand is k-block kb + kb_negd (-Z)
     uint32_t kb_negd;
-    unsigned int *wave_ctr; // CTA-pair kernel: pairs that have issued all loads of their n-th work item (null = no wave sync)
+    unsigned int *wave_ctr; // pairs that have issued all loads of their n-th work item
 };
 __device__ __forceinline__ WorkItem work_item(const WorkList &wl, uint32_t w) {
     if (w < wl.n_full) {
@@ -647,199 +604,21 @@ enum : int {
 };
 
 // ------------------------------------------------------------------------------------------------
-// the GEMM
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(GEMM_THREADS, 1) syrk_kernel(const __grid_constant__ CUtensorMap map_u,
-                                                               const WorkList wl, int32_t *__restrict__ S,
-                                                               int32_t *__restrict__ D, uint32_t n_cells, int sign,
-                                                               int epi_mode) {
-    const uint32_t n_work = wl.n_work;
-    extern __shared__ uint8_t smem_raw[];
-    // 128B swizzle needs 1024-byte aligned tiles
-    uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + STAGES * STAGE_BYTES);
-    // bars[0..S) full, [S..2S) empty, [2S] tmem_full, [2S+1] tmem_empty, then the TMEM base address
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * STAGES + 2);
-    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + STAGES);
-    const uint32_t tmem_full = smem_u32(bars + 2 * STAGES), tmem_empty = smem_u32(bars + 2 * STAGES + 1);
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_u) : "memory");
-        for (int s = 0; s < STAGES; ++s) {
-            mbar_init(full0 + 8 * s, 1);
-            mbar_init(empty0 + 8 * s, 1);
-        }
-        mbar_init(tmem_full, 1);
-        mbar_init(tmem_empty, 128);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tmem_Q = tmem_base, tmem_T = tmem_base + BN; // columns [0,256) and [256,512)
-
-    if (warp == 0) {
-        // ===== TMA producer =====
-        if (elect_one()) {
-            uint32_t stage = 0, phase = 0;
-            for (uint32_t w = blockIdx.x; w < n_work; w += gridDim.x) {
-                const WorkItem wi = work_item(wl, w);
-                for (uint32_t kb = wi.k0; kb < wi.k1; ++kb) {
-                    if (PREFETCH_KB && kb + PREFETCH_KB < wi.k1 && kb + PREFETCH_KB < wl.kb_neg0) {
-                        const uint32_t kp = kb + PREFETCH_KB;
-                        const int32_t chp = static_cast<int32_t>(kp >> wl.ck_shift);
-                        const int32_t kxp = static_cast<int32_t>((kp - (static_cast<uint32_t>(chp) << wl.ck_shift)) * KB_BYTES);
-                        tma_prefetch_3d(&map_u, kxp, wi.rb * BM, chp);
-                        tma_prefetch_3d(&map_u, kxp, wi.cb * BN, chp);
-                        tma_prefetch_3d(&map_u, kxp, wi.cb * BN + 128, chp);
-                    }
-                    mbar_wait(empty0 + 8 * stage, phase ^ 1);
-                    const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES), sb = sa + A_BYTES;
-                    const uint32_t bar = full0 + 8 * stage;
-                    mbar_expect_tx(bar, STAGE_BYTES);
-                    const int32_t ch = static_cast<int32_t>(kb >> wl.ck_shift);
-                    const int32_t kx = static_cast<int32_t>((kb - (static_cast<uint32_t>(ch) << wl.ck_shift)) * KB_BYTES);
-                    const uint32_t kbb = kb >= wl.kb_neg0 ? kb + wl.kb_negd : kb;
-                    const int32_t chb = static_cast<int32_t>(kbb >> wl.ck_shift);
-                    const int32_t kxb = static_cast<int32_t>((kbb - (static_cast<uint32_t>(chb) << wl.ck_shift)) * KB_BYTES);
-                    tma_load_3d(sa, &map_u, bar, kx, wi.rb * BM, ch);
-                    tma_load_3d(sb, &map_u, bar, kxb, wi.cb * BN, chb);
-                    tma_load_3d(sb + A_BYTES, &map_u, bar, kxb, wi.cb * BN + 128, chb);
-                    if (++stage == STAGES) {
-                        stage = 0;
-                        phase ^= 1;
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer =====
-        if (elect_one()) {
-            uint32_t stage = 0, phase = 0, acc_phase = 0;
-            for (uint32_t w = blockIdx.x; w < n_work; w += gridDim.x) {
-                const WorkItem wi = work_item(wl, w);
-                mbar_wait(tmem_empty, acc_phase ^ 1); // epilogue has drained the accumulators
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                for (uint32_t kb = wi.k0; kb < wi.k1; ++kb) {
-                    mbar_wait(full0 + 8 * stage, phase);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES), sb = sa + A_BYTES;
-                    const uint32_t first = kb == wi.k0 ? 0u : 1u;
-                    // plane 0 (u_0 = reads per cell) -> T; planes 1..3 -> Q = 4S - T
-                    umma_i8(tmem_T, make_desc(sa), make_desc(sb), first);
-                    umma_i8(tmem_Q, make_desc(sa + 32), make_desc(sb + 32), first);
-                    umma_i8(tmem_Q, make_desc(sa + 64), make_desc(sb + 64), 1u);
-                    umma_i8(tmem_Q, make_desc(sa + 96), make_desc(sb + 96), 1u);
-                    umma_commit(empty0 + 8 * stage); // frees the smem slot once these MMAs retire
-                    if (++stage == STAGES) {
-                        stage = 0;
-                        phase ^= 1;
-                    }
-                }
-                umma_commit(tmem_full); // accumulators complete
-                acc_phase ^= 1;
-            }
-        }
-    } else {
-        // ===== epilogue: warps 2..5, TMEM lanes 32*(warp%4) .. +31 =====
-        const uint32_t lane_base = 32 * (warp & 3);
-        uint32_t acc_phase = 0;
-        for (uint32_t w = blockIdx.x; w < n_work; w += gridDim.x) {
-            const WorkItem wi = work_item(wl, w);
-            mbar_wait(tmem_full, acc_phase);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint32_t row = wi.rb * BM + lane_base + lane;
-            int32_t *Srow = S + static_cast<uint64_t>(row) * n_cells;
-            int32_t *Drow = D + static_cast<uint64_t>(row) * n_cells;
-            // a tile strictly above the diagonal and inside the matrix needs no per-element guards
-            const bool interior = wi.cb * BN >= wi.rb * BM + BM && wi.cb * BN + BN <= n_cells && wi.rb * BM + BM <= n_cells;
-            const bool vec = interior && !wi.partial && epi_mode != EPI_RED && (n_cells & 3u) == 0;
-#pragma unroll 1
-            for (uint32_t cc = 0; cc < BN / 32; ++cc) {
-                uint32_t q[32], t[32];
-                tmem_ld32(tmem_Q + (lane_base << 16) + cc * 32, q);
-                tmem_ld32(tmem_T + (lane_base << 16) + cc * 32, t);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                const uint32_t col0 = wi.cb * BN + cc * 32;
-                if (vec) {
-                    // each thread owns 128 contiguous bytes of its row in either plane
-                    int4 *ps = reinterpret_cast<int4 *>(Srow + col0), *pd = reinterpret_cast<int4 *>(Drow + col0);
-                    int4 os[8], od[8];
-                    if (epi_mode == EPI_RMW) {
-#pragma unroll
-                        for (int k = 0; k < 8; ++k) {
-                            os[k] = ps[k];
-                            od[k] = pd[k];
-                        }
-                    }
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        int32_t sv[4], dv[4];
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const int32_t tv = static_cast<int32_t>(t[4 * k + e]);
-                            sv[e] = (static_cast<int32_t>(q[4 * k + e]) + tv) >> 2; // (4S - T + T) / 4
-                            dv[e] = tv - sv[e];
-                        }
-                        int4 vs = make_int4(sign * sv[0], sign * sv[1], sign * sv[2], sign * sv[3]);
-                        int4 vd = make_int4(sign * dv[0], sign * dv[1], sign * dv[2], sign * dv[3]);
-                        if (epi_mode == EPI_RMW) {
-                            vs.x += os[k].x, vs.y += os[k].y, vs.z += os[k].z, vs.w += os[k].w;
-                            vd.x += od[k].x, vd.y += od[k].y, vd.z += od[k].z, vd.w += od[k].w;
-                        }
-                        ps[k] = vs;
-                        pd[k] = vd;
-                    }
-                } else if (row < n_cells && col0 + 31 > row) {
-#pragma unroll
-                    for (int k = 0; k < 32; ++k) {
-                        const uint32_t col = col0 + k;
-                        const int32_t tv = static_cast<int32_t>(t[k]);
-                        const int32_t sv = (static_cast<int32_t>(q[k]) + tv) >> 2; // (4S - T + T) / 4
-                        const int32_t dv = tv - sv;
-                        if (col > row && col < n_cells) {
-                            if (sv) {
-                                atomicAdd(Srow + col, sign * sv);
-                            }
-                            if (dv) {
-                                atomicAdd(Drow + col, sign * dv);
-                            }
-                        }
-                    }
-                }
-            }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            mbar_arrive(tmem_empty);
-            acc_phase ^= 1;
-        }
-    }
-    __syncthreads();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
-    }
-}
-
-
-// ------------------------------------------------------------------------------------------------
-// the same GEMM on CTA pairs (tcgen05 cta_group::2): a cluster of two CTAs owns a 256 x 256 output tile,
+// the GEMM on CTA pairs (tcgen05 cta_group::2): a cluster of two CTAs owns a 256 x 256 output tile,
 // each CTA 128 of its rows (its own TMEM) and HALF of the B operand (128 of the 256 columns' rows), which
 // the tensor cores of both SMs read across the pair. Per CTA and k-block that is 32 KB of operands
-// instead of 48 KB (6 pipeline stages instead of 4, a third less L2->SM traffic and shared-memory
-// bandwidth). Only the leader CTA issues MMAs; both CTAs' TMA loads report to the leader's barrier; the
-// leader's commits release the stage / publish the accumulators in both CTAs (multicast).
+// instead of the 48 KB of a single CTA with a 128 x 256 tile (a deeper ring, a third less L2->SM traffic
+// and shared-memory bandwidth). Only the leader CTA issues MMAs; both CTAs' TMA loads report to the leader's
+// barrier; the leader's commits release the stage / publish the accumulators in both CTAs (multicast).
 // ------------------------------------------------------------------------------------------------
 constexpr int HALF_B_BYTES = 128 * KB_BYTES;             // 16 KB
-constexpr int STAGE2_BYTES = A_BYTES + HALF_B_BYTES;     // 32 KB per CTA
-// the operand ring is a template parameter: 6 stages (193 KB) when the kernel has the SM to itself, 5 or 4 (161 / 129 KB) to
-// leave shared memory to the staging kernels of the next batch that run beside it (sgpu_ctx::tensor_jobs)
-constexpr int smem2_bytes(int stages) { return stages * STAGE2_BYTES + 1024 + 256; }
-constexpr uint32_t IDESC2 = (2u << 4) | (1u << 7) | (1u << 10) | ((256u >> 3) << 17) | ((256u >> 4) << 24); // M = 256, N = 256
+constexpr int STAGE_BYTES = A_BYTES + HALF_B_BYTES;      // 32 KB per CTA
+// 5 stages (161 KB) leave shared memory to the staging kernels of the next batch that run beside the deferred kernel
+// (sgpu_ctx::tensor_jobs); 4 are slower. With the SM to itself (SECEDO_B200_ASYNC_GEMM=0) 6 stages (193 KB) would be
+// 2-3 % faster per launch (DESIGN.md 4, K3)
+constexpr int STAGES = 5;
+constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */;
+constexpr uint32_t IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((256u >> 3) << 17) | ((256u >> 4) << 24); // M = 256, N = 256
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
@@ -877,7 +656,7 @@ __device__ __forceinline__ void umma_i8_2sm(uint32_t d_tmem, uint64_t a_desc, ui
             "setp.ne.b32 p, %4, 0;\n\t"
             "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t"
             "}" ::"r"(d_tmem),
-            "l"(a_desc), "l"(b_desc), "r"(IDESC2), "r"(accumulate)
+            "l"(a_desc), "l"(b_desc), "r"(IDESC), "r"(accumulate)
             : "memory");
 }
 __device__ __forceinline__ void umma_commit_2sm(uint32_t bar) { // arrives on `bar` in BOTH CTAs of the pair
@@ -887,17 +666,16 @@ __device__ __forceinline__ void umma_commit_2sm(uint32_t bar) { // arrives on `b
 }
 
 // work item of a pair: tiles are (row block of 256, column block of 256)
-template <int STAGES2>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
         syrk2_kernel(const __grid_constant__ CUtensorMap map_u, const WorkList wl, int32_t *__restrict__ S, int32_t *__restrict__ D,
                      uint32_t n_cells, int epi_mode) {
     const uint32_t n_work = wl.n_work;
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + STAGES2 * STAGE2_BYTES);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * STAGES2 + 2);
-    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + STAGES2);
-    const uint32_t tmem_full = smem_u32(bars + 2 * STAGES2), tmem_empty = smem_u32(bars + 2 * STAGES2 + 1);
+    uint64_t *bars = reinterpret_cast<uint64_t *>(smem + STAGES * STAGE_BYTES);
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * STAGES + 2);
+    const uint32_t full0 = smem_u32(bars), empty0 = smem_u32(bars + STAGES);
+    const uint32_t tmem_full = smem_u32(bars + 2 * STAGES), tmem_empty = smem_u32(bars + 2 * STAGES + 1);
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
     const uint32_t pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
@@ -905,7 +683,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&map_u) : "memory");
-        for (int s = 0; s < STAGES2; ++s) {
+        for (int s = 0; s < STAGES; ++s) {
             mbar_init(full0 + 8 * s, 2);  // one arrive.expect_tx per CTA of the pair (only the leader's is used)
             mbar_init(empty0 + 8 * s, 1); // the leader's commit, multicast
         }
@@ -934,7 +712,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
                 // slabs through L2, but L2 only holds what was fetched during the last ~30 us; without this the pairs
                 // drift apart (diagonal tiles have slower epilogues) and every pair streams its slabs from HBM again.
                 // All pairs are resident (grid <= SM count, one CTA per SM), every wave before the last one is full.
-                if (wl.wave_ctr != nullptr && leader && wave > 0) {
+                if (leader && wave > 0) {
                     atomicAdd(wl.wave_ctr, 1u);
                     // arrivals so far: n_pairs per earlier wave, and the pairs that have an item in this (maybe last, partial) wave
                     const uint32_t want = (wave - 1) * n_pairs + min(n_pairs, n_work - wave * n_pairs);
@@ -948,9 +726,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
                 }
                 for (uint32_t kb = wi.k0; kb < wi.k1; ++kb) {
                     mbar_wait(empty0 + 8 * stage, phase ^ 1);
-                    const uint32_t sa = smem_u32(smem + stage * STAGE2_BYTES), sb = sa + A_BYTES;
+                    const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES), sb = sa + A_BYTES;
                     const uint32_t bar = mapa_u32(full0 + 8 * stage, 0); // the leader's barrier
-                    mbar_expect_tx_remote(bar, STAGE2_BYTES);
+                    mbar_expect_tx_remote(bar, STAGE_BYTES);
                     const int32_t ch = static_cast<int32_t>(kb >> wl.ck_shift);
                     const int32_t kx = static_cast<int32_t>((kb - (static_cast<uint32_t>(ch) << wl.ck_shift)) * KB_BYTES);
                     const uint32_t kbb = kb >= wl.kb_neg0 ? kb + wl.kb_negd : kb;
@@ -958,7 +736,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
                     const int32_t kxb = static_cast<int32_t>((kbb - (static_cast<uint32_t>(chb) << wl.ck_shift)) * KB_BYTES);
                     tma_load_3d_2sm(sa, &map_u, bar, kx, wi.rb * 256 + rank * 128, ch);
                     tma_load_3d_2sm(sb, &map_u, bar, kxb, wi.cb * 256 + rank * 128, chb);
-                    if (++stage == STAGES2) {
+                    if (++stage == STAGES) {
                         stage = 0;
                         phase ^= 1;
                     }
@@ -976,14 +754,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
                 for (uint32_t kb = wi.k0; kb < wi.k1; ++kb) {
                     mbar_wait(full0 + 8 * stage, phase);
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    const uint32_t sa = smem_u32(smem + stage * STAGE2_BYTES), sb = sa + A_BYTES;
+                    const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES), sb = sa + A_BYTES;
                     const uint32_t first = kb == wi.k0 ? 0u : 1u;
                     umma_i8_2sm(tmem_T, make_desc(sa), make_desc(sb), first);
                     umma_i8_2sm(tmem_Q, make_desc(sa + 32), make_desc(sb + 32), first);
                     umma_i8_2sm(tmem_Q, make_desc(sa + 64), make_desc(sb + 64), 1u);
                     umma_i8_2sm(tmem_Q, make_desc(sa + 96), make_desc(sb + 96), 1u);
                     umma_commit_2sm(empty0 + 8 * stage); // frees the slot in both CTAs once these MMAs retire
-                    if (++stage == STAGES2) {
+                    if (++stage == STAGES) {
                         stage = 0;
                         phase ^= 1;
                     }
@@ -1084,10 +862,7 @@ struct TensorLaunch {
     int32_t *S = nullptr, *D = nullptr;
     uint32_t N = 0;
     int epi = EPI_RMW;
-    unsigned grid = 0;
-    int stages2 = 6;
-    bool pairs = true;
-    int *err = nullptr;                    // [1]: wave counter (null: no wave sync)
+    unsigned grid = 0;                     // CTA pairs
     sgpu_ctx::TensorJob job;               // events + what the job will own
     cudaEvent_t staged = nullptr;          // on ctx->stream, behind the staging kernel (late launches only)
 };
@@ -1095,21 +870,9 @@ struct TensorLaunch {
 // t0, memset of the wave counter, kernel, t1 on stream gs; the job joins the context's list
 int issue_tensor_launch(sgpu_ctx *ctx, cudaStream_t gs, TensorLaunch &tl) {
     ctx->tensor_jobs.push_back(tl.job); // the list owns the events and the panel from here on, whatever happens below
-    if (tl.err && tl.wl.wave_ctr) {
-        SGPU_CUDA(ctx, cudaMemsetAsync(tl.err + 1, 0, sizeof(int), gs));
-    }
+    SGPU_CUDA(ctx, cudaMemsetAsync(tl.wl.wave_ctr, 0, sizeof(unsigned int), gs));
     SGPU_CUDA(ctx, cudaEventRecord(tl.job.t0, gs));
-    if (tl.pairs) {
-        if (tl.stages2 == 4) {
-            SGPU_LAUNCH(ctx, (syrk2_kernel<4><<<2 * tl.grid, GEMM_THREADS, smem2_bytes(4), gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, tl.epi)));
-        } else if (tl.stages2 == 5) {
-            SGPU_LAUNCH(ctx, (syrk2_kernel<5><<<2 * tl.grid, GEMM_THREADS, smem2_bytes(5), gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, tl.epi)));
-        } else {
-            SGPU_LAUNCH(ctx, (syrk2_kernel<6><<<2 * tl.grid, GEMM_THREADS, smem2_bytes(6), gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, tl.epi)));
-        }
-    } else {
-        SGPU_LAUNCH(ctx, (syrk_kernel<<<tl.grid, GEMM_THREADS, SMEM_BYTES, gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, 1, tl.epi)));
-    }
+    SGPU_LAUNCH(ctx, (syrk2_kernel<<<2 * tl.grid, GEMM_THREADS, SMEM_BYTES, gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, tl.epi)));
     const cudaError_t le = cudaGetLastError();
     SGPU_CUDA(ctx, cudaEventRecord(tl.job.t1, gs));
     SGPU_CUDA(ctx, le);
@@ -1152,28 +915,24 @@ int sgpu_tensor_flush(sgpu_ctx *ctx, bool after_main) {
     return issue_tensor_launch(ctx, gs, *tl);
 }
 
-// Upper-triangle output tiles in an order that keeps the tiles in flight (one per SM) inside a block
-// of ~18 row blocks x 8 column blocks, so that a wave touches ~4 400 distinct operand rows instead of
+// Upper-triangle 256 x 256 output tiles in an order that keeps the tiles in flight (one per CTA pair) inside a block
+// of ~9 row blocks x 8 column blocks, so that a wave touches ~4 400 distinct operand rows instead of
 // ~20 000: bands of 8 column blocks, row-block-major inside a band.
-static int tile_list(sgpu_ctx *ctx, uint32_t N, uint32_t n_pad, uint32_t bm /* tile height: 128, or 256 for CTA pairs */,
-                     const uint2 **d_tiles, uint32_t *n_tiles) {
-    uint32_t BAND = 8;
-    if (const char *env = getenv("SECEDO_B200_TILE_BAND")) { // raster experiments (profiles/)
-        BAND = static_cast<uint32_t>(std::max(1, atoi(env)));
-    }
-    if (ctx->tile_cache && ctx->tile_cache_cells == N && ctx->tile_cache_bm == (bm | (BAND << 16))) {
+static int tile_list(sgpu_ctx *ctx, uint32_t N, uint32_t n_pad, const uint2 **d_tiles, uint32_t *n_tiles) {
+    constexpr uint32_t BAND = 8;
+    if (ctx->tile_cache && ctx->tile_cache_cells == N) {
         *d_tiles = static_cast<const uint2 *>(ctx->tile_cache);
         *n_tiles = ctx->tile_cache_n;
         return SGPU_OK;
     }
     std::vector<uint2> tiles;
-    const uint32_t n_cb = n_pad / BN, n_rb = n_pad / bm;
+    const uint32_t n_cb = n_pad / BN, n_rb = n_pad / BN;
     for (uint32_t band = 0; band < n_cb; band += BAND) {
         const uint32_t cb_end = std::min(n_cb, band + BAND);
         for (uint32_t rb = 0; rb < n_rb; ++rb) {
             for (uint32_t cb = band; cb < cb_end; ++cb) {
                 // the tile intersects the upper triangle: its last column > its first row
-                if (cb * BN + BN - 1 > rb * bm && rb * bm < N && cb * BN < N) {
+                if (cb * BN + BN - 1 > rb * BN && rb * BN < N && cb * BN < N) {
                     tiles.push_back(make_uint2(rb, cb));
                 }
             }
@@ -1187,7 +946,6 @@ static int tile_list(sgpu_ctx *ctx, uint32_t N, uint32_t n_pad, uint32_t bm /* t
     SGPU_CUDA(ctx, cudaMalloc(&ctx->tile_cache, std::max<size_t>(1, tiles.size()) * sizeof(uint2)));
     SGPU_CUDA(ctx, cudaMemcpy(ctx->tile_cache, tiles.data(), tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice));
     ctx->tile_cache_cells = N;
-    ctx->tile_cache_bm = bm | (BAND << 16);
     ctx->tile_cache_n = static_cast<uint32_t>(tiles.size());
     *d_tiles = static_cast<const uint2 *>(ctx->tile_cache);
     *n_tiles = ctx->tile_cache_n;
@@ -1246,9 +1004,6 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
     const uint64_t kbs_max = panel / LOCI_PER_KB + 2ull * kbs_tail;
     PanelLayout pl;
     pl.ck_shift = 5; // 32 k-blocks = 1 024 loci per chunk: 4 KB per cell, 33.8 MB per chunk at 8 192 cells
-    if (const char *env = getenv("SECEDO_B200_CHUNK_SHIFT")) {
-        pl.ck_shift = static_cast<uint32_t>(std::min(10, std::max(0, atoi(env))));
-    }
     const uint32_t ck = 1u << pl.ck_shift;
     pl.cell_words = (ck | 1u) * 32u; // odd number of lines: consecutive cells do not alias in the L2 sets
     pl.chunk_words = static_cast<uint64_t>(n_pad) * pl.cell_words;
@@ -1257,9 +1012,7 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
 
     // tensor kernels of earlier batches: issue the one still pending, retire the finished ones; never more than two operand
     // panels in flight
-    if (ctx->flush_point != 2) {
-        SGPU_TRY(sgpu_tensor_flush(ctx, false));
-    }
+    SGPU_TRY(sgpu_tensor_flush(ctx, false));
     SGPU_TRY(sgpu_tensor_poll(ctx, false));
     while (ctx->tensor_jobs.size() >= 2) {
         SGPU_CUDA(ctx, cudaEventSynchronize(ctx->tensor_jobs.front().t1));
@@ -1290,32 +1043,17 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
         if (fn == nullptr || qres != cudaDriverEntryPointSuccess) {
             return sgpu_fail(ctx, SGPU_E_CUDA, "driver does not provide cuTensorMapEncodeTiled");
         }
-        CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-        if (const char *env = getenv("SECEDO_B200_L2_PROMO")) { // 0 / 64 / 128 / 256 (profiles/)
-            const int v = atoi(env);
-            promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                    : v == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-        }
         CUresult r = reinterpret_cast<encode_fn>(fn)(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, U.p, gdim, gstride, box, estr,
                                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                            promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) {
             return sgpu_fail(ctx, SGPU_E_CUDA, "cuTensorMapEncodeTiled failed (%d)", static_cast<int>(r));
         }
     }
-    // CTA pairs (tcgen05 cta_group::2, 256 x 256 tiles) or single CTAs (128 x 256 tiles)
-    const char *env_pair = getenv("SECEDO_B200_GEMM_PAIRS");
-    const bool pairs = env_pair ? env_pair[0] == '1' : (ctx->sm_count % 2 == 0); // default; SECEDO_B200_GEMM_PAIRS=0 for single CTAs
-    const char *env_ws = getenv("SECEDO_B200_WAVE_SYNC");
-    const bool wave_sync = env_ws ? env_ws[0] == '1' : true;
-    const int stages2 = ctx->gemm_stages == 4 ? 4 : ctx->gemm_stages == 5 ? 5 : 6;
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2_bytes(4)));
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2_bytes(5)));
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2_bytes(6)));
+    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     const uint2 *d_tiles = nullptr;
     uint32_t n_tiles = 0;
-    SGPU_TRY(tile_list(ctx, N, n_pad, pairs ? 256 : BM, &d_tiles, &n_tiles));
+    SGPU_TRY(tile_list(ctx, N, n_pad, &d_tiles, &n_tiles));
     SGPU_TRACE(ctx, "gemm: tensor map + tiles");
 
     // The tensor kernel goes to the context's tensor stream behind an event of its staging kernel and the call returns
@@ -1363,12 +1101,8 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
         }
     } event_return{ ctx, &ev_s0, &ev_s1 };
     const uint32_t sms = static_cast<uint32_t>(ctx->sm_count);
-    // stripes of cells per staging CTA: as few as a 104 KB tile allows
-    uint32_t st_cells = ST_MAX_CELLS;
-    if (const char *env = getenv("SECEDO_B200_STAGE_CELLS")) { // experiments (profiles/): smaller tiles, more staging CTAs per SM
-        st_cells = static_cast<uint32_t>(std::min<int>(ST_MAX_CELLS, std::max(64, atoi(env))));
-    }
-    const uint32_t n_stripes = std::min<uint32_t>(ST_MAX_STRIPES, (n_pad + st_cells - 1) / st_cells);
+    // stripes of cells per staging CTA: as few as the largest tile (ST_MAX_CELLS) allows
+    const uint32_t n_stripes = std::min<uint32_t>(ST_MAX_STRIPES, (n_pad + ST_MAX_CELLS - 1) / ST_MAX_CELLS);
     const uint32_t cells_per_cta = ((n_pad + n_stripes - 1) / n_stripes + 3) / 4 * 4;
     const size_t st_smem = static_cast<size_t>(cells_per_cta) * 128;
     SGPU_CUDA(ctx, cudaFuncSetAttribute(stage_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(st_smem)));
@@ -1409,9 +1143,6 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
             return SGPU_OK;
         };
         SGPU_TRY(in.gid_base32 ? run_partition(in.gid_base32) : run_partition(in.gid_base));
-        if (ctx->flush_point == 2) {
-            SGPU_TRY(sgpu_tensor_flush(ctx, true));
-        }
     }
 
     bool first = true;
@@ -1482,10 +1213,10 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
         wl.ck_shift = pl.ck_shift;
         wl.kb_neg0 = kbs_main;
         wl.kb_negd = kt;
-        wl.wave_ctr = nullptr;
+        wl.wave_ctr = reinterpret_cast<unsigned int *>(errp + 1);
         // whole tiles in full rounds of the grid; the rest (or everything, when there are few tiles) in
         // K ranges so that every SM has work in the last round
-        const uint32_t units = pairs ? sms / 2 : sms; // CTAs or CTA pairs that take work items
+        const uint32_t units = sms / 2; // CTA pairs that take work items
         wl.n_full = n_tiles >= 2 * units ? n_tiles / units * units : 0;
         const uint32_t rest = n_tiles - wl.n_full;
         uint32_t splits = 1;
@@ -1507,17 +1238,11 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
         tl.N = N;
         tl.epi = epi;
         tl.grid = grid;
-        tl.stages2 = stages2;
-        tl.pairs = pairs;
-        tl.err = errp;
         tl.job.planes = S_plane;
-        if (pairs && wave_sync) {
-            tl.wl.wave_ctr = reinterpret_cast<unsigned int *>(errp + 1);
-        }
         SGPU_CUDA(ctx, get_event(&tl.job.t0));
         SGPU_CUDA(ctx, get_event(&tl.job.t1));
         *fresh = false;
-        if (last && defer && ctx->late_gemm) {
+        if (last && defer) {
             // prepared, not issued: sgpu_tensor_flush (behind the next batch's link_window kernel, or at the first join)
             TensorLaunch *pending = new TensorLaunch(tl);
             if (get_event(&pending->staged) != cudaSuccess || cudaEventRecord(pending->staged, st) != cudaSuccess) {

@@ -1127,13 +1127,6 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
     // table geometry: slots >= 3 x the largest locus if shared memory allows, never below 1.25 x; the ring holds the
     // read ids of WIN_RING loci (each slot: the largest locus + up to 3 elements of alignment offset)
     const uint32_t id_cap = (max_n + 3 + 3) & ~3u;
-    unsigned long long slot_factor = 3;
-    if (const char *env = getenv("SECEDO_B200_WIN_SLOT_FACTOR")) { // experiments (profiles/): table size / occupancy trade-off
-        slot_factor = static_cast<unsigned long long>(std::max(1, atoi(env)));
-    }
-    // shared memory a CTA may take: everything, or what the tensor kernel of the previous batch leaves on its SM
-    // (sgpu_ctx::tensor_jobs; a CTA that does not fit beside it would wait for that kernel to end)
-    const size_t win_limit = ctx->win_smem_limit ? std::min<size_t>(ctx->win_smem_limit, WIN_SMEM_LIMIT) : WIN_SMEM_LIMIT;
     auto pow2_slots = [&](unsigned long long want) {
         uint32_t sl = 1024;
         while (sl < want && sl < 65536) {
@@ -1146,29 +1139,27 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
         return static_cast<size_t>(n_ring) * id_cap * 4 + REC_BUF * sizeof(uint2) + static_cast<size_t>(s) * 2;
     };
     // preference: a ring of at least two loci (no exposed global latency per owner) before a sparse table (fewer second
-    // probes); huge loci (cfg5: 20 000 reads) end at one resident locus and the largest table that fits
-    auto choose_geometry = [&](size_t limit) {
-        const uint32_t s_full = pow2_slots(slot_factor * max_n), s_half = std::min(s_full, pow2_slots(2ull * max_n));
+    // probes); huge loci (cfg5: 20 000 reads) end at one resident locus and the largest table that fits. A CTA takes a
+    // whole SM's shared memory: a geometry that fits beside the previous batch's tensor kernel (60 KB: one CTA per SM, a
+    // denser table) was slower than letting link_window wait for it (profiles/r2_overlap_probes.txt).
+    auto choose_geometry = [&]() {
+        const uint32_t s_full = pow2_slots(3ull * max_n), s_half = std::min(s_full, pow2_slots(2ull * max_n));
         const uint32_t cand[4][2] = { { WIN_RING, s_full }, { 2, s_full }, { WIN_RING, s_half }, { 2, s_half } };
-        const char *env_ring = getenv("SECEDO_B200_WIN_RING"); // experiments (profiles/): 1 = one resident locus, full table
         for (const auto &cd : cand) {
             n_ring = cd[0];
             slots = cd[1];
-            if (win_smem(slots) <= limit && !(env_ring && env_ring[0] == '1')) {
+            if (win_smem(slots) <= WIN_SMEM_LIMIT) {
                 return true;
             }
         }
         n_ring = 1;
         slots = s_full;
-        while (slots > 1024 && win_smem(slots) > limit) {
+        while (slots > 1024 && win_smem(slots) > WIN_SMEM_LIMIT) {
             slots >>= 1;
         }
-        return win_smem(slots) <= limit && 4ull * slots >= 5ull * max_n;
+        return win_smem(slots) <= WIN_SMEM_LIMIT && 4ull * slots >= 5ull * max_n;
     };
-    bool window_fits = choose_geometry(win_limit);
-    if (!window_fits && win_limit < WIN_SMEM_LIMIT) { // rather wait for the whole SM than fall back to the global hash
-        window_fits = choose_geometry(WIN_SMEM_LIMIT);
-    }
+    const bool window_fits = choose_geometry();
     // SECEDO_B200_FORCE_GLOBAL_HASH=1 forces the large-locus path (tests)
     const char *force_global = getenv("SECEDO_B200_FORCE_GLOBAL_HASH");
     const bool use_window = max_n <= WIN_MAX_ENTRIES && window_fits && 4ull * slots >= 5ull * max_n
@@ -1215,9 +1206,7 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
         SGPU_CUDA(ctx, cudaGetLastError());
         // the previous batch's tensor kernel, if its launch has been held back: behind the dense linking pass, beside
         // everything that follows (sgpu_tensor_flush)
-        if (ctx->flush_point == 0) {
-            SGPU_TRY(sgpu_tensor_flush(ctx, true));
-        }
+        SGPU_TRY(sgpu_tensor_flush(ctx, true));
         SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_ctr.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         SGPU_CUDA(ctx, cudaStreamSynchronize(st));
         NL = ctx->h_scratch[0];
@@ -1447,9 +1436,6 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
     SGPU_CUDA(ctx, cudaGetLastError());
 
     SGPU_TRACE(ctx, "link: cutoff+finish");
-    if (ctx->flush_point == 1) { // the held-back tensor kernel behind the special-entry chain instead of behind link_window
-        SGPU_TRY(sgpu_tensor_flush(ctx, true));
-    }
     // scalars to the host: errors, stats, reads created, tail loci per chromosome
     std::vector<uint64_t> h_nt(p->n_chr), h_tl(p->n_chr);
     SGPU_CUDA(ctx, cudaMemcpyAsync(h_tl.data(), out->tail_locus.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));

@@ -270,10 +270,10 @@ def test_filtered_view_of_read_ids(gpu_ctx, path, monkeypatch):
     c.free()
 
 
-def test_scheduling_knobs_do_not_change_results():
-    """the tensor kernel beside the next batch (own stream, held-back launch, operand ring, cache preference): whatever the
-    knobs say, a filter -> accumulate loop over several batches gives the same count planes and the same matrix, and they
-    are the oracle's"""
+def test_scheduling_options_do_not_change_results():
+    """the tensor kernel beside the next batch (own stream, held-back launch, cache preference): whatever the knobs say, a
+    filter -> accumulate loop over several batches gives the same count planes and the same matrix, and they are the
+    oracle's; the knobs of earlier versions and out-of-range values are refused"""
     ctx = api.Context(0)
     n = 1536
     ident = np.arange(n, dtype=np.uint32)
@@ -286,8 +286,7 @@ def test_scheduling_knobs_do_not_change_results():
         want = [o.S1, o.D1, o.H] if want is None else [want[0] + o.S1, want[1] + o.D1, want[2] + o.H]
     c = api.Counts(ctx, n)
     first_M = None
-    for knobs in ({"async_gemm": 0}, {"async_gemm": 1, "late_gemm": 0}, {"async_gemm": 1, "late_gemm": 1, "gemm_stages": 6},
-                  {"gemm_stages": 4, "prefer_shared": 1}, {"gemm_stages": 5, "prefer_shared": 0}, {"prefer_shared": 2}):
+    for knobs in ({"async_gemm": 0}, {"async_gemm": 1, "prefer_shared": 0}, {"prefer_shared": 1}):
         for k, v in knobs.items():
             ctx.set_option(k, v)
         c.zero()
@@ -301,8 +300,9 @@ def test_scheduling_knobs_do_not_change_results():
         if first_M is None:
             first_M = M
         assert np.array_equal(M, first_M), knobs
-    with pytest.raises(api.SgpuError):
-        ctx.set_option("no_such_knob", 1)
+    for name, value in (("no_such_knob", 1), ("late_gemm", 1), ("gemm_stages", 5), ("win_smem_kb", 60), ("prefer_shared", 2)):
+        with pytest.raises(api.SgpuError):
+            ctx.set_option(name, value)
     c.free()
     for fd in devs:
         fd.free()
