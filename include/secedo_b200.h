@@ -42,7 +42,9 @@ enum {
     SGPU_E_CELL_RANGE = -3,    /* group id >= n_groups or mapped cell >= num_cells (mat.hpp:119 assert) */
     SGPU_E_FRAGMENT_SPAN = -4, /* a read id chained over >= max_fragment_length, only with SECEDO_B200_STRICT_SPAN=1 (by
                                   default such a chain is split into reads the way the reference's retirement does) */
-    SGPU_E_CLASS_RANGE = -5,   /* a read pair overlaps at >= SGPU_MAX_CLASS (or >= L) loci */
+    SGPU_E_CLASS_RANGE = -5,   /* a read pair overlaps in a class (x_s, x_d) without a log-likelihood: x_s or x_d >=
+                                  SGPU_MAX_CLASS or >= L, or x_s + x_d >= min(max(L, 2), 132), the length of the
+                                  reference's power tables (L = max_fragment_length) */
     SGPU_E_POSITIONS = -6,     /* loci not strictly increasing inside a chromosome */
     SGPU_E_COUNT_RANGE = -7,   /* internal int8/int32 range exceeded */
     SGPU_E_CONVERGENCE = -8    /* eigen-solver did not reach the tolerance (sgpu_spectral_embedding) */
@@ -205,6 +207,9 @@ int sgpu_similarity(sgpu_ctx *ctx, const sgpu_pileup *filtered, uint32_t num_cel
 int sgpu_counts_create(sgpu_ctx *ctx, uint32_t num_cells, sgpu_counts **out);
 int sgpu_counts_zero(sgpu_ctx *ctx, sgpu_counts *c);
 void sgpu_counts_free(sgpu_ctx *ctx, sgpu_counts *c);
+/* A failed accumulation (also _range) either leaves the counts object exactly as it was (an error found before any
+ * count was issued, such as SGPU_E_COUNT_RANGE of the GEMM path's first panel), or leaves a partial sum in it (e.g.
+ * SGPU_E_CLASS_RANGE): then every accumulation fails with SGPU_E_ARG until sgpu_counts_zero. */
 int sgpu_counts_accumulate(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *filtered,
                            uint32_t max_fragment_length, const uint32_t *group_id_to_pos,
                            uint32_t n_groups, double mutation_rate, double homozygous_rate,

@@ -895,11 +895,21 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
     s.n_tail_reads = lr.n_tail;
     s.n_span_splits = static_cast<int32_t>(std::min<uint64_t>(lr.n_span_splits, 0x7FFFFFFF));
     ctx->ms_stage = 0.f;
+    // Once first-order counts have been issued, a failure leaves a partial sum behind, possibly in every plane (the
+    // order-2 / order-3 atomics of the other pairs land too): later accumulations are then refused until
+    // sgpu_counts_zero, and that clears all planes. Failures before that point leave the object as it was.
+    auto issued = [c](int rc) {
+        if (rc != SGPU_OK) {
+            c->poisoned = true;
+            c->planes_dirty = N_PLANES;
+        }
+        return rc;
+    };
     EventTimer t_first(ctx->stream);
     if (path == SGPU_PATH_SCATTER) {
         SGPU_TRY(sgpu_link_dense_codes(ctx, filtered, &lr));
         SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // the atomics go to the planes a tensor kernel in flight adds to
-        SGPU_TRY(sgpu_scatter_pairs(ctx, filtered, lr, c, +1, false, &s.n_pairs_first));
+        SGPU_TRY(issued(sgpu_scatter_pairs(ctx, filtered, lr, c, +1, false, &s.n_pairs_first)));
         c->fresh = false;
     } else {
         // incl. the tail x tail correction. More than 127 reads of one cell at one locus do not fit int8: the first
@@ -910,7 +920,7 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
             s.path_used = SGPU_PATH_SCATTER;
             SGPU_TRY(sgpu_link_dense_codes(ctx, filtered, &lr));
             SGPU_TRY(sgpu_tensor_join(ctx, c->i32));
-            rc = sgpu_scatter_pairs(ctx, filtered, lr, c, +1, false, &s.n_pairs_first);
+            rc = issued(sgpu_scatter_pairs(ctx, filtered, lr, c, +1, false, &s.n_pairs_first));
             c->fresh = false;
         }
         SGPU_TRY(rc);
@@ -920,14 +930,14 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
     // second / third order planes, spill plane, histogram: none of them is touched by the first-order tensor kernel
     // that may still be running
     EventTimer t_multi(ctx->stream);
-    SGPU_TRY(sgpu_multilocus(ctx, filtered, lr, c, max_fragment_length, &s.n_pairs_multi));
+    SGPU_TRY(issued(sgpu_multilocus(ctx, filtered, lr, c, max_fragment_length, &s.n_pairs_multi)));
     t_multi.mark();
     s.ms_multi = t_multi.ms(); // the one host wait for the three phases
     s.ms_link = t_link.ms();
     s.ms_first_order = t_first.ms();
     // Tensor kernels retired during this call (with SECEDO_B200_ASYNC_GEMM=0: this call's own; otherwise mostly the one of
     // the batch before; sgpu_tensor_times returns what is left)
-    SGPU_TRY(sgpu_tensor_poll(ctx, false));
+    SGPU_TRY(issued(sgpu_tensor_poll(ctx, false)));
     s.ms_gemm = ctx->ms_syrk;
     s.gemm_launches = ctx->n_syrk;
     ctx->ms_syrk = 0.f;

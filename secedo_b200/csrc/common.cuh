@@ -390,6 +390,10 @@ int sgpu_multilocus(sgpu_ctx *ctx, const sgpu_pileup *p, LinkResult &lr, sgpu_co
                     uint32_t L, uint64_t *n_pairs_multi);
 
 // epilogue.cu
+// The log-probability power tables hold min(max(L, 2), LOGPROB_TBL) entries (similarity_matrix.cpp:42-67, capped like
+// the oracle's): a class with x_s + x_d >= that length has no LS / LD and is refused
+constexpr uint32_t LOGPROB_TBL = 132;
+inline uint32_t logprob_table_len(uint32_t L) { return L < 2 ? 2u : (L > LOGPROB_TBL ? LOGPROB_TBL : L); }
 struct FTable {
     double F[SGPU_MAX_CLASS * SGPU_MAX_CLASS]; // LD - LS, NaN where never needed
 };

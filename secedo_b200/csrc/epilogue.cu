@@ -16,7 +16,7 @@
 
 namespace {
 
-constexpr int TBL = 132; // power tables / Pascal rows kept (x_s + x_d <= 126 for classes < 64)
+constexpr int TBL = LOGPROB_TBL; // power tables / Pascal rows kept (x_s + x_d <= 126 for classes < 64)
 
 struct CacheTables {
     double pss[TBL], psd[TBL], pds[TBL], pdd[TBL];
@@ -37,10 +37,7 @@ void make_cache(CacheTables *c, double epsilon, double h, double theta, uint32_t
     const double p_same_same = 1 - p_same_diff;
     const double p_diff_same = 2 * (1 - theta) * theta / 3 + 2 * theta2 / 9;
     const double p_diff_diff = 1 - p_diff_same;
-    uint32_t n = max_read_size < 2 ? 2 : max_read_size;
-    if (n > TBL) {
-        n = TBL;
-    }
+    const uint32_t n = logprob_table_len(max_read_size);
     c->len = n;
     auto init = [n](double *arr, double v) {
         arr[0] = 1;

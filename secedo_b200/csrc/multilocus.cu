@@ -43,6 +43,7 @@ struct MultiArgs {
     uint32_t n_cells;
     uint64_t nn;
     uint32_t L;
+    uint32_t tbl_len;         // logprob_table_len(L): classes with x_s + x_d >= tbl_len have no log-likelihood
     int spill_only;           // second pass: record only the classes with x_s + x_d >= 4
     uint32_t min_order;       // 2: every multi-locus pair is enumerated here; 3: the pairs of order 2 come from
                               // the second-order GEMM, which counts every pair of order >= 3 C(x_s,2) / x_s x_d /
@@ -118,7 +119,7 @@ __global__ void __launch_bounds__(TB) multilocus_kernel(MultiArgs a) {
             if (xs + xd < a.min_order) {
                 continue;
             }
-            if (xs >= SGPU_MAX_CLASS || xd >= SGPU_MAX_CLASS || xs >= a.L || xd >= a.L) {
+            if (xs >= SGPU_MAX_CLASS || xd >= SGPU_MAX_CLASS || xs >= a.L || xd >= a.L || xs + xd >= a.tbl_len) {
                 atomicExch(a.err, SGPU_E_CLASS_RANGE);
                 continue;
             }
@@ -568,6 +569,9 @@ int sgpu_multilocus(sgpu_ctx *ctx, const sgpu_pileup *p, LinkResult &lr, sgpu_co
     const double n_pad = (c->n + 255) / 256 * 256.0;
     bool use_gemm = env ? env[0] == 'g'
                         : (c->n >= 512 && static_cast<double>(lr.n_multi) > 224.0 * n_pad / 8192.0 * static_cast<double>(p->n_loci));
+    if (logprob_table_len(L) <= 2) {
+        use_gemm = false; // no class of order 2 has a log-likelihood: the enumeration must see (and refuse) every such pair
+    }
     uint64_t hist2_before[3] = { 0, 0, 0 };
     if (use_gemm) {
         // the order-2 classes are not enumerated: their number is read off the class histogram afterwards
@@ -619,6 +623,7 @@ int sgpu_multilocus(sgpu_ctx *ctx, const sgpu_pileup *p, LinkResult &lr, sgpu_co
     a.n_cells = c->n;
     a.nn = c->nn;
     a.L = L;
+    a.tbl_len = logprob_table_len(L);
     a.spill_only = 0;
     a.min_order = use_gemm ? 3 : 2;
     a.max_order = d_max.p;
@@ -634,7 +639,9 @@ int sgpu_multilocus(sgpu_ctx *ctx, const sgpu_pileup *p, LinkResult &lr, sgpu_co
     SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[2], d_err.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     SGPU_CUDA(ctx, cudaStreamSynchronize(st));
     if (static_cast<int>(ctx->h_scratch[2] & 0xFFFFFFFFu) != 0) {
-        return sgpu_fail(ctx, SGPU_E_CLASS_RANGE, "a read pair overlaps at >= %d loci (or >= max_fragment_length)", SGPU_MAX_CLASS);
+        return sgpu_fail(ctx, SGPU_E_CLASS_RANGE,
+                         "a read pair overlaps with x_s or x_d >= %d (or >= max_fragment_length), or x_s + x_d >= %u",
+                         SGPU_MAX_CLASS, logprob_table_len(L));
     }
     if (n_pairs_multi) {
         *n_pairs_multi = ctx->h_scratch[0];
