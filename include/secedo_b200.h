@@ -303,7 +303,9 @@ int sgpu_output_wait(sgpu_ctx *ctx);
  * share is written (returned in *device_out). All ranks must have agreed on the layout (sgpu_counts_set_layout) and
  * finished accumulating before any of them calls sgpu_slab_raw. peer_spill: the fp64 spill planes of the GPUs (read
  * pairs that overlap at >= 4 loci; sgpu_counts_set_layout with want_spill on every rank once one of them has one), or
- * NULL when no GPU holds one; they are added in the order of the array (fp64: agrees with one GPU to rounding). */
+ * NULL when no GPU holds one; they are added in the order of the array (fp64: agrees with one GPU to rounding). Entries
+ * of GPUs without a spill plane may be NULL. Like sgpu_similarity_finalize, it fails with SGPU_E_ARG when c holds a
+ * spill plane and the likelihood parameters differ from those c was accumulated with. */
 int sgpu_slab_raw(sgpu_ctx *ctx, sgpu_counts *c, const int32_t *const *peer_planes, const double *const *peer_spill,
                   uint32_t n_peers, uint32_t slab, uint32_t n_slabs, uint32_t max_fragment_length, double mutation_rate,
                   double homozygous_rate, double seq_error_rate, double **extrema);

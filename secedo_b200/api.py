@@ -439,13 +439,16 @@ class Counts:
         self.ctx.check(self.ctx._lib.sgpu_counts_ipc_handle(self.ctx._h, self._h, 1 if spill else 0, buf))
         return buf.raw
 
-    def _peer_array(self, peer_planes: Sequence[int]):
-        return (C.c_void_p * len(peer_planes))(*[C.c_void_p(int(p)) for p in peer_planes])
+    def _peer_array(self, peer_planes: Sequence[Optional[int]]):
+        """device pointers as a C array; None is a null pointer (a GPU without a spill plane)"""
+        return (C.c_void_p * len(peer_planes))(*[C.c_void_p(None if p is None else int(p)) for p in peer_planes])
 
     def slab_raw(self, peer_planes: Sequence[int], slab: int, n_slabs: int, max_fragment_length: int, mutation_rate: float,
-                 homozygous_rate: float, seq_error_rate: float, peer_spill: Optional[Sequence[int]] = None) -> int:
+                 homozygous_rate: float, seq_error_rate: float, peer_spill: Optional[Sequence[Optional[int]]] = None) -> int:
         """Sum the planes of all GPUs (device pointers valid on this GPU, own planes included) over this GPU's share of
-        the tiles and transform them; returns the device pointer of {-min, max} (2 doubles) of the share."""
+        the tiles and transform them; returns the device pointer of {-min, max} (2 doubles) of the share. ``peer_spill``:
+        one entry per peer, None for a GPU without a spill plane."""
+        assert peer_spill is None or len(peer_spill) == len(peer_planes), "one spill entry per peer"
         ext = C.c_void_p()
         self.ctx.check(self.ctx._lib.sgpu_slab_raw(self.ctx._h, self._h, self._peer_array(peer_planes),
                                                    self._peer_array(peer_spill) if peer_spill else None, len(peer_planes),

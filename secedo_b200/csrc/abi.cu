@@ -1272,6 +1272,11 @@ int sgpu_slab_raw(sgpu_ctx *ctx, sgpu_counts *c, const int32_t *const *peer_plan
                   double homozygous_rate, double seq_error_rate, double **extrema) {
     SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
     SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    // the spill plane holds G(x_s, x_d) evaluated with the accumulation's parameters; F and G must not be mixed
+    if (c->have_params && c->spill
+        && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
+        return sgpu_fail(ctx, SGPU_E_ARG, "slab epilogue called with likelihood parameters different from accumulate");
+    }
     return sgpu_slab_raw_impl(ctx, c, peer_planes, peer_spill, n_peers, slab, n_slabs, max_fragment_length, mutation_rate,
                               homozygous_rate, seq_error_rate, extrema);
 }
