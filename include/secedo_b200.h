@@ -388,8 +388,8 @@ int sgpu_laplacian(sgpu_ctx *ctx, const double *similarity, uint32_t n, double *
  * :166-171, :218, :236): the k smallest eigenvalues (ascending) and their eigenvectors, eigenvectors[i * n + r] =
  * component r of eigenvector i (Armadillo's column-major layout), unit norm, the component of largest magnitude
  * positive (LAPACK's sign is arbitrary). Residuals |L v - lambda v| <= tol (0 selects 1e-10). 1 <= k <= 32,
- * n >= 2 * block (block = 16 for k <= 8, 32 for k <= 16, else 64); similarities must be non-negative. The full
- * decomposition of the reference is not computed: nothing else of it is used. */
+ * n >= 2 * block (block = 16 for k <= 8, 32 for k <= 16, else 64); similarities must be non-negative. All n
+ * eigenvalues (the reference's sim_mat_eigenvalues CSV) come from sgpu_laplacian_eigenvalues. */
 int sgpu_spectral_embedding(sgpu_ctx *ctx, const double *similarity, uint32_t n, uint32_t k, double tol,
                             double *eigenvalues, double *eigenvectors, sgpu_spectral_stats *stats);
 /* sgpu_similarity_finalize followed by sgpu_spectral_embedding without the matrix leaving the device
@@ -398,6 +398,31 @@ int sgpu_similarity_finalize_spectral(sgpu_ctx *ctx, sgpu_counts *c, uint32_t ma
                                       double mutation_rate, double homozygous_rate, double seq_error_rate,
                                       int normalization, double *out, uint32_t k, double tol, double *eigenvalues,
                                       double *eigenvectors, sgpu_stats *stats, sgpu_spectral_stats *spectral_stats);
+/* ---- every eigenvalue of the Laplacian (the sim_mat_eigenvalues CSV of spectral_clustering.cpp:141-143) ---------- */
+typedef struct sgpu_eigenvalue_stats {
+    uint64_t launches;     /* all kernels of the call */
+    float ms_laplacian;    /* degrees + scaling */
+    float ms_tridiagonal;  /* blocked Householder reduction to tridiagonal form */
+    float ms_bisection;    /* Sturm bisection of the tridiagonal matrix */
+    uint64_t bytes_matvec; /* bytes the symmetric matrix-vector products must read: one triangle of the trailing
+                              matrix per column, 8 (n-1) n (n+1) / 6 */
+    uint32_t reserved;
+} sgpu_eigenvalue_stats;
+/* All n eigenvalues of laplacian(similarity) = I - D^-1/2 A D^-1/2, ascending, as arma::eig_sym returns them
+ * (spectral_clustering.cpp:127-138), computed on the device in fp64: B = D^-1/2 A D^-1/2 is reduced to tridiagonal
+ * form by blocked Householder reflections (LAPACK DSYTRD) and the eigenvalues of B are found by bisection on Sturm
+ * counts (DSTEBZ); eigenvalues[i] = 1 - (the i-th largest of B). similarity: host n x n, symmetric, non-negative
+ * (a negative or NaN degree is SGPU_E_ARG); a cell of degree 0 has eigenvalue 1, an all-zero matrix n ones. The
+ * device holds 8 ld^2 bytes of working copy (ld = n rounded up to 64). Bit-reproducible. */
+int sgpu_laplacian_eigenvalues(sgpu_ctx *ctx, const double *similarity, uint32_t n, double *eigenvalues,
+                               sgpu_eigenvalue_stats *stats);
+/* sgpu_similarity_finalize followed by sgpu_laplacian_eigenvalues without the matrix leaving the device (out may be
+ * NULL: the n x n matrix is then not downloaded). Refuses, like sgpu_similarity_finalize, likelihood parameters other
+ * than the accumulation's when c holds a spill plane. */
+int sgpu_similarity_finalize_eigenvalues(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragment_length,
+                                         double mutation_rate, double homozygous_rate, double seq_error_rate,
+                                         int normalization, double *out, double *eigenvalues, sgpu_stats *stats,
+                                         sgpu_eigenvalue_stats *eig_stats);
 /* test hook of the block product kernel: out = alpha M X + beta X + gamma W, M n x n symmetric, blocks n x width
  * row-major (width 8, 16, 32 or 64), all on the host */
 int sgpu_spectral_matvec(sgpu_ctx *ctx, const double *M, uint32_t n, int width, const double *X, const double *W,

@@ -54,6 +54,16 @@ class SpectralStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class EigenvalueStats(C.Structure):
+    _fields_ = [
+        ("launches", C.c_uint64), ("ms_laplacian", C.c_float), ("ms_tridiagonal", C.c_float), ("ms_bisection", C.c_float),
+        ("bytes_matvec", C.c_uint64), ("reserved", C.c_uint32),
+    ]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
 class SynthParams(C.Structure):
     _fields_ = [
         ("n_cells", C.c_uint32), ("n_chr", C.c_uint32), ("loci_per_chr", C.c_uint32), ("n_clones", C.c_uint32),
@@ -142,6 +152,9 @@ SIGNATURES = {
     "sgpu_similarity_finalize_spectral": (C.c_int, [_vp, _vp, C.c_uint32, C.c_double, C.c_double, C.c_double, C.c_int, _vp,
                                                     C.c_uint32, C.c_double, _vp, _vp, C.POINTER(Stats),
                                                     C.POINTER(SpectralStats)]),
+    "sgpu_laplacian_eigenvalues": (C.c_int, [_vp, _vp, C.c_uint32, _vp, C.POINTER(EigenvalueStats)]),
+    "sgpu_similarity_finalize_eigenvalues": (C.c_int, [_vp, _vp, C.c_uint32, C.c_double, C.c_double, C.c_double, C.c_int, _vp,
+                                                       _vp, C.POINTER(Stats), C.POINTER(EigenvalueStats)]),
     "sgpu_spectral_matvec": (C.c_int, [_vp, _vp, C.c_uint32, C.c_int, _vp, _vp, C.c_double, C.c_double, C.c_double, _vp]),
 }
 

@@ -22,7 +22,7 @@ from typing import Optional, Sequence, Tuple, Union
 import numpy as np
 
 from . import _lib
-from ._lib import NORMALIZATIONS, PATHS, SgpuError, SpectralStats, Stats
+from ._lib import NORMALIZATIONS, PATHS, EigenvalueStats, SgpuError, SpectralStats, Stats
 from .pileup import NO_POS, Pileup
 
 
@@ -555,6 +555,24 @@ class Counts:
         d["ms_epilogue"] = st.ms_epilogue
         return ev, np.ascontiguousarray(vec.T), d, out
 
+    def finalize_eigenvalues(self, max_fragment_length: int, mutation_rate: float, homozygous_rate: float,
+                             seq_error_rate: float, normalization: str, want_matrix: bool = False):
+        """Epilogue + Laplacian + all n eigenvalues (ascending) without the matrix leaving HBM (the
+        ``sim_mat_eigenvalues`` CSV of ``spectral_clustering``, spectral_clustering.cpp:127-143).
+        Returns (eigenvalues[n], stats, matrix or None)."""
+        if normalization not in NORMALIZATIONS:
+            raise ValueError("Invalid normalization: " + str(normalization))
+        n = self.num_cells
+        out = np.zeros((n, n), np.float64) if want_matrix else None
+        ev = np.zeros(n, np.float64)
+        st, es = Stats(), EigenvalueStats()
+        self.ctx.check(self.ctx._lib.sgpu_similarity_finalize_eigenvalues(
+            self.ctx._h, self._h, int(max_fragment_length), float(mutation_rate), float(homozygous_rate),
+            float(seq_error_rate), NORMALIZATIONS[normalization], _ptr(out), _ptr(ev), C.byref(st), C.byref(es)))
+        d = es.as_dict()
+        d["ms_epilogue"] = st.ms_epilogue
+        return ev, d, out
+
     def free(self) -> None:
         if self._h and self.ctx._h:
             self.ctx._lib.sgpu_counts_free(self.ctx._h, self._h)
@@ -672,6 +690,18 @@ def spectral_embedding(similarity: np.ndarray, k: int = 7, tol: float = 0.0, ctx
     return (ev, vec, sp.as_dict()) if return_stats else (ev, vec)
 
 
+def laplacian_eigenvalues(similarity: np.ndarray, ctx: Optional[Context] = None, return_stats: bool = False):
+    """All eigenvalues of ``laplacian(similarity)``, ascending, as ``arma::eig_sym`` returns them
+    (spectral_clustering.cpp:127-143): Householder tridiagonalisation and Sturm bisection on the device, in fp64."""
+    ctx = ctx or default_context()
+    a = np.ascontiguousarray(similarity, np.float64)
+    assert a.ndim == 2 and a.shape[0] == a.shape[1]
+    ev = np.zeros(a.shape[0], np.float64)
+    es = EigenvalueStats()
+    ctx.check(ctx._lib.sgpu_laplacian_eigenvalues(ctx._h, _ptr(a), a.shape[0], _ptr(ev), C.byref(es)))
+    return (ev, es.as_dict()) if return_stats else ev
+
+
 def spectral_matvec(m: np.ndarray, x: np.ndarray, w: Optional[np.ndarray] = None, alpha: float = 1.0, beta: float = 0.0,
                     gamma: float = 0.0, ctx: Optional[Context] = None) -> np.ndarray:
     """Test hook of the block product kernel of the eigen-solver: alpha M X + beta X + gamma W."""
@@ -686,4 +716,5 @@ def spectral_matvec(m: np.ndarray, x: np.ndarray, w: Optional[np.ndarray] = None
 
 
 __all__ = ["Context", "DevicePileup", "Filter", "Counts", "compute_similarity_matrix", "log_probs", "default_context", "expectation_maximization", "laplacian", "spectral_embedding",
+           "laplacian_eigenvalues",
            "NO_POS", "SgpuError"]

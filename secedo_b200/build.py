@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "obj")
 LIB = os.path.join(HERE, "libsecedo_b200.so")
-SOURCES = ["abi.cu", "scan.cu", "filter.cu", "reads.cu", "scatter.cu", "multilocus.cu", "epilogue.cu", "gemm.cu", "synth.cu", "ingest.cu", "spectral.cu", "em.cu", "multi.cu"]
+SOURCES = ["abi.cu", "scan.cu", "filter.cu", "reads.cu", "scatter.cu", "multilocus.cu", "epilogue.cu", "gemm.cu", "synth.cu", "ingest.cu", "spectral.cu", "eigenvalues.cu", "em.cu", "multi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false",
          "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

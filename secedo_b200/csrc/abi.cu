@@ -1447,6 +1447,38 @@ int sgpu_similarity_finalize_spectral(sgpu_ctx *ctx, sgpu_counts *c, uint32_t ma
     return rc;
 }
 
+int sgpu_laplacian_eigenvalues(sgpu_ctx *ctx, const double *similarity, uint32_t n, double *eigenvalues,
+                               sgpu_eigenvalue_stats *stats) {
+    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    DevBuf<double> d;
+    SGPU_TRY(upload_matrix(ctx, similarity, n, d));
+    return sgpu_eigenvalues_device(ctx, d.p, n, eigenvalues, stats);
+}
+
+int sgpu_similarity_finalize_eigenvalues(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragment_length, double mutation_rate,
+                                         double homozygous_rate, double seq_error_rate, int normalization, double *out,
+                                         double *eigenvalues, sgpu_stats *stats, sgpu_eigenvalue_stats *eig_stats) {
+    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
+    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (c->have_params && c->spill
+        && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
+        return sgpu_fail(ctx, SGPU_E_ARG, "finalize called with likelihood parameters different from accumulate");
+    }
+    double *d_mat = nullptr;
+    EventTimer t(ctx->stream);
+    SGPU_TRY(sgpu_epilogue(ctx, c, max_fragment_length, mutation_rate, homozygous_rate, seq_error_rate, normalization, out, &d_mat));
+    const float ms = t.stop();
+    if (stats) {
+        stats->ms_epilogue = ms;
+    }
+    if (!d_mat) {
+        return sgpu_fail(ctx, SGPU_E_ARG, "eigenvalues: empty similarity matrix");
+    }
+    const int rc = sgpu_eigenvalues_device(ctx, d_mat, c->n, eigenvalues, eig_stats);
+    sgpu_dev_free(ctx, d_mat);
+    return rc;
+}
+
 int sgpu_spectral_matvec(sgpu_ctx *ctx, const double *M, uint32_t n, int width, const double *X, const double *W, double alpha,
                          double beta, double gamma, double *out) {
     SGPU_CUDA(ctx, cudaSetDevice(ctx->device));

@@ -416,6 +416,11 @@ int sgpu_em_impl(sgpu_ctx *ctx, const sgpu_pileup *p, const uint32_t *h_id_to_po
 int sgpu_spectral_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t k, double tol, double *h_evals,
                          double *h_evecs, sgpu_spectral_stats *stats);
 int sgpu_laplacian_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, double *h_out);
+// B = D^-1/2 A D^-1/2 (minus v0 v0^T when d_v0 is given) into M, ld x ld with zero padding; see spectral.cu
+int sgpu_scaled_similarity(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t ld, DevBuf<double> &M, DevBuf<double> *d_v0,
+                           bool *all_zero);
+// eigenvalues.cu: all n eigenvalues of laplacian(A), ascending, into the host array h_evals
+int sgpu_eigenvalues_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, double *h_evals, sgpu_eigenvalue_stats *stats);
 int sgpu_spectral_matvec_host(sgpu_ctx *ctx, const double *h_M, uint32_t n, int width, const double *h_X, const double *h_W,
                               double alpha, double beta, double gamma, double *h_out);
 // device table of G(s,d) = F(s,d) - s F(1,0) - d F(0,1) for the spill plane (SGPU_MAX_CLASS^2 doubles)

@@ -450,8 +450,9 @@ __global__ void rowsum_kernel(const double *__restrict__ A, uint32_t n, double *
     }
 }
 
-// M[r][c] = s_r s_c A[r][c] - v0_r v0_c for r, c < n, zero in the padding (ld x ld); with lap != 0 instead the
-// reference's Laplacian itself: out[r][c] = (r == c) - s_r s_c A[r][c], n x n (spectral_clustering.cpp:44-50)
+// M[r][c] = s_r s_c A[r][c] - v0_r v0_c for r, c < n (without the v0 term when v0 is null), zero in the padding
+// (ld x ld); with lap != 0 instead the reference's Laplacian itself: out[r][c] = (r == c) - s_r s_c A[r][c], n x n
+// (spectral_clustering.cpp:44-50)
 __global__ void scale_kernel(const double *__restrict__ A, uint32_t n, uint32_t ld, const double *__restrict__ s,
                              const double *__restrict__ v0, int lap, double *__restrict__ out) {
     const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
@@ -467,7 +468,10 @@ __global__ void scale_kernel(const double *__restrict__ A, uint32_t n, uint32_t 
     }
     double v = 0.0;
     if (r < n && c < n) {
-        v = (s[r] * s[c]) * A[static_cast<size_t>(r) * n + c] - v0[r] * v0[c];
+        v = (s[r] * s[c]) * A[static_cast<size_t>(r) * n + c];
+        if (v0) {
+            v -= v0[r] * v0[c];
+        }
     }
     out[static_cast<size_t>(r) * ld + c] = v;
 }
@@ -793,6 +797,49 @@ int block_width_for(uint32_t k) {
 
 } // namespace
 
+// B = D^-1/2 A D^-1/2 of the reference's laplacian() (spectral_clustering.cpp:33-52), L = I - B, into M (allocated
+// here, ld x ld, zero padding); with d_v0 the unit vector v0 = sqrt(d / sum d) (B v0 = v0) is stored there and M = B -
+// v0 v0^T. A cell of degree 0 gets scale 0 (its row of L is the unit row, eigenvalue 1); a negative or NaN degree is
+// SGPU_E_ARG (the reference would take the square root of a negative number). An all-zero A (L = I) sets *all_zero and
+// allocates nothing.
+int sgpu_scaled_similarity(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t ld, DevBuf<double> &M, DevBuf<double> *d_v0,
+                           bool *all_zero) {
+    cudaStream_t st = ctx->stream;
+    DevBuf<double> d_deg, d_s;
+    SGPU_CUDA(ctx, d_deg.alloc(n, ctx));
+    SGPU_LAUNCH(ctx, (rowsum_kernel<<<(n + 7) / 8, 256, 0, st>>>(d_A, n, d_deg.p)));
+    std::vector<double> deg(n), sc(n);
+    SGPU_CUDA(ctx, cudaMemcpyAsync(deg.data(), d_deg.p, n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+    double total = 0.0;
+    for (uint32_t r = 0; r < n; ++r) {
+        if (!(deg[r] >= 0.0)) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "spectral: cell %u has degree %g (similarities must be non-negative)", r, deg[r]);
+        }
+        sc[r] = deg[r] == 0.0 ? 0.0 : 1.0 / std::sqrt(deg[r]);
+        total += deg[r];
+    }
+    *all_zero = !(total > 0.0);
+    if (*all_zero) {
+        return SGPU_OK;
+    }
+    // stream-ordered copies from pageable memory return after staging the source: the locals may go
+    SGPU_CUDA(ctx, d_s.alloc(n, ctx));
+    SGPU_CUDA(ctx, cudaMemcpyAsync(d_s.p, sc.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (d_v0) {
+        std::vector<double> v0(n);
+        for (uint32_t r = 0; r < n; ++r) {
+            v0[r] = std::sqrt(deg[r] / total);
+        }
+        SGPU_CUDA(ctx, d_v0->alloc(n, ctx));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(d_v0->p, v0.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    SGPU_CUDA(ctx, M.alloc(static_cast<size_t>(ld) * ld, ctx));
+    SGPU_LAUNCH(ctx, (scale_kernel<<<dim3((ld + 255) / 256, ld), 256, 0, st>>>(d_A, n, ld, d_s.p, d_v0 ? d_v0->p : nullptr, 0, M.p)));
+    SGPU_CUDA(ctx, cudaGetLastError());
+    return SGPU_OK;
+}
+
 // d_A: n x n similarity matrix on the device (row-major, symmetric, zero diagonal)
 int sgpu_spectral_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t k, double tol, double *h_evals,
                          double *h_evecs, sgpu_spectral_stats *stats) {
@@ -835,23 +882,10 @@ int sgpu_spectral_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t 
     S.kq = kq;
 
     // ---- Laplacian: degrees, scaling, trivial eigenvector (spectral_clustering.cpp:33-52) ----
-    DevBuf<double> d_deg, d_s, d_v0;
-    SGPU_CUDA(ctx, d_deg.alloc(n, ctx));
-    SGPU_CUDA(ctx, d_s.alloc(n, ctx));
-    SGPU_CUDA(ctx, d_v0.alloc(n, ctx));
-    SGPU_LAUNCH(ctx, (rowsum_kernel<<<(n + 7) / 8, 256, 0, st>>>(d_A, n, d_deg.p)));
-    std::vector<double> deg(n), sc(n), v0(n);
-    SGPU_CUDA(ctx, cudaMemcpyAsync(deg.data(), d_deg.p, n * sizeof(double), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-    double total = 0.0;
-    for (uint32_t r = 0; r < n; ++r) {
-        if (!(deg[r] >= 0.0)) { // the reference would take the square root of a negative number
-            return sgpu_fail(ctx, SGPU_E_ARG, "spectral: cell %u has degree %g (similarities must be non-negative)", r, deg[r]);
-        }
-        sc[r] = deg[r] == 0.0 ? 0.0 : 1.0 / std::sqrt(deg[r]);
-        total += deg[r];
-    }
-    if (!(total > 0.0)) {
+    DevBuf<double> d_v0;
+    bool all_zero = false;
+    SGPU_TRY(sgpu_scaled_similarity(ctx, d_A, n, ld, S.M, &d_v0, &all_zero));
+    if (all_zero) {
         // all-zero similarity (tests/test_spectral_clustering.cpp:186-196 exercises it): the reference's Laplacian is
         // the identity, whose LAPACK decomposition is eigenvalue 1 with the unit vectors
         for (uint32_t i = 0; i < k; ++i) {
@@ -868,14 +902,6 @@ int sgpu_spectral_device(sgpu_ctx *ctx, const double *d_A, uint32_t n, uint32_t 
         }
         return SGPU_OK;
     }
-    for (uint32_t r = 0; r < n; ++r) {
-        v0[r] = std::sqrt(deg[r] / total);
-    }
-    SGPU_CUDA(ctx, cudaMemcpyAsync(d_s.p, sc.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(d_v0.p, v0.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
-    SGPU_CUDA(ctx, S.M.alloc(static_cast<size_t>(ld) * ld, ctx));
-    SGPU_LAUNCH(ctx, (scale_kernel<<<dim3((ld + 255) / 256, ld), 256, 0, st>>>(d_A, n, ld, d_s.p, d_v0.p, 0, S.M.p)));
-    SGPU_CUDA(ctx, cudaGetLastError());
     SGPU_CUDA(ctx, cudaEventRecord(t1, st));
 
     // ---- locked eigenpairs: column 0 = v0 (eigenvalue 1 of B); the iteration itself is spectral_host.hpp ----
