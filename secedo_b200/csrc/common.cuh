@@ -361,14 +361,9 @@ int sgpu_is_significant_impl(sgpu_ctx *ctx, const uint16_t *h_counts4, uint64_t 
 struct RangeSpec {
     const uint32_t *own_pos_begin, *own_pos_end, *tail_position;
 };
-struct CutoffQuery { // suffix mode: only the cutoff is computed (host arrays, one entry per chromosome)
-    const uint8_t *whole;      // in: the chromosome is complete (not just its end)
-    uint32_t *tail_position;   // out
-    uint8_t *resolved;         // out
-};
 int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uint32_t L,
                     const uint32_t *h_group_id_to_pos, uint32_t n_groups, uint32_t num_threads,
-                    LinkResult *out, const RangeSpec *range = nullptr, const CutoffQuery *cutq = nullptr);
+                    LinkResult *out, const RangeSpec *range = nullptr);
 // cutoff K of chromosomes of which only the END is given (suffix): per chromosome the position from which reads are
 // tail reads, and whether the suffix was long enough to decide it
 int sgpu_cutoff_from_suffix(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t L, uint32_t num_threads, const uint8_t *h_whole,

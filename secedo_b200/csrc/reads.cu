@@ -1052,197 +1052,251 @@ __global__ void __launch_bounds__(TB) sp_codes_kernel(const uint32_t *__restrict
 
 unsigned blocks_for(uint64_t n) { return static_cast<unsigned>(ceil_div_u64(n ? n : 1, TB)); }
 
-} // namespace
+bool env_is_1(const char *name) {
+    const char *v = getenv(name);
+    return v && v[0] == '1';
+}
 
-int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uint32_t L,
-                    const uint32_t *h_group_id_to_pos, uint32_t n_groups, uint32_t num_threads,
-                    LinkResult *out, const RangeSpec *range, const CutoffQuery *cutq) {
-    cudaStream_t st = ctx->stream;
-    const uint64_t E = p->n_entries, P = p->n_loci;
-    if (E >= 0x7FFFFFF0ull || P >= 0x7FFFFFF0ull) {
-        return sgpu_fail(ctx, SGPU_E_ARG, "more than 2^31 entries in one call: pass the pileup in batches of chromosomes");
-    }
-    if (p->n_chr > 255) {
-        return sgpu_fail(ctx, SGPU_E_ARG, "more than 255 chromosomes in one call");
-    }
-    if (num_threads == 0) {
-        return sgpu_fail(ctx, SGPU_E_ARG, "num_threads must be >= 1");
-    }
-    if (num_cells >= (1u << 27)) {
-        return sgpu_fail(ctx, SGPU_E_ARG, "num_cells too large");
-    }
-    out->n_reads = out->n_multi = out->n_dropped = out->n_tail = out->n_special = out->n_tail_loci = out->n_own = 0;
-    out->ranged = range != nullptr;
-    out->n_groups = n_groups;
-    out->num_cells = num_cells;
-    SGPU_CUDA(ctx, out->gmap.alloc(n_groups ? n_groups : 1, ctx));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(out->gmap.p, h_group_id_to_pos, n_groups * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    out->gmap_identity = n_groups <= num_cells;
-    for (uint32_t g = 0; g < n_groups && out->gmap_identity; ++g) {
-        out->gmap_identity = h_group_id_to_pos[g] == g;
-    }
-    const uint64_t W = E / 32 + 1; // bitmap words
-    SGPU_CUDA(ctx, out->sp_bits.alloc(W, ctx));
-    SGPU_CUDA(ctx, cudaMemsetAsync(out->sp_bits.p, 0, W * sizeof(uint32_t), st));
-    SGPU_CUDA(ctx, out->lchr.alloc(P ? P : 1, ctx));
-    SGPU_CUDA(ctx, out->tail_locus.alloc(p->n_chr ? p->n_chr : 1, ctx));
-    if (E == 0 || P == 0) {
-        // nothing to link; tail_locus = end of every chromosome
-        if (p->n_chr) {
-            SGPU_CUDA(ctx, cudaMemcpyAsync(out->tail_locus.p, p->d_chr_ptr + 1, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
-        }
-        SGPU_CUDA(ctx, out->tail_loci.alloc(1, ctx));
-        return SGPU_OK;
-    }
+struct WinGeometry {
+    uint32_t n_ring, slots, id_cap;
+    size_t smem;
+    bool use_window; // false: the global hash
+};
 
-    SGPU_TRACE(ctx, "link: enter");
-    DevBuf<int> d_err;            // [0] error code, [1] "third sweep still changed something"
-    DevBuf<unsigned int> d_maxn;
-    DevBuf<WinCounters> d_ctr;
-    DevBuf<unsigned long long> d_stats;
-    DevBuf<uint64_t> readbase, n_tail_reads;
-    SGPU_CUDA(ctx, d_err.alloc(2, ctx));
-    SGPU_CUDA(ctx, d_maxn.alloc(1, ctx));
-    SGPU_CUDA(ctx, d_ctr.alloc(1, ctx));
-    SGPU_CUDA(ctx, d_stats.alloc(2, ctx));
-    SGPU_CUDA(ctx, readbase.alloc(P + 1, ctx));
-    SGPU_CUDA(ctx, n_tail_reads.alloc(p->n_chr, ctx));
-    SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, 2 * sizeof(int), st));
-    SGPU_CUDA(ctx, cudaMemsetAsync(d_maxn.p, 0, sizeof(unsigned int), st));
-    SGPU_CUDA(ctx, cudaMemsetAsync(d_ctr.p, 0, sizeof(WinCounters), st));
-    SGPU_CUDA(ctx, cudaMemsetAsync(d_stats.p, 0, 2 * sizeof(unsigned long long), st));
-
-    SGPU_LAUNCH(ctx, (locus_meta_kernel<<<blocks_for(P), TB, 0, st>>>(p->d_row_ptr, p->d_position, p->d_chr_ptr, p->n_chr, P,
-                                                                       out->lchr.p, d_maxn.p, d_err.p)));
-    uint32_t max_n = p->max_row;
-    if (max_n == 0) {
-        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_maxn.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-        max_n = static_cast<uint32_t>(ctx->h_scratch[0] & 0xFFFFFFFFu);
-        p->max_row = max_n; // cached: the pileup is immutable
-    }
-
-    SGPU_TRACE(ctx, "link: allocs+meta");
-    // ---- links between entries of one read -----------------------------------------------------------
-    // table geometry: slots >= 3 x the largest locus if shared memory allows, never below 1.25 x; the ring holds the
-    // read ids of WIN_RING loci (each slot: the largest locus + up to 3 elements of alignment offset)
-    const uint32_t id_cap = (max_n + 3 + 3) & ~3u;
-    auto pow2_slots = [&](unsigned long long want) {
+// link_window's shared memory for loci of up to max_n entries: table slots >= 3 x the largest locus if shared memory
+// allows, never below 1.25 x (else the global hash); the ring holds the read ids of n_ring loci (each slot: the largest
+// locus + up to 3 elements of alignment offset)
+WinGeometry window_geometry(uint32_t max_n, bool force_global) {
+    WinGeometry g{ WIN_RING, 1024, (max_n + 3 + 3) & ~3u, 0, false };
+    auto pow2_slots = [](unsigned long long want) {
         uint32_t sl = 1024;
         while (sl < want && sl < 65536) {
             sl <<= 1;
         }
         return sl;
     };
-    uint32_t n_ring = WIN_RING, slots = 1024;
-    auto win_smem = [&](uint32_t s) {
-        return static_cast<size_t>(n_ring) * id_cap * 4 + REC_BUF * sizeof(uint2) + static_cast<size_t>(s) * 2;
+    auto win_smem = [&]() {
+        return static_cast<size_t>(g.n_ring) * g.id_cap * 4 + REC_BUF * sizeof(uint2) + static_cast<size_t>(g.slots) * 2;
     };
     // preference: a ring of at least two loci (no exposed global latency per owner) before a sparse table (fewer second
     // probes); huge loci (cfg5: 20 000 reads) end at one resident locus and the largest table that fits. A CTA takes a
     // whole SM's shared memory: a geometry that fits beside the previous batch's tensor kernel (60 KB: one CTA per SM, a
     // denser table) was slower than letting link_window wait for it (profiles/r2_overlap_probes.txt).
-    auto choose_geometry = [&]() {
-        const uint32_t s_full = pow2_slots(3ull * max_n), s_half = std::min(s_full, pow2_slots(2ull * max_n));
-        const uint32_t cand[4][2] = { { WIN_RING, s_full }, { 2, s_full }, { WIN_RING, s_half }, { 2, s_half } };
-        for (const auto &cd : cand) {
-            n_ring = cd[0];
-            slots = cd[1];
-            if (win_smem(slots) <= WIN_SMEM_LIMIT) {
-                return true;
-            }
-        }
-        n_ring = 1;
-        slots = s_full;
-        while (slots > 1024 && win_smem(slots) > WIN_SMEM_LIMIT) {
-            slots >>= 1;
-        }
-        return win_smem(slots) <= WIN_SMEM_LIMIT && 4ull * slots >= 5ull * max_n;
-    };
-    const bool window_fits = choose_geometry();
-    // SECEDO_B200_FORCE_GLOBAL_HASH=1 forces the large-locus path (tests)
-    const char *force_global = getenv("SECEDO_B200_FORCE_GLOBAL_HASH");
-    const bool use_window = max_n <= WIN_MAX_ENTRIES && window_fits && 4ull * slots >= 5ull * max_n
-            && !(force_global && force_global[0] == '1');
-    const unsigned locus_grid = static_cast<unsigned>(std::min<uint64_t>(P, static_cast<uint64_t>(ctx->sm_count) * 16));
-
-    DevBuf<uint2> links;
-    uint64_t cap = std::max<uint64_t>(E / 8, 4096);
-    uint64_t NL = 0;
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        SGPU_CUDA(ctx, links.alloc(cap, ctx));
-        SGPU_CUDA(ctx, cudaMemsetAsync(d_ctr.p, 0, sizeof(WinCounters), st));
-        if (use_window) {
-            const size_t smem = win_smem(slots);
-            SGPU_CUDA(ctx, cudaFuncSetAttribute(link_window_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-            const unsigned per_sm = static_cast<unsigned>(std::max<size_t>(1, std::min<size_t>(4, (224 * 1024) / (smem + 2560))));
-            // contiguous ranges of owner loci, one per CTA, all CTAs resident at once
-            const uint64_t want = std::min<uint64_t>(P, static_cast<uint64_t>(ctx->sm_count) * per_sm);
-            const uint32_t loci_per_cta = static_cast<uint32_t>(ceil_div_u64(P, want));
-            const unsigned wgrid = static_cast<unsigned>(ceil_div_u64(P, loci_per_cta));
-            // this kernel never fits beside the tensor kernel of the previous batch, so it and everything behind it on the
-            // stream run alone: back to the default shared-memory / L1 split
-            SGPU_TRY(sgpu_cache_preference(ctx, false));
-            SGPU_LAUNCH(ctx, (link_window_kernel<<<wgrid, WIN_THREADS, smem, st>>>(p->d_row_ptr, p->d_position,
-                                                                                  p->d_read_id ? p->d_read_id : p->view_read_id,
-                                                                                  p->d_read_id ? nullptr : p->view_off, out->lchr.p, P, L,
-                                                                                  loci_per_cta, slots, id_cap, n_ring, links.p, cap, d_ctr.p)));
-        } else {
-            SGPU_TRY(sgpu_pileup_materialize(ctx, p)); // the global hash reads the ids by entry number
-            DevBuf<uint64_t> keys;
-            DevBuf<uint32_t> vals;
-            uint64_t hcap = 1024;
-            while (hcap < 2 * E) {
-                hcap <<= 1;
-            }
-            SGPU_CUDA(ctx, keys.alloc(hcap, ctx));
-            SGPU_CUDA(ctx, vals.alloc(hcap, ctx));
-            SGPU_CUDA(ctx, cudaMemsetAsync(keys.p, 0xFF, hcap * sizeof(uint64_t), st));
-            SGPU_CUDA(ctx, cudaMemsetAsync(vals.p, 0xFF, hcap * sizeof(uint32_t), st));
-            SGPU_LAUNCH(ctx, (ghash_insert_kernel<<<locus_grid, TB, 0, st>>>(p->d_row_ptr, p->d_read_id, out->lchr.p, P, keys.p, vals.p, hcap - 1)));
-            SGPU_LAUNCH(ctx, (ghash_emit_kernel<<<locus_grid, TB, 0, st>>>(p->d_row_ptr, p->d_read_id, out->lchr.p, P, keys.p, vals.p, hcap - 1,
-                                                                            links.p, cap, d_ctr.p)));
-        }
-        SGPU_CUDA(ctx, cudaGetLastError());
-        // the previous batch's tensor kernel, if its launch has been held back: behind the dense linking pass, beside
-        // everything that follows (sgpu_tensor_flush)
-        SGPU_TRY(sgpu_tensor_flush(ctx, true));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_ctr.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-        NL = ctx->h_scratch[0];
-        if (NL <= cap) {
+    const uint32_t s_full = pow2_slots(3ull * max_n), s_half = std::min(s_full, pow2_slots(2ull * max_n));
+    const uint32_t cand[4][2] = { { WIN_RING, s_full }, { 2, s_full }, { WIN_RING, s_half }, { 2, s_half } };
+    for (const auto &cd : cand) {
+        g.n_ring = cd[0];
+        g.slots = cd[1];
+        if (win_smem() <= WIN_SMEM_LIMIT) {
             break;
         }
-        if (attempt == 1) {
-            return sgpu_fail(ctx, SGPU_E_CUDA, "link list overflow on retry (%llu > %llu)", (unsigned long long)NL, (unsigned long long)cap);
+    }
+    if (win_smem() > WIN_SMEM_LIMIT) {
+        g.n_ring = 1;
+        g.slots = s_full;
+        while (g.slots > 1024 && win_smem() > WIN_SMEM_LIMIT) {
+            g.slots >>= 1;
         }
-        cap = NL; // the list was too small: the count is exact, run once more
+    }
+    g.smem = win_smem();
+    g.use_window = max_n <= WIN_MAX_ENTRIES && g.smem <= WIN_SMEM_LIMIT && 4ull * g.slots >= 5ull * max_n && !force_global;
+    return g;
+}
+
+// device -> host scalars, over the context's pinned scratch
+struct LinkScalars {
+    uint64_t count, unused;      // count: one at a time (largest locus, links, special entries, unsettled sweep, span splits)
+    int err, unsettled;          // d_err
+    uint64_t n_dropped, n_multi; // d_stats
+    uint64_t n_reads;            // readbase[n_loci]
+};
+
+constexpr int LINK_CAREFUL = 1; // status of a fast pass that met a read id chained over >= L bp: run the careful pass
+const char *const MSG_CELL_RANGE = "a group id is >= n_groups or maps to a cell >= num_cells (filter the pileup first)";
+
+// The stages of sgpu_link_reads and sgpu_cutoff_from_suffix, in the order they run, and what they share. A pass (from
+// build_reads on) runs a second time, careful, only when the fast one ends with LINK_CAREFUL.
+struct ReadLinker {
+    sgpu_ctx *ctx;
+    cudaStream_t st;
+    const sgpu_pileup *p;
+    LinkResult *out;
+    uint32_t L;
+    uint64_t E, P, W;    // entries, loci, words of the bitmap of special entries
+    unsigned locus_grid; // kernels that stride over the loci
+    bool strict_span;    // SECEDO_B200_STRICT_SPAN=1: a read id chained over >= L bp is an error instead of being split (tests)
+    LinkScalars *hs;
+    DevBuf<int> d_err;   // [0] error code, [1] "third sweep still changed something"
+    DevBuf<WinCounters> d_ctr;
+    DevBuf<unsigned long long> d_stats; // [0] dropped entries, [1] multi-locus reads
+    DevBuf<uint64_t> readbase, n_tail_reads, nf_scan;
+    DevBuf<uint2> links;
+    uint64_t NL = 0, NS = 0; // links, special entries
+    DevBuf<uint32_t> sp_first, g_cnt, cursor, nf_locus;
+
+    ReadLinker(sgpu_ctx *c, const sgpu_pileup *pl, LinkResult *o, uint32_t L_)
+        : ctx(c), st(c->stream), p(pl), out(o), L(L_), E(pl->n_entries), P(pl->n_loci), W(pl->n_entries / 32 + 1),
+          locus_grid(static_cast<unsigned>(std::min<uint64_t>(pl->n_loci, static_cast<uint64_t>(c->sm_count) * 16))),
+          strict_span(env_is_1("SECEDO_B200_STRICT_SPAN")), hs(reinterpret_cast<LinkScalars *>(c->h_scratch)) {}
+
+    // the status of a pass from the error word in hs: a read id chained over >= L bp ends the fast pass with
+    // LINK_CAREFUL and fails the careful one (or any with strict_span; name_strict: the message says so)
+    int status(bool careful, bool name_strict) {
+        if (hs->err == SGPU_E_CELL_RANGE) {
+            return sgpu_fail(ctx, hs->err, "%s", MSG_CELL_RANGE);
+        }
+        if (hs->err == SGPU_E_POSITIONS) {
+            return sgpu_fail(ctx, hs->err, "positions are not strictly increasing inside a chromosome");
+        }
+        if (hs->err == SGPU_E_FRAGMENT_SPAN || hs->unsettled) {
+            if (careful || strict_span) {
+                return sgpu_fail(ctx, SGPU_E_FRAGMENT_SPAN, "a read id spans >= max_fragment_length (%u)%s", L,
+                                 strict_span && name_strict ? " (SECEDO_B200_STRICT_SPAN=1: not split)" : "");
+            }
+            return LINK_CAREFUL;
+        }
+        return SGPU_OK;
     }
 
-    SGPU_TRACE(ctx, "link: window kernel");
-    // ---- special entries: numbering, first entry of the read, groups, mate rule -----------------------
-    uint64_t NS = 0;
-    DevBuf<uint32_t> nf_locus;
-    DevBuf<uint64_t> nf_scan;
-    if (NL) {
-        DevBuf<uint32_t> pc;
-        SGPU_CUDA(ctx, pc.alloc(W, ctx));
-        SGPU_CUDA(ctx, out->sp_rank.alloc(W + 1, ctx));
-        SGPU_LAUNCH(ctx, (mark_kernel<<<blocks_for(NL), TB, 0, st>>>(links.p, NL, out->sp_bits.p)));
-        SGPU_LAUNCH(ctx, (popc_kernel<<<blocks_for(W), TB, 0, st>>>(out->sp_bits.p, W, pc.p)));
-        SGPU_TRY(sgpu_scan_u32_u64(ctx, pc.p, out->sp_rank.p, W));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], out->sp_rank.p + W, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-        NS = ctx->h_scratch[0];
+    // argument checks, the result's arrays per group and locus, the error and statistics words, the largest locus
+    int prepare(uint32_t num_cells, const uint32_t *h_group_id_to_pos, uint32_t n_groups, uint32_t num_threads, bool ranged) {
+        if (E >= 0x7FFFFFF0ull || P >= 0x7FFFFFF0ull) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "more than 2^31 entries in one call: pass the pileup in batches of chromosomes");
+        }
+        if (p->n_chr > 255) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "more than 255 chromosomes in one call");
+        }
+        if (num_threads == 0) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "num_threads must be >= 1");
+        }
+        if (num_cells >= (1u << 27)) {
+            return sgpu_fail(ctx, SGPU_E_ARG, "num_cells too large");
+        }
+        out->n_reads = out->n_multi = out->n_dropped = out->n_tail = out->n_special = out->n_tail_loci = out->n_own = 0;
+        out->n_span_splits = 0;
+        out->ranged = ranged;
+        out->n_groups = n_groups;
+        out->num_cells = num_cells;
+        SGPU_CUDA(ctx, out->gmap.alloc(n_groups ? n_groups : 1, ctx));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(out->gmap.p, h_group_id_to_pos, n_groups * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        out->gmap_identity = n_groups <= num_cells;
+        for (uint32_t g = 0; g < n_groups && out->gmap_identity; ++g) {
+            out->gmap_identity = h_group_id_to_pos[g] == g;
+        }
+        SGPU_CUDA(ctx, out->sp_bits.alloc(W, ctx));
+        SGPU_CUDA(ctx, cudaMemsetAsync(out->sp_bits.p, 0, W * sizeof(uint32_t), st));
+        SGPU_CUDA(ctx, out->lchr.alloc(P ? P : 1, ctx));
+        SGPU_CUDA(ctx, out->tail_locus.alloc(p->n_chr ? p->n_chr : 1, ctx));
+        if (E == 0 || P == 0) {
+            // nothing to link; tail_locus = end of every chromosome
+            if (p->n_chr) {
+                SGPU_CUDA(ctx, cudaMemcpyAsync(out->tail_locus.p, p->d_chr_ptr + 1, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+            }
+            SGPU_CUDA(ctx, out->tail_loci.alloc(1, ctx));
+            return SGPU_OK;
+        }
+
+        SGPU_TRACE(ctx, "link: enter");
+        DevBuf<unsigned int> d_maxn;
+        SGPU_CUDA(ctx, d_err.alloc(2, ctx));
+        SGPU_CUDA(ctx, d_maxn.alloc(1, ctx));
+        SGPU_CUDA(ctx, d_ctr.alloc(1, ctx));
+        SGPU_CUDA(ctx, d_stats.alloc(2, ctx));
+        SGPU_CUDA(ctx, readbase.alloc(P + 1, ctx));
+        SGPU_CUDA(ctx, n_tail_reads.alloc(p->n_chr, ctx));
+        SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, 2 * sizeof(int), st));
+        SGPU_CUDA(ctx, cudaMemsetAsync(d_maxn.p, 0, sizeof(unsigned int), st));
+        SGPU_CUDA(ctx, cudaMemsetAsync(d_ctr.p, 0, sizeof(WinCounters), st));
+        SGPU_CUDA(ctx, cudaMemsetAsync(d_stats.p, 0, 2 * sizeof(unsigned long long), st));
+
+        SGPU_LAUNCH(ctx, (locus_meta_kernel<<<blocks_for(P), TB, 0, st>>>(p->d_row_ptr, p->d_position, p->d_chr_ptr, p->n_chr, P,
+                                                                           out->lchr.p, d_maxn.p, d_err.p)));
+        if (p->max_row == 0) {
+            SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->count, d_maxn.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+            SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+            p->max_row = static_cast<uint32_t>(hs->count); // cached: the pileup is immutable
+        }
+        SGPU_TRACE(ctx, "link: allocs+meta");
+        return SGPU_OK;
     }
-    SGPU_TRACE(ctx, "link: mark+rank");
-    out->n_special = NS;
-    SGPU_CUDA(ctx, out->sp_start.alloc(P + 1, ctx));
-    if (NS == 0) {
-        SGPU_CUDA(ctx, cudaMemsetAsync(out->sp_start.p, 0, (P + 1) * sizeof(uint32_t), st));
+
+    // links between entries of one read
+    int link_entries() {
+        // SECEDO_B200_FORCE_GLOBAL_HASH=1 forces the large-locus path (tests)
+        const WinGeometry g = window_geometry(p->max_row, env_is_1("SECEDO_B200_FORCE_GLOBAL_HASH"));
+        uint64_t cap = std::max<uint64_t>(E / 8, 4096);
+        for (int attempt = 0; attempt < 2; ++attempt) {
+            SGPU_CUDA(ctx, links.alloc(cap, ctx));
+            SGPU_CUDA(ctx, cudaMemsetAsync(d_ctr.p, 0, sizeof(WinCounters), st));
+            if (g.use_window) {
+                SGPU_CUDA(ctx, cudaFuncSetAttribute(link_window_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(g.smem)));
+                const unsigned per_sm = static_cast<unsigned>(std::max<size_t>(1, std::min<size_t>(4, (224 * 1024) / (g.smem + 2560))));
+                // contiguous ranges of owner loci, one per CTA, all CTAs resident at once
+                const uint64_t want = std::min<uint64_t>(P, static_cast<uint64_t>(ctx->sm_count) * per_sm);
+                const uint32_t loci_per_cta = static_cast<uint32_t>(ceil_div_u64(P, want));
+                const unsigned wgrid = static_cast<unsigned>(ceil_div_u64(P, loci_per_cta));
+                // this kernel never fits beside the tensor kernel of the previous batch, so it and everything behind it on the
+                // stream run alone: back to the default shared-memory / L1 split
+                SGPU_TRY(sgpu_cache_preference(ctx, false));
+                SGPU_LAUNCH(ctx, (link_window_kernel<<<wgrid, WIN_THREADS, g.smem, st>>>(p->d_row_ptr, p->d_position,
+                                                                                        p->d_read_id ? p->d_read_id : p->view_read_id,
+                                                                                        p->d_read_id ? nullptr : p->view_off, out->lchr.p, P, L,
+                                                                                        loci_per_cta, g.slots, g.id_cap, g.n_ring, links.p, cap, d_ctr.p)));
+            } else {
+                SGPU_TRY(sgpu_pileup_materialize(ctx, p)); // the global hash reads the ids by entry number
+                DevBuf<uint64_t> keys;
+                DevBuf<uint32_t> vals;
+                uint64_t hcap = 1024;
+                while (hcap < 2 * E) {
+                    hcap <<= 1;
+                }
+                SGPU_CUDA(ctx, keys.alloc(hcap, ctx));
+                SGPU_CUDA(ctx, vals.alloc(hcap, ctx));
+                SGPU_CUDA(ctx, cudaMemsetAsync(keys.p, 0xFF, hcap * sizeof(uint64_t), st));
+                SGPU_CUDA(ctx, cudaMemsetAsync(vals.p, 0xFF, hcap * sizeof(uint32_t), st));
+                SGPU_LAUNCH(ctx, (ghash_insert_kernel<<<locus_grid, TB, 0, st>>>(p->d_row_ptr, p->d_read_id, out->lchr.p, P, keys.p, vals.p, hcap - 1)));
+                SGPU_LAUNCH(ctx, (ghash_emit_kernel<<<locus_grid, TB, 0, st>>>(p->d_row_ptr, p->d_read_id, out->lchr.p, P, keys.p, vals.p, hcap - 1,
+                                                                                links.p, cap, d_ctr.p)));
+            }
+            SGPU_CUDA(ctx, cudaGetLastError());
+            // the previous batch's tensor kernel, if its launch has been held back: behind the dense linking pass, beside
+            // everything that follows (sgpu_tensor_flush)
+            SGPU_TRY(sgpu_tensor_flush(ctx, true));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->count, d_ctr.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+            NL = hs->count;
+            if (NL <= cap) {
+                break;
+            }
+            if (attempt == 1) {
+                return sgpu_fail(ctx, SGPU_E_CUDA, "link list overflow on retry (%llu > %llu)", (unsigned long long)NL, (unsigned long long)cap);
+            }
+            cap = NL; // the list was too small: the count is exact, run once more
+        }
+        SGPU_TRACE(ctx, "link: window kernel");
+        return SGPU_OK;
     }
-    DevBuf<uint32_t> sp_first, g_cnt, cursor;
-    if (NS) {
+
+    // special entries: numbering, first entry of the read, groups, mate rule
+    int number_special() {
+        if (NL) {
+            DevBuf<uint32_t> pc;
+            SGPU_CUDA(ctx, pc.alloc(W, ctx));
+            SGPU_CUDA(ctx, out->sp_rank.alloc(W + 1, ctx));
+            SGPU_LAUNCH(ctx, (mark_kernel<<<blocks_for(NL), TB, 0, st>>>(links.p, NL, out->sp_bits.p)));
+            SGPU_LAUNCH(ctx, (popc_kernel<<<blocks_for(W), TB, 0, st>>>(out->sp_bits.p, W, pc.p)));
+            SGPU_TRY(sgpu_scan_u32_u64(ctx, pc.p, out->sp_rank.p, W));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->count, out->sp_rank.p + W, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+            NS = hs->count;
+        }
+        SGPU_TRACE(ctx, "link: mark+rank");
+        out->n_special = NS;
+        SGPU_CUDA(ctx, out->sp_start.alloc(P + 1, ctx));
+        if (NS == 0) {
+            SGPU_CUDA(ctx, cudaMemsetAsync(out->sp_start.p, 0, (P + 1) * sizeof(uint32_t), st));
+            return SGPU_OK;
+        }
         SGPU_CUDA(ctx, out->sp_entry.alloc(NS, ctx));
         SGPU_CUDA(ctx, out->sp_locus.alloc(NS, ctx));
         SGPU_CUDA(ctx, out->sp_head.alloc(NS, ctx));
@@ -1266,11 +1320,19 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
                                                                             out->sp_entry.p, sp_first.p, out->sp_locus.p)));
         }
         SGPU_LAUNCH(ctx, (sp_start_kernel<<<blocks_for(P + 1), TB, 0, st>>>(out->sp_locus.p, NS, P, out->sp_start.p)));
+        return SGPU_OK;
     }
+
     // reads from the links: first entry of every read, entry lists, mate rule. careful = false: two sweeps settle every
     // read whose entries all lie within L bp of its first one (a third one verifies); careful = true (only after the fast
-    // pass reported a read id chained over >= L bp): sweep until nothing moves, then split such chains into reads
-    auto build_reads = [&](bool careful) -> int {
+    // pass reported a read id chained over >= L bp): from cleared error and statistics words, sweep until nothing moves,
+    // then split such chains into reads
+    int build_reads(bool careful) {
+        if (careful) {
+            SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, 2 * sizeof(int), st));
+            SGPU_CUDA(ctx, cudaMemsetAsync(d_stats.p, 0, 2 * sizeof(unsigned long long), st));
+            out->n_tail = 0;
+        }
         if (NS == 0) {
             return SGPU_OK;
         }
@@ -1292,9 +1354,9 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
                 SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p + 1, 0, sizeof(int), st));
                 SGPU_LAUNCH(ctx, (link_min_kernel<<<blocks_for(NL), TB, 0, st>>>(links.p, NL, out->sp_bits.p, out->sp_rank.p, sp_first.p,
                                                                                  d_err.p + 1)));
-                SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_err.p + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+                SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->count, d_err.p + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
                 SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-                if (static_cast<int>(ctx->h_scratch[0] & 0xFFFFFFFFu) == 0) {
+                if (static_cast<uint32_t>(hs->count) == 0) {
                     break;
                 }
                 if (sweep > 100000) {
@@ -1316,9 +1378,9 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
             SGPU_CUDA(ctx, cudaMemsetAsync(d_splits.p, 0, sizeof(unsigned long long), st));
             SGPU_LAUNCH(ctx, (split_span_kernel<<<blocks_for(NS), TB, 0, st>>>(out->sp_head.p, out->sp_entry.p, out->sp_locus.p, out->g_off.p, NS,
                                                                                out->g_list.p, p->d_position, L, sp_first.p, d_splits.p)));
-            SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_splits.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->count, d_splits.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
             SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-            out->n_span_splits = ctx->h_scratch[0];
+            out->n_span_splits = hs->count;
             SGPU_CUDA(ctx, cudaMemsetAsync(g_cnt.p, 0, NS * sizeof(uint32_t), st));
             SGPU_CUDA(ctx, cudaMemsetAsync(cursor.p, 0, NS * sizeof(uint32_t), st));
             SGPU_TRY(group());
@@ -1329,59 +1391,38 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
                                                                           out->sp_drop.p, out->g_nst.p, d_err.p))));
         SGPU_TRY(sgpu_scan_u32_u64(ctx, nf_locus.p, nf_scan.p, P));
         return SGPU_OK;
-    };
-    // SECEDO_B200_STRICT_SPAN=1: a read id chained over >= max_fragment_length is an error instead of being split (tests)
-    const char *env_strict = getenv("SECEDO_B200_STRICT_SPAN");
-    const bool strict_span = env_strict && env_strict[0] == '1';
-    out->n_span_splits = 0;
-    for (int pass = 0;; ++pass) {
-    const bool careful = pass > 0;
-    if (careful) { // the fast pass met a read id chained over >= L bp: once more, settling and splitting such chains
-        SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, 2 * sizeof(int), st));
-        SGPU_CUDA(ctx, cudaMemsetAsync(d_stats.p, 0, 2 * sizeof(unsigned long long), st));
-        out->n_tail = 0;
     }
-    SGPU_TRY(build_reads(careful));
-    SGPU_TRACE(ctx, "link: groups+mate rule");
-    // ---- cutoff K per chromosome ----------------------------------------------------------------------
-    SGPU_LAUNCH(ctx, (readbase_kernel<<<blocks_for(P + 1), TB, 0, st>>>(p->d_row_ptr, NS ? nf_scan.p : nullptr, P, readbase.p)));
-    DevBuf<uint64_t> own_lo, own_hi;
-    if (cutq) {
-        // the pileup holds only the END of every chromosome (unless whole[c]): decide the cutoff from there
-        DevBuf<uint8_t> d_whole, d_resolved;
-        DevBuf<uint64_t> exact_from;
-        DevBuf<uint32_t> d_tailpos;
-        SGPU_CUDA(ctx, d_whole.alloc(p->n_chr, ctx));
-        SGPU_CUDA(ctx, d_resolved.alloc(p->n_chr, ctx));
-        SGPU_CUDA(ctx, exact_from.alloc(p->n_chr, ctx));
-        SGPU_CUDA(ctx, d_tailpos.alloc(p->n_chr, ctx));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(d_whole.p, cutq->whole, p->n_chr, cudaMemcpyHostToDevice, st));
-        SGPU_LAUNCH(ctx, (exact_from_kernel<<<(p->n_chr + 63) / 64, 64, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, L, d_whole.p, exact_from.p)));
-        SGPU_LAUNCH(ctx, (cutoff_kernel<<<p->n_chr, CUT_THREADS, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, readbase.p, L, num_threads,
-                                                                          n_tail_reads.p, out->tail_locus.p, exact_from.p, d_resolved.p)));
-        SGPU_LAUNCH(ctx, (tail_position_kernel<<<(p->n_chr + 63) / 64, 64, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, out->tail_locus.p, d_tailpos.p)));
-        SGPU_CUDA(ctx, cudaGetLastError());
-        SGPU_CUDA(ctx, cudaMemcpyAsync(cutq->tail_position, d_tailpos.p, p->n_chr * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(cutq->resolved, d_resolved.p, p->n_chr, cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[2], d_err.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-        const int err = static_cast<int>(ctx->h_scratch[2] & 0xFFFFFFFFu);
-        if (err == SGPU_E_POSITIONS) {
-            return sgpu_fail(ctx, err, "positions are not strictly increasing inside a chromosome");
-        }
-        if (err == SGPU_E_FRAGMENT_SPAN || static_cast<int>(ctx->h_scratch[2] >> 32)) {
-            if (careful || strict_span) {
-                return sgpu_fail(ctx, SGPU_E_FRAGMENT_SPAN, "a read id spans >= max_fragment_length (%u)", L);
-            }
-            continue;
-        }
+
+    int read_bases() {
+        SGPU_TRACE(ctx, "link: groups+mate rule");
+        SGPU_LAUNCH(ctx, (readbase_kernel<<<blocks_for(P + 1), TB, 0, st>>>(p->d_row_ptr, NS ? nf_scan.p : nullptr, P, readbase.p)));
         return SGPU_OK;
     }
-    if (!range) {
+
+    // the cutoff K per chromosome. h_whole (null: all) flags the chromosomes the pileup holds whole; of the others it holds
+    // the END, and resolved[c] = 0 if that is too short to decide the cutoff (cutoff_kernel)
+    int launch_cutoff(uint32_t num_threads, const uint8_t *h_whole = nullptr, DevBuf<uint8_t> *resolved = nullptr) {
+        DevBuf<uint8_t> d_whole;
+        DevBuf<uint64_t> exact_from;
+        if (h_whole) {
+            SGPU_CUDA(ctx, d_whole.alloc(p->n_chr, ctx));
+            SGPU_CUDA(ctx, resolved->alloc(p->n_chr, ctx));
+            SGPU_CUDA(ctx, exact_from.alloc(p->n_chr, ctx));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(d_whole.p, h_whole, p->n_chr, cudaMemcpyHostToDevice, st));
+            SGPU_LAUNCH(ctx, (exact_from_kernel<<<(p->n_chr + 63) / 64, 64, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, L, d_whole.p, exact_from.p)));
+        }
         SGPU_LAUNCH(ctx, (cutoff_kernel<<<p->n_chr, CUT_THREADS, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, readbase.p, L, num_threads,
-                                                                          n_tail_reads.p, out->tail_locus.p)));
-    } else {
-        // a piece of the chromosomes: the cutoff comes from outside (sgpu_chromosome_cutoff), ownership from positions
+                                                                          n_tail_reads.p, out->tail_locus.p, exact_from.p,
+                                                                          h_whole ? resolved->p : nullptr)));
+        return SGPU_OK;
+    }
+
+    // the cutoff of a whole call; a piece of the chromosomes (range) gets it from outside (sgpu_chromosome_cutoff) or, for
+    // SGPU_TAIL_AUTO, from the piece itself, and its owned loci [own_lo[c], own_hi[c]) from positions
+    int cutoff(uint32_t num_threads, const RangeSpec *range, DevBuf<uint64_t> &own_lo, DevBuf<uint64_t> &own_hi) {
+        if (!range) {
+            return launch_cutoff(num_threads);
+        }
         DevBuf<uint32_t> spec;
         SGPU_CUDA(ctx, spec.alloc(3 * static_cast<size_t>(p->n_chr), ctx));
         SGPU_CUDA(ctx, own_lo.alloc(p->n_chr, ctx));
@@ -1391,24 +1432,16 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
         SGPU_CUDA(ctx, cudaMemcpyAsync(spec.p + p->n_chr, range->own_pos_end, p->n_chr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         SGPU_CUDA(ctx, cudaMemcpyAsync(spec.p + 2 * p->n_chr, range->tail_position, p->n_chr * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
         SGPU_CUDA(ctx, cudaMemsetAsync(n_tail_reads.p, 0, p->n_chr * sizeof(uint64_t), st));
-        // SGPU_TAIL_AUTO: the piece holds the END of the chromosome, the cutoff is decided from the piece itself (the
-        // part of it more than L bp behind its first locus is exact; everything is, if the piece starts the chromosome)
+        // SGPU_TAIL_AUTO: the piece holds the END of the chromosome (all of it if the piece starts the chromosome)
         bool any_auto = false;
         std::vector<uint8_t> h_whole(p->n_chr, 0);
         for (uint32_t c = 0; c < p->n_chr; ++c) {
             any_auto = any_auto || range->tail_position[c] == SGPU_TAIL_AUTO;
             h_whole[c] = range->own_pos_begin[c] == 0;
         }
-        DevBuf<uint8_t> d_whole, d_resolved;
-        DevBuf<uint64_t> exact_from;
+        DevBuf<uint8_t> d_resolved;
         if (any_auto) {
-            SGPU_CUDA(ctx, d_whole.alloc(p->n_chr, ctx));
-            SGPU_CUDA(ctx, d_resolved.alloc(p->n_chr, ctx));
-            SGPU_CUDA(ctx, exact_from.alloc(p->n_chr, ctx));
-            SGPU_CUDA(ctx, cudaMemcpyAsync(d_whole.p, h_whole.data(), p->n_chr, cudaMemcpyHostToDevice, st));
-            SGPU_LAUNCH(ctx, (exact_from_kernel<<<(p->n_chr + 63) / 64, 64, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, L, d_whole.p, exact_from.p)));
-            SGPU_LAUNCH(ctx, (cutoff_kernel<<<p->n_chr, CUT_THREADS, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, readbase.p, L, num_threads,
-                                                                              n_tail_reads.p, out->tail_locus.p, exact_from.p, d_resolved.p)));
+            SGPU_TRY(launch_cutoff(num_threads, h_whole.data(), &d_resolved));
         }
         SGPU_LAUNCH(ctx, (range_bounds_kernel<<<(p->n_chr + 63) / 64, 64, 0, st>>>(p->d_chr_ptr, p->n_chr, p->d_position, spec.p, spec.p + p->n_chr,
                                                                                   spec.p + 2 * p->n_chr, out->tail_locus.p, own_lo.p, own_hi.p)));
@@ -1424,81 +1457,98 @@ int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uin
                                  "use sgpu_chromosome_cutoff with a longer suffix", c);
             }
         }
+        return SGPU_OK;
     }
-    if (NS) {
-        const unsigned fin_grid = std::min<unsigned>(blocks_for(NS), static_cast<unsigned>(ctx->sm_count) * 16u);
-        SGPU_GB(p, SGPU_LAUNCH(ctx, (sp_finish_kernel<GB><<<fin_grid, TB, 0, st>>>(out->sp_head.p, out->sp_entry.p, out->sp_locus.p, out->sp_drop.p,
-                                                                          out->g_nst.p, gid_base_, out->lchr.p, out->tail_locus.p,
-                                                                          out->gmap.p, n_groups, num_cells, NS, out->sp_code.p,
-                                                                          out->sp_rcode.p, d_stats.p, d_err.p))));
-        SGPU_TRY(sgpu_link_candidates(ctx, out, 2));
-    }
-    SGPU_CUDA(ctx, cudaGetLastError());
 
-    SGPU_TRACE(ctx, "link: cutoff+finish");
-    // scalars to the host: errors, stats, reads created, tail loci per chromosome
-    std::vector<uint64_t> h_nt(p->n_chr), h_tl(p->n_chr);
-    SGPU_CUDA(ctx, cudaMemcpyAsync(h_tl.data(), out->tail_locus.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(h_nt.data(), n_tail_reads.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[2], d_err.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[4], d_stats.p, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[6], readbase.p + P, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-    const int err = static_cast<int>(ctx->h_scratch[2] & 0xFFFFFFFFu);
-    const int unsettled = static_cast<int>(ctx->h_scratch[2] >> 32);
-    if (err == SGPU_E_CELL_RANGE) {
-        return sgpu_fail(ctx, err, "a group id is >= n_groups or maps to a cell >= num_cells (filter the pileup first)");
-    }
-    if (err == SGPU_E_POSITIONS) {
-        return sgpu_fail(ctx, err, "positions are not strictly increasing inside a chromosome");
-    }
-    if (err == SGPU_E_FRAGMENT_SPAN || unsettled) {
-        if (careful || strict_span) {
-            return sgpu_fail(ctx, SGPU_E_FRAGMENT_SPAN, "a read id spans >= max_fragment_length (%u)%s", L,
-                             strict_span ? " (SECEDO_B200_STRICT_SPAN=1: not split)" : "");
+    int finish() {
+        if (NS) {
+            const unsigned fin_grid = std::min<unsigned>(blocks_for(NS), static_cast<unsigned>(ctx->sm_count) * 16u);
+            SGPU_GB(p, SGPU_LAUNCH(ctx, (sp_finish_kernel<GB><<<fin_grid, TB, 0, st>>>(out->sp_head.p, out->sp_entry.p, out->sp_locus.p, out->sp_drop.p,
+                                                                              out->g_nst.p, gid_base_, out->lchr.p, out->tail_locus.p,
+                                                                              out->gmap.p, out->n_groups, out->num_cells, NS, out->sp_code.p,
+                                                                              out->sp_rcode.p, d_stats.p, d_err.p))));
+            SGPU_TRY(sgpu_link_candidates(ctx, out, 2));
         }
-        continue;
+        SGPU_CUDA(ctx, cudaGetLastError());
+        SGPU_TRACE(ctx, "link: cutoff+finish");
+        return SGPU_OK;
     }
-    out->n_dropped = ctx->h_scratch[4];
-    out->n_multi = ctx->h_scratch[5];
-    out->n_reads = ctx->h_scratch[6];
-    std::vector<uint32_t> h_tail_loci, h_own_loci;
-    std::vector<uint64_t> h_lo(p->n_chr), h_hi(p->n_chr);
-    out->h_tail_locus = h_tl;
-    if (range) {
-        SGPU_CUDA(ctx, cudaMemcpyAsync(h_lo.data(), own_lo.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        SGPU_CUDA(ctx, cudaMemcpyAsync(h_hi.data(), own_hi.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+
+    // scalars to the host: errors, stats, reads created, tail loci per chromosome; then the lists of tail loci and, for a
+    // piece, of owned loci
+    int collect(bool careful, const RangeSpec *range, const DevBuf<uint64_t> &own_lo, const DevBuf<uint64_t> &own_hi) {
+        std::vector<uint64_t> h_nt(p->n_chr), h_tl(p->n_chr);
+        SGPU_CUDA(ctx, cudaMemcpyAsync(h_tl.data(), out->tail_locus.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(h_nt.data(), n_tail_reads.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->err, d_err.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->n_dropped, d_stats.p, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(&hs->n_reads, readbase.p + P, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-    }
-    for (uint32_t c = 0; c < p->n_chr; ++c) {
-        out->n_tail += h_nt[c];
-        const uint64_t lo = range ? h_lo[c] : p->h_chr_ptr[c], hi = range ? h_hi[c] : p->h_chr_ptr[c + 1];
-        for (uint64_t l = std::max(h_tl[c], lo); l < hi; ++l) { // tail x tail pairs are taken out at the OWNED loci only
-            h_tail_loci.push_back(static_cast<uint32_t>(l));
-        }
+        SGPU_TRY(status(careful, true));
+        out->n_dropped = hs->n_dropped;
+        out->n_multi = hs->n_multi;
+        out->n_reads = hs->n_reads;
+        std::vector<uint32_t> h_tail_loci, h_own_loci;
+        std::vector<uint64_t> h_lo(p->n_chr), h_hi(p->n_chr);
+        out->h_tail_locus = h_tl;
         if (range) {
-            for (uint64_t l = lo; l < hi; ++l) {
-                h_own_loci.push_back(static_cast<uint32_t>(l));
-            }
-        }
-    }
-    if (range) {
-        out->n_own = h_own_loci.size();
-        SGPU_CUDA(ctx, out->own_loci.alloc(h_own_loci.size() ? h_own_loci.size() : 1, ctx));
-        if (!h_own_loci.empty()) {
-            SGPU_CUDA(ctx, cudaMemcpyAsync(out->own_loci.p, h_own_loci.data(), h_own_loci.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(h_lo.data(), own_lo.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            SGPU_CUDA(ctx, cudaMemcpyAsync(h_hi.data(), own_hi.p, p->n_chr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
             SGPU_CUDA(ctx, cudaStreamSynchronize(st));
         }
+        for (uint32_t c = 0; c < p->n_chr; ++c) {
+            out->n_tail += h_nt[c];
+            const uint64_t lo = range ? h_lo[c] : p->h_chr_ptr[c], hi = range ? h_hi[c] : p->h_chr_ptr[c + 1];
+            for (uint64_t l = std::max(h_tl[c], lo); l < hi; ++l) { // tail x tail pairs are taken out at the OWNED loci only
+                h_tail_loci.push_back(static_cast<uint32_t>(l));
+            }
+            if (range) {
+                for (uint64_t l = lo; l < hi; ++l) {
+                    h_own_loci.push_back(static_cast<uint32_t>(l));
+                }
+            }
+        }
+        if (range) {
+            out->n_own = h_own_loci.size();
+            SGPU_CUDA(ctx, out->own_loci.alloc(h_own_loci.size() ? h_own_loci.size() : 1, ctx));
+            if (!h_own_loci.empty()) {
+                SGPU_CUDA(ctx, cudaMemcpyAsync(out->own_loci.p, h_own_loci.data(), h_own_loci.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+                SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+            }
+        }
+        SGPU_TRACE(ctx, "link: scalars");
+        out->n_tail_loci = h_tail_loci.size();
+        SGPU_CUDA(ctx, out->tail_loci.alloc(h_tail_loci.size() ? h_tail_loci.size() : 1, ctx));
+        if (!h_tail_loci.empty()) {
+            SGPU_CUDA(ctx, cudaMemcpyAsync(out->tail_loci.p, h_tail_loci.data(), h_tail_loci.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+            SGPU_CUDA(ctx, cudaStreamSynchronize(st)); // h_tail_loci is pageable
+        }
+        return SGPU_OK;
     }
-    SGPU_TRACE(ctx, "link: scalars");
-    out->n_tail_loci = h_tail_loci.size();
-    SGPU_CUDA(ctx, out->tail_loci.alloc(h_tail_loci.size() ? h_tail_loci.size() : 1, ctx));
-    if (!h_tail_loci.empty()) {
-        SGPU_CUDA(ctx, cudaMemcpyAsync(out->tail_loci.p, h_tail_loci.data(), h_tail_loci.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st)); // h_tail_loci is pageable
+};
+
+} // namespace
+
+int sgpu_link_reads(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t num_cells, uint32_t L,
+                    const uint32_t *h_group_id_to_pos, uint32_t n_groups, uint32_t num_threads,
+                    LinkResult *out, const RangeSpec *range) {
+    ReadLinker k(ctx, p, out, L);
+    SGPU_TRY(k.prepare(num_cells, h_group_id_to_pos, n_groups, num_threads, range != nullptr));
+    if (k.E == 0 || k.P == 0) {
+        return SGPU_OK;
     }
-    return SGPU_OK;
-    } // pass
+    SGPU_TRY(k.link_entries());
+    SGPU_TRY(k.number_special());
+    auto pass = [&](bool careful) -> int {
+        DevBuf<uint64_t> own_lo, own_hi;
+        SGPU_TRY(k.build_reads(careful));
+        SGPU_TRY(k.read_bases());
+        SGPU_TRY(k.cutoff(num_threads, range, own_lo, own_hi));
+        SGPU_TRY(k.finish());
+        return k.collect(careful, range, own_lo, own_hi);
+    };
+    const int rc = pass(false);
+    return rc == LINK_CAREFUL ? pass(true) : rc;
 }
 
 int sgpu_link_candidates(sgpu_ctx *ctx, LinkResult *out, uint32_t min_nst) {
@@ -1549,11 +1599,10 @@ int sgpu_link_dense_codes(sgpu_ctx *ctx, const sgpu_pileup *p, LinkResult *lr) {
     SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[0], d_err.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     SGPU_CUDA(ctx, cudaStreamSynchronize(st));
     if (static_cast<int>(ctx->h_scratch[0] & 0xFFFFFFFFu) != 0) {
-        return sgpu_fail(ctx, SGPU_E_CELL_RANGE, "a group id is >= n_groups or maps to a cell >= num_cells (filter the pileup first)");
+        return sgpu_fail(ctx, SGPU_E_CELL_RANGE, "%s", MSG_CELL_RANGE);
     }
     return SGPU_OK;
 }
-
 int sgpu_cutoff_from_suffix(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t L, uint32_t num_threads, const uint8_t *h_whole,
                             uint32_t *h_tail_position, uint8_t *h_resolved) {
     for (uint32_t c = 0; c < p->n_chr; ++c) { // chromosomes without loci: nothing is tail, trivially decided
@@ -1564,10 +1613,27 @@ int sgpu_cutoff_from_suffix(sgpu_ctx *ctx, const sgpu_pileup *p, uint32_t L, uin
         return SGPU_OK;
     }
     LinkResult lr;
-    CutoffQuery q;
-    q.whole = h_whole;
-    q.tail_position = h_tail_position;
-    q.resolved = h_resolved;
+    ReadLinker k(ctx, p, &lr, L);
     const uint32_t none = 0;
-    return sgpu_link_reads(ctx, p, 1, L, &none, 0, num_threads, &lr, nullptr, &q);
+    SGPU_TRY(k.prepare(1, &none, 0, num_threads, false));
+    SGPU_TRY(k.link_entries());
+    SGPU_TRY(k.number_special());
+    auto pass = [&](bool careful) -> int {
+        SGPU_TRY(k.build_reads(careful));
+        SGPU_TRY(k.read_bases());
+        DevBuf<uint8_t> d_resolved;
+        SGPU_TRY(k.launch_cutoff(num_threads, h_whole, &d_resolved));
+        DevBuf<uint32_t> d_tailpos;
+        SGPU_CUDA(ctx, d_tailpos.alloc(p->n_chr, ctx));
+        SGPU_LAUNCH(ctx, (tail_position_kernel<<<(p->n_chr + 63) / 64, 64, 0, k.st>>>(p->d_chr_ptr, p->n_chr, p->d_position, lr.tail_locus.p,
+                                                                                      d_tailpos.p)));
+        SGPU_CUDA(ctx, cudaGetLastError());
+        SGPU_CUDA(ctx, cudaMemcpyAsync(h_tail_position, d_tailpos.p, p->n_chr * sizeof(uint32_t), cudaMemcpyDeviceToHost, k.st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(h_resolved, d_resolved.p, p->n_chr, cudaMemcpyDeviceToHost, k.st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(&k.hs->err, k.d_err.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, k.st));
+        SGPU_CUDA(ctx, cudaStreamSynchronize(k.st));
+        return k.status(careful, false);
+    };
+    const int rc = pass(false);
+    return rc == LINK_CAREFUL ? pass(true) : rc;
 }
