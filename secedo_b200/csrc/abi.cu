@@ -318,13 +318,13 @@ int sgpu_init(int device, sgpu_ctx **out) {
         // kernels it shares the SMs with
         int least = 0, greatest = 0;
         SGPU_CUDA(ctx, cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        SGPU_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->tensor_stream, cudaStreamNonBlocking, greatest));
+        SGPU_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->tensor.stream, cudaStreamNonBlocking, greatest));
         const char *as = getenv("SECEDO_B200_ASYNC_GEMM");
-        ctx->async_gemm = !(as && as[0] == '0');
+        ctx->tensor.async = !(as && as[0] == '0');
         // kernels only run beside the tensor kernel while the device-wide cache preference is PreferShared (sgpu_ctx::prefer_shared,
         // profiles/coresidency_probe.cu): switched on and off around the window in which that can happen
         const char *ps = getenv("SECEDO_B200_PREFER_SHARED");
-        ctx->prefer_shared = ps ? ps[0] != '0' : ctx->async_gemm;
+        ctx->prefer_shared = ps ? ps[0] != '0' : ctx->tensor.async;
     }
     return SGPU_OK;
 }
@@ -336,22 +336,15 @@ void sgpu_shutdown(sgpu_ctx *ctx) {
     if (ctx->own_stream) { // contexts that failed in sgpu_init carry only the error text
         cudaSetDevice(ctx->device);
         cudaStreamSynchronize(ctx->stream);
-        if (ctx->tensor_stream) {
-            sgpu_tensor_poll(ctx, true); // issues a launch that is still pending, waits for all of them
-            cudaStreamSynchronize(ctx->tensor_stream);
-            for (auto &j : ctx->tensor_jobs) { // only after a failed kernel
-                cudaEventDestroy(j.t0);
-                cudaEventDestroy(j.t1);
-                sgpu_dev_free(ctx, j.U);
-                sgpu_dev_free(ctx, j.err);
-            }
-            ctx->tensor_jobs.clear();
-            for (cudaEvent_t e : ctx->event_pool) {
+        if (ctx->tensor.stream) {
+            sgpu_tensor_drain(ctx); // issues a launch that is still held back, waits for all of them
+            cudaStreamSynchronize(ctx->tensor.stream);
+            for (cudaEvent_t e : ctx->tensor.event_pool) {
                 cudaEventDestroy(e);
             }
-            ctx->event_pool.clear();
-            cudaStreamDestroy(ctx->tensor_stream);
-            ctx->tensor_stream = nullptr;
+            ctx->tensor.event_pool.clear();
+            cudaStreamDestroy(ctx->tensor.stream);
+            ctx->tensor.stream = nullptr;
         }
         if (ctx->cache_pref_now == 1) { // the device-wide preference this context switched on goes with it
             cudaDeviceSetCacheConfig(cudaFuncCachePreferNone);
@@ -396,7 +389,7 @@ int sgpu_set_stream(sgpu_ctx *ctx, void *cuda_stream) {
     SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
     // cached blocks are only safe to reuse in the order of ONE stream: drain the old one first
     SGPU_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    SGPU_TRY(sgpu_tensor_poll(ctx, true));
+    SGPU_TRY(sgpu_tensor_drain(ctx));
     ctx->stream = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
     return SGPU_OK;
 }
@@ -409,7 +402,7 @@ int sgpu_synchronize(sgpu_ctx *ctx) {
         SGPU_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
     }
     SGPU_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    SGPU_TRY(sgpu_tensor_poll(ctx, true)); // tensor kernels still in flight (sgpu_ctx::tensor_jobs)
+    SGPU_TRY(sgpu_tensor_poll(ctx, true)); // tensor kernels still in flight (sgpu_ctx::tensor)
     return SGPU_OK;
 }
 
@@ -424,19 +417,28 @@ int sgpu_cache_preference(sgpu_ctx *ctx, bool shared) {
     return SGPU_OK;
 }
 
+// The prologue of every entry point that reads or writes the count planes of c: a first-order tensor kernel may still be
+// adding to them (sgpu_ctx::tensor), so ctx->stream waits for it. The device is set first: the join may issue a held-back
+// launch.
+static int planes_ready(sgpu_ctx *ctx, const sgpu_counts *c) {
+    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    return sgpu_tensor_join(ctx, c->i32);
+}
+
 extern "C" {
 
 int sgpu_tensor_times(sgpu_ctx *ctx, float *ms, uint64_t *launches) {
     SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
     SGPU_TRY(sgpu_tensor_poll(ctx, true));
+    float m = 0.f;
+    uint64_t n = 0;
+    sgpu_tensor_take_times(ctx, &m, &n);
     if (ms) {
-        *ms = ctx->ms_syrk;
+        *ms = m;
     }
     if (launches) {
-        *launches = ctx->n_syrk;
+        *launches = n;
     }
-    ctx->ms_syrk = 0.f;
-    ctx->n_syrk = 0;
     return SGPU_OK;
 }
 
@@ -448,7 +450,7 @@ int sgpu_set_option(sgpu_ctx *ctx, const char *name, int value) {
     SGPU_TRY(sgpu_synchronize(ctx));
     const std::string n(name);
     if (n == "async_gemm") {
-        ctx->async_gemm = value != 0;
+        ctx->tensor.async = value != 0;
     } else if (n == "prefer_shared") {
         if (value != 0 && value != 1) {
             return sgpu_fail(ctx, SGPU_E_ARG, "prefer_shared must be 0 or 1");
@@ -808,8 +810,7 @@ int sgpu_counts_create(sgpu_ctx *ctx, uint32_t num_cells, sgpu_counts **out) {
 }
 
 int sgpu_counts_zero(sgpu_ctx *ctx, sgpu_counts *c) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     // only the planes that were used since the last zeroing can be non-zero
     SGPU_CUDA(ctx, cudaMemsetAsync(c->i32, 0, static_cast<uint64_t>(c->planes_dirty) * c->nn * sizeof(int32_t), ctx->stream));
     SGPU_CUDA(ctx, cudaMemsetAsync(c->hist, 0, SGPU_MAX_CLASS * SGPU_MAX_CLASS * sizeof(uint64_t), ctx->stream));
@@ -831,7 +832,7 @@ void sgpu_counts_free(sgpu_ctx *ctx, sgpu_counts *c) {
     if (ctx) {
         cudaSetDevice(ctx->device);
         cudaStreamSynchronize(ctx->stream);
-        sgpu_tensor_poll(ctx, true);
+        sgpu_tensor_drain(ctx);
     }
     cudaFree(c->i32);
     cudaFree(c->hist);
@@ -894,7 +895,7 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
     s.n_multi_reads = lr.n_multi;
     s.n_tail_reads = lr.n_tail;
     s.n_span_splits = static_cast<int32_t>(std::min<uint64_t>(lr.n_span_splits, 0x7FFFFFFF));
-    ctx->ms_stage = 0.f;
+    ctx->tensor.ms_stage = 0.f;
     // Once first-order counts have been issued, a failure leaves a partial sum behind, possibly in every plane (the
     // order-2 / order-3 atomics of the other pairs land too): later accumulations are then refused until
     // sgpu_counts_zero, and that clears all planes. Failures before that point leave the object as it was.
@@ -926,7 +927,7 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
         SGPU_TRY(rc);
     }
     t_first.mark();
-    s.ms_stage = ctx->ms_stage;
+    s.ms_stage = ctx->tensor.ms_stage;
     // second / third order planes, spill plane, histogram: none of them is touched by the first-order tensor kernel
     // that may still be running
     EventTimer t_multi(ctx->stream);
@@ -938,10 +939,7 @@ static int accumulate_impl(sgpu_ctx *ctx, sgpu_counts *c, const sgpu_pileup *fil
     // Tensor kernels retired during this call (with SECEDO_B200_ASYNC_GEMM=0: this call's own; otherwise mostly the one of
     // the batch before; sgpu_tensor_times returns what is left)
     SGPU_TRY(issued(sgpu_tensor_poll(ctx, false)));
-    s.ms_gemm = ctx->ms_syrk;
-    s.gemm_launches = ctx->n_syrk;
-    ctx->ms_syrk = 0.f;
-    ctx->n_syrk = 0;
+    sgpu_tensor_take_times(ctx, &s.ms_gemm, &s.gemm_launches);
     c->planes_dirty = std::max(c->planes_dirty, c->planes_used);
     if (stats) {
         *stats = s;
@@ -995,10 +993,9 @@ int sgpu_counts_buffers(sgpu_counts *c, int32_t **i32, uint64_t *n_i32, double *
         return SGPU_E_ARG;
     }
     if (c->owner) {
-        SGPU_CUDA(c->owner, cudaSetDevice(c->owner->device)); // a held-back tensor kernel may be launched here
         // whoever reads the planes through these pointers is ordered behind the context's stream (a collective, a peer's
-        // kernel after a barrier): make that stream wait for a first-order tensor kernel that is still adding to them
-        SGPU_TRY(sgpu_tensor_join(c->owner, c->i32));
+        // kernel after a barrier)
+        SGPU_TRY(planes_ready(c->owner, c));
     }
     if (i32) {
         *i32 = c->i32;
@@ -1022,8 +1019,7 @@ int sgpu_counts_buffers(sgpu_counts *c, int32_t **i32, uint64_t *n_i32, double *
 }
 
 int sgpu_counts_set_layout(sgpu_ctx *ctx, sgpu_counts *c, int planes_used, int want_spill) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (planes_used != 2 && planes_used != PLANE_H3 && planes_used != N_PLANES) {
         return sgpu_fail(ctx, SGPU_E_ARG, "planes_used must be 2, %d or %d", PLANE_H3, N_PLANES);
     }
@@ -1037,8 +1033,7 @@ int sgpu_counts_set_layout(sgpu_ctx *ctx, sgpu_counts *c, int planes_used, int w
 }
 
 int sgpu_counts_pack_range(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, int n_planes, int32_t **packed, uint64_t *n) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (first_plane < 0 || n_planes < 0 || first_plane + n_planes > c->planes_used) {
         return sgpu_fail(ctx, SGPU_E_ARG, "plane range [%d, %d) outside the %d planes in use", first_plane, first_plane + n_planes, c->planes_used);
     }
@@ -1066,8 +1061,7 @@ int sgpu_counts_pack_range(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, int n
 }
 
 int sgpu_counts_unpack_range(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, int n_planes) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (first_plane < 0 || n_planes < 0 || first_plane + n_planes > c->planes_used) {
         return sgpu_fail(ctx, SGPU_E_ARG, "plane range [%d, %d) outside the %d planes in use", first_plane, first_plane + n_planes, c->planes_used);
     }
@@ -1095,8 +1089,7 @@ int sgpu_counts_unpack(sgpu_ctx *ctx, sgpu_counts *c) {
 }
 
 int sgpu_counts_sparse_pack(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, uint32_t **idx, int32_t **val, uint64_t *nnz) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     cudaStream_t st = ctx->stream;
     const int n_planes = c->planes_used - first_plane;
     if (first_plane < 0 || n_planes < 0) {
@@ -1148,8 +1141,7 @@ int sgpu_counts_sparse_pack(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, uint
 }
 
 int sgpu_counts_sparse_add(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, const uint32_t *idx, const int32_t *val, uint64_t nnz) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (first_plane < 0 || first_plane > c->planes_used) {
         return sgpu_fail(ctx, SGPU_E_ARG, "first plane %d outside the %d planes in use", first_plane, c->planes_used);
     }
@@ -1163,8 +1155,7 @@ int sgpu_counts_sparse_add(sgpu_ctx *ctx, sgpu_counts *c, int first_plane, const
 }
 
 int sgpu_counts_download(sgpu_ctx *ctx, sgpu_counts *c, int32_t *S1, int32_t *D1, int32_t *H, uint64_t *hist) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     cudaStream_t st = ctx->stream;
     const uint64_t nn = c->nn, n = c->n;
     std::vector<int32_t> tmp(nn);
@@ -1200,8 +1191,7 @@ int sgpu_counts_download(sgpu_ctx *ctx, sgpu_counts *c, int32_t *S1, int32_t *D1
 int sgpu_similarity_finalize(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragment_length, double mutation_rate,
                              double homozygous_rate, double seq_error_rate, int normalization, double *out,
                              sgpu_stats *stats) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (c->have_params && c->spill
         && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
         return sgpu_fail(ctx, SGPU_E_ARG, "finalize called with likelihood parameters different from accumulate");
@@ -1217,8 +1207,7 @@ int sgpu_similarity_finalize(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragmen
 
 int sgpu_similarity_finalize_async(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragment_length, double mutation_rate,
                                    double homozygous_rate, double seq_error_rate, int normalization, double *out) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (!out) {
         return sgpu_fail(ctx, SGPU_E_ARG, "finalize_async needs a (page-locked) host buffer");
     }
@@ -1250,10 +1239,7 @@ int sgpu_similarity(sgpu_ctx *ctx, const sgpu_pileup *filtered, uint32_t num_cel
                                     homozygous_rate, seq_error_rate, num_threads, path, &s);
     if (rc == SGPU_OK) { // one-shot call: nothing to overlap the tensor kernel with; its time belongs to these statistics
         rc = sgpu_tensor_poll(ctx, true);
-        s.ms_gemm += ctx->ms_syrk;
-        s.gemm_launches += ctx->n_syrk;
-        ctx->ms_syrk = 0.f;
-        ctx->n_syrk = 0;
+        sgpu_tensor_take_times(ctx, &s.ms_gemm, &s.gemm_launches);
     }
     if (rc == SGPU_OK) {
         rc = sgpu_similarity_finalize(ctx, c, max_fragment_length, mutation_rate, homozygous_rate, seq_error_rate,
@@ -1270,8 +1256,7 @@ int sgpu_similarity(sgpu_ctx *ctx, const sgpu_pileup *filtered, uint32_t num_cel
 int sgpu_slab_raw(sgpu_ctx *ctx, sgpu_counts *c, const int32_t *const *peer_planes, const double *const *peer_spill,
                   uint32_t n_peers, uint32_t slab, uint32_t n_slabs, uint32_t max_fragment_length, double mutation_rate,
                   double homozygous_rate, double seq_error_rate, double **extrema) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     // the spill plane holds G(x_s, x_d) evaluated with the accumulation's parameters; F and G must not be mixed
     if (c->have_params && c->spill
         && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
@@ -1342,8 +1327,7 @@ int sgpu_host_unregister(sgpu_ctx *ctx, void *host) {
 
 int sgpu_counts_checksum(sgpu_ctx *ctx, sgpu_counts *c, const int32_t *const *peer_planes, uint32_t n_peers, uint32_t slab,
                          uint32_t n_slabs, uint64_t *checksum) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (n_peers > SGPU_MAX_PEERS || n_slabs == 0 || slab >= n_slabs) {
         return sgpu_fail(ctx, SGPU_E_ARG, "checksum: %u peers, slab %u of %u", n_peers, slab, n_slabs);
     }
@@ -1426,8 +1410,7 @@ int sgpu_similarity_finalize_spectral(sgpu_ctx *ctx, sgpu_counts *c, uint32_t ma
                                       double homozygous_rate, double seq_error_rate, int normalization, double *out,
                                       uint32_t k, double tol, double *eigenvalues, double *eigenvectors, sgpu_stats *stats,
                                       sgpu_spectral_stats *spectral_stats) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (c->have_params && c->spill
         && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
         return sgpu_fail(ctx, SGPU_E_ARG, "finalize called with likelihood parameters different from accumulate");
@@ -1458,8 +1441,7 @@ int sgpu_laplacian_eigenvalues(sgpu_ctx *ctx, const double *similarity, uint32_t
 int sgpu_similarity_finalize_eigenvalues(sgpu_ctx *ctx, sgpu_counts *c, uint32_t max_fragment_length, double mutation_rate,
                                          double homozygous_rate, double seq_error_rate, int normalization, double *out,
                                          double *eigenvalues, sgpu_stats *stats, sgpu_eigenvalue_stats *eig_stats) {
-    SGPU_TRY(sgpu_tensor_join(ctx, c->i32)); // a first-order tensor kernel may still be adding to the planes (sgpu_ctx::tensor_jobs)
-    SGPU_CUDA(ctx, cudaSetDevice(ctx->device));
+    SGPU_TRY(planes_ready(ctx, c));
     if (c->have_params && c->spill
         && (c->eps != mutation_rate || c->h != homozygous_rate || c->theta != seq_error_rate || c->L != max_fragment_length)) {
         return sgpu_fail(ctx, SGPU_E_ARG, "finalize called with likelihood parameters different from accumulate");

@@ -1,6 +1,7 @@
 // Shared declarations of the CUDA side of secedo_b200 (sm_100a only).
 #pragma once
 
+#include <cuda.h> // CUtensorMap (a held-back tensor-kernel launch keeps its arguments by value); no driver call is linked
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -9,11 +10,66 @@
 #include <cstdio>
 #include <deque>
 #include <map>
+#include <optional>
 #include <string>
 #include <unordered_map>
 #include <vector>
 
 #include "../../include/secedo_b200.h"
+
+// ------------------------------------------------------------------------------------------------
+// gemm.cu — the first-order tensor kernel and its lifetime
+// ------------------------------------------------------------------------------------------------
+// The arguments of one launch, by value: a held-back launch is issued by a later call. gemm.cu builds the kernel's WorkList
+// from them; the output tiles are cut into work items there: whole tiles first, the rest in K ranges.
+struct TensorArgs {
+    CUtensorMap map;             // over the operand panel
+    const uint2 *tiles;          // upper-triangle output tiles, rasterised
+    uint32_t kbs_main, kbs_tail; // k-blocks of the panel's loci; of the tail reads (Z, then as many of -Z)
+    uint32_t n_full, n_work;     // tiles processed whole; work items
+    uint32_t splits, per;        // K ranges per remaining tile; k-blocks per range
+    unsigned grid;               // CTA pairs
+    unsigned int *wave_ctr;      // in the error words of the panel
+    int32_t *S, *D;
+    uint32_t N;
+    int epi;                     // how whole tiles reach the planes (EPI_STORE / EPI_RMW)
+};
+struct sgpu_ctx;
+// One launch of the tensor kernel and what it owns. Whatever it holds goes back (events to the pool, blocks to the cache)
+// when it is destroyed, on every path; it is destroyed only when no launched kernel can still read its blocks: after its t1
+// has been seen, or after the stream a kernel reading them was launched on has been synchronised (sgpu_gemm_run).
+struct TensorJob {
+    sgpu_ctx *ctx;
+    const void *planes = nullptr; // first of the count planes the kernel adds to (whom a join concerns)
+    TensorArgs args{};
+    void *U = nullptr;            // operand panel (context cache; the job of a call's last panel only)
+    int *err = nullptr;           // [0] range check of the staging, [1] wave counter (context cache; last panel only)
+    cudaEvent_t t0 = nullptr, t1 = nullptr; // around the kernel, on the stream it was launched on
+    cudaEvent_t staged = nullptr; // held back: on ctx->stream, behind the staging kernel
+    explicit TensorJob(sgpu_ctx *c) : ctx(c) {}
+    TensorJob(TensorJob &&o) noexcept;
+    TensorJob &operator=(TensorJob &&) = delete;
+    ~TensorJob();
+};
+// The tensor kernel of a first-order accumulation runs on a stream of its own (highest priority), behind an event of its
+// staging kernel, and the call returns without waiting for it: the filter / read linking / staging kernels of the NEXT
+// batch (issue and latency bound, on ctx->stream) then run beside it on the same SMs (the tensor kernel keeps one CTA of
+// 6 warps per SM and leaves ~95 % of the issue slots idle). The launch of the last one is held back until the next batch's
+// link_window kernel has been issued (sgpu_tensor_flush) or somebody needs it first; everything that touches the count
+// planes first makes ctx->stream wait for the last job (sgpu_tensor_join). SECEDO_B200_ASYNC_GEMM=0: the kernel runs on
+// ctx->stream. A job gives its events to event_pool and its blocks to the context's cache: both are declared before the
+// jobs, so that they outlive them (sgpu_shutdown drains the queue anyway).
+struct TensorQueue {
+    cudaStream_t stream = nullptr;
+    bool async = true;                   // option async_gemm
+    std::vector<cudaEvent_t> event_pool; // recycled events
+    std::deque<TensorJob> jobs;          // issued, in launch order (they finish in this order)
+    std::optional<TensorJob> held;       // prepared, not issued
+    // device time not yet reported through sgpu_stats / sgpu_tensor_times, from CUDA events: the tensor kernels retired so
+    // far, the staging of the current accumulation
+    float ms = 0.f, ms_stage = 0.f;
+    uint64_t launches = 0;
+};
 
 // ------------------------------------------------------------------------------------------------
 // context / error handling
@@ -33,28 +89,6 @@ struct sgpu_ctx {
     uint64_t *h_scratch = nullptr; // 64 x u64, pinned
     uint64_t *d_scratch = nullptr; // 64 x u64, device
     uint64_t launches = 0;         // kernels launched by this context (sgpu_launch_count)
-    // device time of the dominant kernels not yet reported through sgpu_stats / sgpu_tensor_times, from CUDA events
-    // recorded on ctx->stream around the launches
-    float ms_syrk = 0.f, ms_stage = 0.f;
-    uint64_t n_syrk = 0;
-    // gemm.cu: the tensor kernel of a first-order accumulation runs on a stream of its own (highest priority), behind an
-    // event of the staging kernel, and the call returns without waiting for it: the filter / read linking / staging
-    // kernels of the NEXT batch (issue and latency bound, on ctx->stream) then run beside it on the same SMs (the tensor
-    // kernel keeps one CTA of 6 warps per SM and leaves ~95 % of the issue slots idle). A job owns what its kernel reads
-    // (the operand panel) until its end event has been seen; everything that touches the count planes first makes
-    // ctx->stream wait for the last job (sgpu_tensor_join). SECEDO_B200_ASYNC_GEMM=0: the kernel runs on ctx->stream.
-    cudaStream_t tensor_stream = nullptr;
-    bool async_gemm = true;
-    struct TensorJob {
-        const void *planes = nullptr; // first of the count planes the kernel adds to (whom a join concerns)
-        void *U = nullptr;   // operand panel (context cache)
-        int *err = nullptr;  // [0] range check of the staging, [1] wave counter of the tensor kernel (context cache)
-        cudaEvent_t t0 = nullptr, t1 = nullptr; // around the kernel, on the stream it was launched on
-    };
-    std::deque<TensorJob> tensor_jobs;
-    void *pending_gemm = nullptr;        // gemm.cu: prepared launch of the last deferred tensor kernel, issued behind the next
-                                         // batch's link_window kernel (sgpu_tensor_flush)
-    std::vector<cudaEvent_t> event_pool; // recycled timing events
     // Kernels only share an SM with the tensor kernel while the DEVICE-WIDE cache preference is cudaFuncCachePreferShared: a
     // kernel with 16 KB of static shared memory otherwise waited for the whole tensor kernel, and neither the carve-out
     // attribute nor cudaFuncSetCacheConfig of that kernel changed it (profiles/coresidency_probe.cu, r2_coresidency.txt,
@@ -79,6 +113,7 @@ struct sgpu_ctx {
     std::multimap<size_t, void *> free_blocks;
     std::unordered_map<void *, size_t> live_blocks;
     size_t cached_bytes = 0;
+    TensorQueue tensor; // gemm.cu: the first-order tensor kernels held back or in flight (after the cache: see TensorQueue)
     // SECEDO_B200_TRACE=1: synchronise and print the wall-clock time between trace points (debug aid)
     bool trace = false;
     bool trace_alloc = false; // SECEDO_B200_TRACE=2: log every real cudaMalloc
@@ -102,13 +137,19 @@ void sgpu_trace_point(sgpu_ctx *ctx, const char *what);
 int sgpu_fail(sgpu_ctx *ctx, int code, const char *fmt, ...);
 // device-wide shared-memory / L1 preference, switched only when it changes (see sgpu_ctx::prefer_shared)
 int sgpu_cache_preference(sgpu_ctx *ctx, bool shared);
-// gemm.cu — tensor kernels in flight on ctx->tensor_stream (see sgpu_ctx::tensor_jobs)
-int sgpu_tensor_poll(sgpu_ctx *ctx, bool wait_all); // retire finished jobs (timing, operand panel back to the cache)
+// gemm.cu — the operations of sgpu_ctx::tensor
+int sgpu_tensor_flush(sgpu_ctx *ctx, bool after_main); // issue the held-back launch, if any (after_main: behind everything queued on ctx->stream)
+// retire the finished jobs (kernel time into the queue's statistics); wait_all: issue the held-back launch, wait for all
+int sgpu_tensor_poll(sgpu_ctx *ctx, bool wait_all);
 // ctx->stream waits (on the device) for the last job that writes the count planes starting at `planes` (null: any job); a
 // launch still held back is issued first if it writes them. A caller that alternates between two counts objects thereby
 // keeps the other object's tensor kernel in flight (or held back) across its epilogue.
 int sgpu_tensor_join(sgpu_ctx *ctx, const void *planes = nullptr);
-int sgpu_tensor_flush(sgpu_ctx *ctx, bool after_main); // issue the prepared launch, if any (after_main: behind everything queued on ctx->stream)
+// sgpu_tensor_poll(wait_all) for callers that need the queue empty afterwards (sgpu_set_stream, sgpu_counts_free,
+// sgpu_shutdown): after a failure the tensor stream is synchronised and the jobs left over are given back
+int sgpu_tensor_drain(sgpu_ctx *ctx);
+// adds the time and number of the tensor kernels retired so far to *ms and *launches, and starts counting again
+void sgpu_tensor_take_times(sgpu_ctx *ctx, float *ms, uint64_t *launches);
 // make the context's stream wait for an asynchronously uploaded pileup
 #define SGPU_WAIT_PILEUP(ctx, p)                                                                   \
     do {                                                                                           \
@@ -440,7 +481,7 @@ struct GemmInput {
     const uint32_t *tail_loci; // loci whose entries are subtracted as Z Z^T (ascending)
     uint64_t n_tail_loci;
     bool may_defer = false;    // the tensor kernel of the last panel may still be running when the call returns (see
-                               // sgpu_ctx::tensor_jobs); false: the result is complete in the order of ctx->stream
+                               // TensorQueue); false: the result is complete in the order of ctx->stream
 };
 int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t num_cells, int32_t *S_plane, int32_t *D_plane, bool *fresh,
                   bool *poisoned = nullptr);

@@ -34,6 +34,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 namespace {
@@ -614,7 +615,7 @@ enum : int {
 constexpr int HALF_B_BYTES = 128 * KB_BYTES;             // 16 KB
 constexpr int STAGE_BYTES = A_BYTES + HALF_B_BYTES;      // 32 KB per CTA
 // 5 stages (161 KB) leave shared memory to the staging kernels of the next batch that run beside the deferred kernel
-// (sgpu_ctx::tensor_jobs); 4 are slower. With the SM to itself (SECEDO_B200_ASYNC_GEMM=0) 6 stages (193 KB) would be
+// (TensorQueue); 4 are slower. With the SM to itself (SECEDO_B200_ASYNC_GEMM=0) 6 stages (193 KB) would be
 // 2-3 % faster per launch (DESIGN.md 4, K3)
 constexpr int STAGES = 5;
 constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */;
@@ -853,66 +854,126 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 
 } // namespace
 
-// One launch of the tensor kernel, with everything it needs held by value: the launch may be issued later than the call that
-// prepared it (sgpu_ctx::tensor_jobs, late launch).
 namespace {
-struct TensorLaunch {
-    CUtensorMap map;
-    WorkList wl;
-    int32_t *S = nullptr, *D = nullptr;
-    uint32_t N = 0;
-    int epi = EPI_RMW;
-    unsigned grid = 0;                     // CTA pairs
-    sgpu_ctx::TensorJob job;               // events + what the job will own
-    cudaEvent_t staged = nullptr;          // on ctx->stream, behind the staging kernel (late launches only)
-};
 
-// t0, memset of the wave counter, kernel, t1 on stream gs; the job joins the context's list
-int issue_tensor_launch(sgpu_ctx *ctx, cudaStream_t gs, TensorLaunch &tl) {
-    ctx->tensor_jobs.push_back(tl.job); // the list owns the events and the panel from here on, whatever happens below
-    SGPU_CUDA(ctx, cudaMemsetAsync(tl.wl.wave_ctr, 0, sizeof(unsigned int), gs));
-    SGPU_CUDA(ctx, cudaEventRecord(tl.job.t0, gs));
-    SGPU_LAUNCH(ctx, (syrk2_kernel<<<2 * tl.grid, GEMM_THREADS, SMEM_BYTES, gs>>>(tl.map, tl.wl, tl.S, tl.D, tl.N, tl.epi)));
+// 32 k-blocks = 1 024 loci per chunk of the panel layout: 4 KB per cell, 33.8 MB per chunk at 8 192 cells
+constexpr uint32_t CK_SHIFT = 5;
+
+// an event from the context's pool (created when the pool is empty)
+cudaError_t take_event(sgpu_ctx *ctx, cudaEvent_t *e) {
+    std::vector<cudaEvent_t> &pool = ctx->tensor.event_pool;
+    if (!pool.empty()) {
+        *e = pool.back();
+        pool.pop_back();
+        return cudaSuccess;
+    }
+    return cudaEventCreateWithFlags(e, cudaEventDefault);
+}
+
+// The one launch site of the tensor kernel: memset of the wave counter, t0, kernel, t1 on stream gs. The job joins the list
+// first, so that a launch error leaves it there.
+int issue(sgpu_ctx *ctx, cudaStream_t gs, TensorJob &&job) {
+    const TensorJob &j = ctx->tensor.jobs.emplace_back(std::move(job));
+    const TensorArgs &a = j.args;
+    const WorkList wl{ a.tiles, a.n_full, a.n_work, a.splits, a.kbs_main + a.kbs_tail, a.per, CK_SHIFT, a.kbs_main, a.kbs_tail,
+                       a.wave_ctr };
+    SGPU_CUDA(ctx, cudaMemsetAsync(a.wave_ctr, 0, sizeof(unsigned int), gs));
+    SGPU_CUDA(ctx, cudaEventRecord(j.t0, gs));
+    SGPU_LAUNCH(ctx, (syrk2_kernel<<<2 * a.grid, GEMM_THREADS, SMEM_BYTES, gs>>>(a.map, wl, a.S, a.D, a.N, a.epi)));
     const cudaError_t le = cudaGetLastError();
-    SGPU_CUDA(ctx, cudaEventRecord(tl.job.t1, gs));
+    SGPU_CUDA(ctx, cudaEventRecord(j.t1, gs));
     SGPU_CUDA(ctx, le);
     return SGPU_OK;
 }
+
 } // namespace
 
-// The prepared launch of the last deferred tensor kernel, if it has not been issued yet. It is issued behind the NEXT batch's
-// link_window kernel (after_main = true: that kernel needs whole SMs and would otherwise wait for the tensor kernel to end,
-// with the stream's other kernels queued behind it; issued in this order the tensor kernel runs beside the special-entry
-// chain, the partition and the staging of the next batch instead), or by whoever needs the result or the stream first.
+// The held-back launch of the last deferred tensor kernel, if any. It is issued behind the NEXT batch's link_window kernel
+// (after_main = true: that kernel needs whole SMs and would otherwise wait for the tensor kernel to end, with the stream's
+// other kernels queued behind it; issued in this order the tensor kernel runs beside the special-entry chain, the partition
+// and the staging of the next batch instead), or by whoever needs the result or the stream first.
 int sgpu_tensor_flush(sgpu_ctx *ctx, bool after_main) {
-    TensorLaunch *tl = static_cast<TensorLaunch *>(ctx->pending_gemm);
-    if (!tl) {
+    TensorQueue &q = ctx->tensor;
+    if (!q.held) {
         return SGPU_OK;
     }
-    ctx->pending_gemm = nullptr;
-    struct Cleanup {
-        sgpu_ctx *ctx;
-        TensorLaunch *tl;
-        bool issued = false;
-        ~Cleanup() {
-            ctx->event_pool.push_back(tl->staged);
-            if (!issued) { // an error before the launch: the job never reached the list
-                ctx->event_pool.push_back(tl->job.t0);
-                ctx->event_pool.push_back(tl->job.t1);
-                sgpu_dev_free(ctx, tl->job.U);
-                sgpu_dev_free(ctx, tl->job.err);
-            }
-            delete tl;
-        }
-    } cleanup{ ctx, tl };
-    cudaStream_t gs = ctx->tensor_stream;
+    TensorJob job(std::move(*q.held));
+    q.held.reset();
     if (after_main) {
-        SGPU_CUDA(ctx, cudaEventRecord(tl->staged, ctx->stream)); // re-recorded: behind everything queued so far (incl. the staging)
+        SGPU_CUDA(ctx, cudaEventRecord(job.staged, ctx->stream)); // re-recorded: behind everything queued so far (incl. the staging)
     }
-    SGPU_CUDA(ctx, cudaStreamWaitEvent(gs, tl->staged, 0));
+    SGPU_CUDA(ctx, cudaStreamWaitEvent(q.stream, job.staged, 0));
+    q.event_pool.push_back(std::exchange(job.staged, nullptr)); // the wait is enqueued: the event may be recorded again
     SGPU_TRY(sgpu_cache_preference(ctx, true)); // what is launched from now on may run beside this kernel
-    cleanup.issued = true; // from here on the job is in the list (issue_tensor_launch appends it before it reports a launch error)
-    return issue_tensor_launch(ctx, gs, *tl);
+    return issue(ctx, q.stream, std::move(job));
+}
+
+TensorJob::TensorJob(TensorJob &&o) noexcept
+    : ctx(o.ctx), planes(o.planes), args(o.args), U(std::exchange(o.U, nullptr)), err(std::exchange(o.err, nullptr)),
+      t0(std::exchange(o.t0, nullptr)), t1(std::exchange(o.t1, nullptr)), staged(std::exchange(o.staged, nullptr)) {}
+
+TensorJob::~TensorJob() {
+    for (cudaEvent_t e : { t0, t1, staged }) {
+        if (e) {
+            ctx->tensor.event_pool.push_back(e);
+        }
+    }
+    sgpu_dev_free(ctx, U);
+    sgpu_dev_free(ctx, err);
+}
+
+// Jobs whose end event has been reached: kernel time into the queue's statistics, events back to the pool, operand panel
+// back to the cache (whoever gets it next is ordered behind this call on ctx->stream, and the kernel is done).
+int sgpu_tensor_poll(sgpu_ctx *ctx, bool wait_all) {
+    TensorQueue &q = ctx->tensor;
+    if (wait_all) {
+        SGPU_TRY(sgpu_tensor_flush(ctx, false));
+    }
+    while (!q.jobs.empty()) {
+        const TensorJob &j = q.jobs.front();
+        const cudaError_t r = wait_all ? cudaEventSynchronize(j.t1) : cudaEventQuery(j.t1);
+        if (r == cudaErrorNotReady) {
+            break; // jobs finish in order
+        }
+        if (r != cudaSuccess) {
+            return sgpu_fail(ctx, SGPU_E_CUDA, "tensor kernel failed: %s", cudaGetErrorString(r));
+        }
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, j.t0, j.t1) == cudaSuccess) {
+            q.ms += ms;
+            ++q.launches;
+        }
+        q.jobs.pop_front();
+    }
+    return SGPU_OK;
+}
+
+int sgpu_tensor_join(sgpu_ctx *ctx, const void *planes) {
+    TensorQueue &q = ctx->tensor;
+    if (q.held && (planes == nullptr || q.held->planes == planes)) {
+        SGPU_TRY(sgpu_tensor_flush(ctx, false));
+    }
+    for (auto it = q.jobs.rbegin(); it != q.jobs.rend(); ++it) {
+        if (planes == nullptr || it->planes == planes) { // jobs finish in order: the last one of these planes covers the earlier ones
+            SGPU_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, it->t1, 0));
+            break;
+        }
+    }
+    return sgpu_cache_preference(ctx, false); // what the caller launches next runs alone (or at most beside another object's kernel)
+}
+
+int sgpu_tensor_drain(sgpu_ctx *ctx) {
+    const int rc = sgpu_tensor_poll(ctx, true);
+    if (rc != SGPU_OK) { // a failed kernel: none of the jobs left over may still be running when they give their blocks back
+        cudaStreamSynchronize(ctx->tensor.stream);
+        ctx->tensor.jobs.clear();
+    }
+    return rc;
+}
+
+void sgpu_tensor_take_times(sgpu_ctx *ctx, float *ms, uint64_t *launches) {
+    *ms += std::exchange(ctx->tensor.ms, 0.f);
+    *launches += std::exchange(ctx->tensor.launches, uint64_t{ 0 });
 }
 
 // Upper-triangle 256 x 256 output tiles in an order that keeps the tiles in flight (one per CTA pair) inside a block
@@ -978,150 +1039,160 @@ int sgpu_gemm_counts(sgpu_ctx *ctx, const sgpu_pileup *p, const LinkResult &lr, 
     return sgpu_gemm_run(ctx, in, c->n, c->i32 + PLANE_S * c->nn, c->i32 + PLANE_D * c->nn, &c->fresh, &c->poisoned);
 }
 
-// The GEMM path on any CSR of (cell group, letter) entries: loci [0, n_main) are counted, the loci listed
-// in tail_loci are subtracted as Z Z^T. Used for the pileup itself and for the derived pileup of locus
-// pairs of the second-order correction (multilocus.cu).
-int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_plane, int32_t *D_plane, bool *fresh, bool *poisoned) {
-    cudaStream_t st = ctx->stream;
-    const uint64_t P = in.n_main;
-    if (P == 0 || in.n_entries == 0 || N < 2) {
-        return SGPU_OK;
-    }
-    if (N > ST_MAX_STRIPES * (ST_MAX_CELLS & ~3u) - 256) { // stripes of the staging tiles; cells are 16-bit in the partition's group map
-        return sgpu_fail(ctx, SGPU_E_ARG, "the GEMM path supports at most %u cells", ST_MAX_STRIPES * (ST_MAX_CELLS & ~3u) - 256);
-    }
-    const uint32_t n_pad = (N + BN - 1) / BN * BN;
-    // the tail k-blocks (Z and -Z) ride along with the first panel
-    const uint32_t kbs_tail = static_cast<uint32_t>((in.n_tail_loci + LOCI_PER_KB - 1) / LOCI_PER_KB);
-    // panel: at most 3 GB of Hadamard planes (98 304 loci at 8 192 padded cells: a bench sub-batch of ~65 700 significant
-    // loci used to spill a few hundred loci into a second panel, i.e. a second read-modify-write pass over the planes)
+namespace {
+
+// Loci per operand panel, a multiple of LOCI_PER_KB and no more than the P loci need: at most 3 GB of Hadamard planes
+// (98 304 loci at 8 192 padded cells: a bench sub-batch of ~65 700 significant loci used to spill a few hundred loci into a
+// second panel, i.e. a second read-modify-write pass over the planes). SECEDO_B200_PANEL_LOCI (tests) forces several panels
+// on small inputs.
+uint64_t panel_loci(uint32_t n_pad, uint64_t P) {
     uint64_t panel = (3ull << 30) / (4ull * n_pad) / LOCI_PER_KB * LOCI_PER_KB;
-    if (const char *env = getenv("SECEDO_B200_PANEL_LOCI")) { // tests: force several panels on small inputs
+    if (const char *env = getenv("SECEDO_B200_PANEL_LOCI")) {
         panel = std::max(1, atoi(env)) / LOCI_PER_KB * LOCI_PER_KB;
     }
     panel = std::max<uint64_t>(panel, LOCI_PER_KB);
-    panel = std::min<uint64_t>(panel, (P + LOCI_PER_KB - 1) / LOCI_PER_KB * LOCI_PER_KB);
-    const uint64_t kbs_max = panel / LOCI_PER_KB + 2ull * kbs_tail;
+    return std::min<uint64_t>(panel, (P + LOCI_PER_KB - 1) / LOCI_PER_KB * LOCI_PER_KB);
+}
+
+// The work items of a launch over n_tiles output tiles of a.kbs_main + a.kbs_tail k-blocks on sms SMs: whole tiles in
+// full rounds of the grid; the rest (or everything, when there are few tiles) in K ranges so that every SM has work in
+// the last round
+void split_work(uint32_t n_tiles, uint32_t sms, TensorArgs &w) {
+    const uint32_t units = sms / 2; // CTA pairs that take work items
+    const uint32_t kbs = w.kbs_main + w.kbs_tail;
+    w.n_full = n_tiles >= 2 * units ? n_tiles / units * units : 0;
+    const uint32_t rest = n_tiles - w.n_full;
+    uint32_t splits = 1;
+    if (rest) {
+        const uint32_t target = w.n_full ? units : 2 * units;
+        splits = static_cast<uint32_t>(std::min<uint64_t>(kbs, std::max<uint32_t>(1, target / rest)));
+    }
+    w.per = (kbs + splits - 1) / splits;
+    w.splits = (kbs + w.per - 1) / w.per; // no empty range
+    w.n_work = w.n_full + rest * w.splits;
+    w.grid = static_cast<unsigned>(std::min<uint64_t>(w.n_work, units));
+}
+
+// tensor map over the panel U: [chunk][cell][ck x 128 bytes], box = 128 cells x 128 bytes, 128B swizzle
+int encode_panel_map(sgpu_ctx *ctx, void *U, const PanelLayout &pl, uint32_t n_pad, uint64_t n_chunks, CUtensorMap *map) {
+    const cuuint64_t gdim[3] = { static_cast<cuuint64_t>(1u << pl.ck_shift) * KB_BYTES, n_pad, n_chunks };
+    const cuuint64_t gstride[2] = { static_cast<cuuint64_t>(pl.cell_words) * 4, pl.chunk_words * 4 };
+    const cuuint32_t box[3] = { KB_BYTES, 128, 1 };
+    const cuuint32_t estr[3] = { 1, 1, 1 };
+    // resolved through the runtime so that the library does not link libcuda.so (it must load, and
+    // fail loudly in sgpu_init, on a machine without a driver)
+    typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
+                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    void *fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    SGPU_CUDA(ctx, cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+    if (fn == nullptr || qres != cudaDriverEntryPointSuccess) {
+        return sgpu_fail(ctx, SGPU_E_CUDA, "driver does not provide cuTensorMapEncodeTiled");
+    }
+    CUresult r = reinterpret_cast<encode_fn>(fn)(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, U, gdim, gstride, box, estr,
+                                                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        return sgpu_fail(ctx, SGPU_E_CUDA, "cuTensorMapEncodeTiled failed (%d)", static_cast<int>(r));
+    }
+    return SGPU_OK;
+}
+
+// The range checks of the partition and staging kernels, read BEFORE the tensor kernel of the panel touches the count
+// planes: an input outside the int8 path (more than 127 reads of one cell at one locus) or with bad group ids leaves the
+// planes as they were (first panel; SGPU_PATH_AUTO then takes the scatter path) or holding the sum of the panels before it.
+int range_status(sgpu_ctx *ctx, int err, bool first, bool *poisoned) {
+    if (err == SGPU_E_CELL_RANGE) {
+        return sgpu_fail(ctx, err, "a group id is >= n_groups or maps to a cell >= num_cells (filter the pileup first)");
+    }
+    if (err == 0) {
+        return SGPU_OK;
+    }
+    if (first) {
+        return sgpu_fail(ctx, SGPU_E_COUNT_RANGE, "more than 127 reads of one cell at one locus: outside the int8 GEMM path, use the "
+                         "scatter path (count planes untouched)");
+    }
+    if (poisoned) {
+        *poisoned = true; // the panels before this one have been added: the planes hold a partial sum
+    }
+    return sgpu_fail(ctx, SGPU_E_COUNT_RANGE, "more than 127 reads of one cell at one locus: outside the int8 GEMM path, use the scatter "
+                     "path (the counts object holds a partial sum: sgpu_counts_zero before using it again)");
+}
+
+// The stages of sgpu_gemm_run, in the order they run, and what they share
+struct GemmRun {
+    sgpu_ctx *ctx;
+    cudaStream_t st;
+    const GemmInput &in;
+    uint32_t N, n_pad, sms;
+    // The tensor kernel goes to the context's tensor stream behind an event of its staging kernel and the launch of the last
+    // panel is held back (in.may_defer: the first-order counts of sgpu_counts_accumulate; callers that read the result
+    // right away keep the kernel on ctx->stream).
+    bool defer;
+    cudaStream_t gs;
     PanelLayout pl;
-    pl.ck_shift = 5; // 32 k-blocks = 1 024 loci per chunk: 4 KB per cell, 33.8 MB per chunk at 8 192 cells
-    const uint32_t ck = 1u << pl.ck_shift;
-    pl.cell_words = (ck | 1u) * 32u; // odd number of lines: consecutive cells do not alias in the L2 sets
-    pl.chunk_words = static_cast<uint64_t>(n_pad) * pl.cell_words;
-    const uint64_t n_chunks_max = (kbs_max + ck - 1) / ck;
-    SGPU_TRACE(ctx, "gemm: enter");
-
-    // tensor kernels of earlier batches: issue the one still pending, retire the finished ones; never more than two operand
-    // panels in flight
-    SGPU_TRY(sgpu_tensor_flush(ctx, false));
-    SGPU_TRY(sgpu_tensor_poll(ctx, false));
-    while (ctx->tensor_jobs.size() >= 2) {
-        SGPU_CUDA(ctx, cudaEventSynchronize(ctx->tensor_jobs.front().t1));
-        SGPU_TRY(sgpu_tensor_poll(ctx, false));
-    }
-    DevBuf<uint32_t> U;
-    DevBuf<int> d_err;
-    SGPU_CUDA(ctx, U.alloc(n_chunks_max * pl.chunk_words, ctx));
-    SGPU_CUDA(ctx, d_err.alloc(2, ctx));
-    SGPU_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, 2 * sizeof(int), st));
-    SGPU_TRACE(ctx, "gemm: alloc");
-
-    // tensor map over U: [chunk][cell][ck x 128 bytes], box = 128 cells x 128 bytes, 128B swizzle
+    uint32_t n_stripes, cells_per_cta; // stripes of cells per staging CTA: as few as the largest tile (ST_MAX_CELLS) allows
+    size_t st_smem;
     CUtensorMap map;
-    {
-        const cuuint64_t gdim[3] = { static_cast<cuuint64_t>(ck) * KB_BYTES, n_pad, n_chunks_max };
-        const cuuint64_t gstride[2] = { static_cast<cuuint64_t>(pl.cell_words) * 4, pl.chunk_words * 4 };
-        const cuuint32_t box[3] = { KB_BYTES, 128, 1 };
-        const cuuint32_t estr[3] = { 1, 1, 1 };
-        // resolved through the runtime so that the library does not link libcuda.so (it must load, and
-        // fail loudly in sgpu_init, on a machine without a driver)
-        typedef CUresult (*encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                      const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                      CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        SGPU_CUDA(ctx, cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (fn == nullptr || qres != cudaDriverEntryPointSuccess) {
-            return sgpu_fail(ctx, SGPU_E_CUDA, "driver does not provide cuTensorMapEncodeTiled");
-        }
-        CUresult r = reinterpret_cast<encode_fn>(fn)(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, U.p, gdim, gstride, box, estr,
-                                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            return sgpu_fail(ctx, SGPU_E_CUDA, "cuTensorMapEncodeTiled failed (%d)", static_cast<int>(r));
-        }
-    }
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    const uint2 *d_tiles = nullptr;
+    const uint2 *tiles = nullptr;
     uint32_t n_tiles = 0;
-    SGPU_TRY(tile_list(ctx, N, n_pad, &d_tiles, &n_tiles));
-    SGPU_TRACE(ctx, "gemm: tensor map + tiles");
+    TensorJob job;                          // the last panel's: owns the operand panel and the error words from the start
+    cudaStream_t readers = nullptr;         // an earlier panel's tensor kernel has been launched here
+    cudaEvent_t s0 = nullptr, s1 = nullptr; // staging time, on ctx->stream
+    DevBuf<uint16_t> cellbase;              // per-entry (cell, base), partitioned by stripe inside every locus
+    DevBuf<uint32_t> seg;
 
-    // The tensor kernel goes to the context's tensor stream behind an event of its staging kernel and the call returns
-    // without waiting for it (in.may_defer: the first-order counts of sgpu_counts_accumulate; callers that read the
-    // result right away keep the kernel on ctx->stream). The panel and the error / wave-counter words belong to the job of
-    // the LAST panel; an error return before that job exists waits for the kernels already launched.
-    const bool defer = in.may_defer && ctx->async_gemm && ctx->tensor_stream != nullptr;
-    cudaStream_t gs = defer ? ctx->tensor_stream : st;
-    struct PanelOwner {
-        sgpu_ctx *ctx;
-        cudaStream_t gs;
-        void *U;
-        int *err;
-        bool launched = false;
-        ~PanelOwner() {
-            if (U || err) {
-                if (launched) {
-                    cudaStreamSynchronize(gs);
-                }
-                sgpu_dev_free(ctx, U);
-                sgpu_dev_free(ctx, err);
+    GemmRun(sgpu_ctx *c, const GemmInput &in_, uint32_t N_)
+        : ctx(c), st(c->stream), in(in_), N(N_), n_pad((N_ + BN - 1) / BN * BN), sms(static_cast<uint32_t>(c->sm_count)),
+          defer(in_.may_defer && c->tensor.async && c->tensor.stream != nullptr), gs(defer ? c->tensor.stream : c->stream),
+          n_stripes(std::min<uint32_t>(ST_MAX_STRIPES, (n_pad + ST_MAX_CELLS - 1) / ST_MAX_CELLS)),
+          cells_per_cta(((n_pad + n_stripes - 1) / n_stripes + 3) / 4 * 4), st_smem(static_cast<size_t>(cells_per_cta) * 128),
+          job(c) {
+        pl.ck_shift = CK_SHIFT;
+        pl.cell_words = ((1u << CK_SHIFT) | 1u) * 32u; // odd number of lines: consecutive cells do not alias in the L2 sets
+        pl.chunk_words = static_cast<uint64_t>(n_pad) * pl.cell_words;
+    }
+    ~GemmRun() {
+        if (job.U && readers) { // an error return after an earlier panel's launch: that kernel may still read the panel
+            cudaStreamSynchronize(readers);
+        }
+        for (cudaEvent_t e : { s0, s1 }) {
+            if (e) {
+                ctx->tensor.event_pool.push_back(e);
             }
         }
-    } owner{ ctx, gs, U.take(), d_err.take() };
-    uint32_t *const Up = static_cast<uint32_t *>(owner.U);
-    int *const errp = owner.err;
-    auto get_event = [&](cudaEvent_t *e) -> cudaError_t {
-        if (!ctx->event_pool.empty()) {
-            *e = ctx->event_pool.back();
-            ctx->event_pool.pop_back();
-            return cudaSuccess;
-        }
-        return cudaEventCreateWithFlags(e, cudaEventDefault);
-    };
-    // staging time: events on ctx->stream, read after the synchronisation that follows every staging kernel
-    cudaEvent_t ev_s0 = nullptr, ev_s1 = nullptr;
-    SGPU_CUDA(ctx, get_event(&ev_s0));
-    SGPU_CUDA(ctx, get_event(&ev_s1));
-    struct EventReturn {
-        sgpu_ctx *ctx;
-        cudaEvent_t *a, *b;
-        ~EventReturn() {
-            ctx->event_pool.push_back(*a);
-            ctx->event_pool.push_back(*b);
-        }
-    } event_return{ ctx, &ev_s0, &ev_s1 };
-    const uint32_t sms = static_cast<uint32_t>(ctx->sm_count);
-    // stripes of cells per staging CTA: as few as the largest tile (ST_MAX_CELLS) allows
-    const uint32_t n_stripes = std::min<uint32_t>(ST_MAX_STRIPES, (n_pad + ST_MAX_CELLS - 1) / ST_MAX_CELLS);
-    const uint32_t cells_per_cta = ((n_pad + n_stripes - 1) / n_stripes + 3) / 4 * 4;
-    const size_t st_smem = static_cast<size_t>(cells_per_cta) * 128;
-    SGPU_CUDA(ctx, cudaFuncSetAttribute(stage_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(st_smem)));
+    }
 
-    // per-entry (cell, base) with the group map and the special bitmap applied, partitioned by stripe
-    // inside every locus, once per call
-    DevBuf<uint16_t> cellbase;
-    DevBuf<uint32_t> seg;
-    const uint64_t E = in.n_entries;
-    SGPU_CUDA(ctx, cellbase.alloc(E + 8, ctx));
-    SGPU_CUDA(ctx, seg.alloc(in.n_loci * (n_stripes + 1), ctx));
-    SGPU_CUDA(ctx, cudaEventRecord(ev_s0, st)); // the partition is folded into the first panel's staging time
-    {
+    // operand panel for kbs_max k-blocks, error words, tensor map, tile list, staging events and buffers
+    int prepare(uint64_t kbs_max) {
+        const uint64_t n_chunks = (kbs_max + (1u << CK_SHIFT) - 1) >> CK_SHIFT;
+        SGPU_CUDA(ctx, sgpu_dev_alloc(ctx, &job.U, n_chunks * pl.chunk_words * sizeof(uint32_t)));
+        SGPU_CUDA(ctx, sgpu_dev_alloc(ctx, reinterpret_cast<void **>(&job.err), 2 * sizeof(int)));
+        SGPU_CUDA(ctx, cudaMemsetAsync(job.err, 0, 2 * sizeof(int), st));
+        SGPU_TRACE(ctx, "gemm: alloc");
+        SGPU_TRY(encode_panel_map(ctx, job.U, pl, n_pad, n_chunks, &map));
+        SGPU_CUDA(ctx, cudaFuncSetAttribute(syrk2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        SGPU_TRY(tile_list(ctx, N, n_pad, &tiles, &n_tiles));
+        SGPU_TRACE(ctx, "gemm: tensor map + tiles");
+        SGPU_CUDA(ctx, take_event(ctx, &s0));
+        SGPU_CUDA(ctx, take_event(ctx, &s1));
+        SGPU_CUDA(ctx, cudaFuncSetAttribute(stage_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(st_smem)));
+        SGPU_CUDA(ctx, cellbase.alloc(in.n_entries + 8, ctx));
+        SGPU_CUDA(ctx, seg.alloc(in.n_loci * (n_stripes + 1), ctx));
+        return SGPU_OK;
+    }
+
+    // per-entry (cell, base) with the group map and the special bitmap applied, partitioned by stripe inside every locus,
+    // once per call
+    int partition() {
+        SGPU_CUDA(ctx, cudaEventRecord(s0, st)); // the partition is folded into the first panel's staging time
         const unsigned grid = static_cast<unsigned>(std::min<uint64_t>(in.n_loci, static_cast<uint64_t>(sms) * 16));
         const size_t psmem = (static_cast<size_t>(PART_OUT) + (in.gmap_identity ? 0 : in.n_groups)) * sizeof(uint16_t);
         if (psmem > 200 * 1024) {
             return sgpu_fail(ctx, SGPU_E_ARG, "too many groups (%u) for the shared-memory group map of the GEMM path", in.n_groups);
         }
-        auto run_partition = [&](auto *gid_base) -> int {
+        auto run = [&](auto *gid_base) -> int {
             using GB = std::remove_const_t<std::remove_pointer_t<decltype(gid_base)>>;
             PartitionArgs<GB> pa;
             pa.row_ptr = in.row_ptr;
@@ -1137,23 +1208,19 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
             pa.cells_per_cta = cells_per_cta;
             pa.cellbase = cellbase.p;
             pa.seg = seg.p;
-            pa.err = errp;
+            pa.err = job.err;
             SGPU_CUDA(ctx, cudaFuncSetAttribute(partition_kernel<GB>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(psmem)));
             SGPU_LAUNCH(ctx, (partition_kernel<GB><<<grid, 256, psmem, st>>>(pa)));
             return SGPU_OK;
         };
-        SGPU_TRY(in.gid_base32 ? run_partition(in.gid_base32) : run_partition(in.gid_base));
+        return in.gid_base32 ? run(in.gid_base32) : run(in.gid_base);
     }
 
-    bool first = true;
-    for (uint64_t l0 = 0; l0 < P; l0 += panel) {
-        const uint64_t l1 = std::min<uint64_t>(P, l0 + panel);
-        const uint64_t nl = l1 - l0;
-        const bool last = l1 == P;
-        const uint32_t kbs_main = static_cast<uint32_t>((nl + LOCI_PER_KB - 1) / LOCI_PER_KB);
-        const uint32_t kt = first ? kbs_tail : 0;
-        if (!first) {
-            SGPU_CUDA(ctx, cudaEventRecord(ev_s0, st));
+    // the loci [l0, l0 + nl) (and, with the first panel, the kt tail k-blocks) into the panel; *err: the range checks so
+    // far, read back while the tensor stream is busy with the previous batch
+    int stage(uint64_t l0, uint64_t nl, uint32_t kbs_main, uint32_t kt, int *err) {
+        if (l0 != 0) {
+            SGPU_CUDA(ctx, cudaEventRecord(s0, st));
         }
         StageArgs sa;
         sa.row_ptr = in.row_ptr;
@@ -1173,155 +1240,99 @@ int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_pla
         sa.cells_per_cta = cells_per_cta;
         sa.n_stripes = n_stripes;
         sa.pl = pl;
-        sa.U = Up;
-        sa.err = errp;
+        sa.U = static_cast<uint32_t *>(job.U);
+        sa.err = job.err;
         SGPU_LAUNCH(ctx, (stage_tile_kernel<<<(kbs_main + kt) * n_stripes, ST_THREADS, st_smem, st>>>(sa)));
         SGPU_CUDA(ctx, cudaGetLastError());
-        SGPU_CUDA(ctx, cudaEventRecord(ev_s1, st));
+        SGPU_CUDA(ctx, cudaEventRecord(s1, st));
         SGPU_TRACE(ctx, "gemm: stage");
-        // The range checks of the partition and staging kernels are looked at BEFORE the tensor kernel touches the count
-        // planes: an input outside the int8 path (more than 127 reads of one cell at one locus) or with bad group ids
-        // leaves the planes as they were (first panel; SGPU_PATH_AUTO then takes the scatter path) or holding the sum of
-        // the panels before it. The tensor stream is busy with the previous batch meanwhile.
-        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[2], errp, sizeof(int), cudaMemcpyDeviceToHost, st));
+        SGPU_CUDA(ctx, cudaMemcpyAsync(&ctx->h_scratch[2], job.err, sizeof(int), cudaMemcpyDeviceToHost, st));
         SGPU_CUDA(ctx, cudaStreamSynchronize(st));
-        {
-            float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, ev_s0, ev_s1) == cudaSuccess) {
-                ctx->ms_stage += ms;
-            }
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, s0, s1) == cudaSuccess) {
+            ctx->tensor.ms_stage += ms;
         }
-        const int err = static_cast<int>(ctx->h_scratch[2] & 0xFFFFFFFFu);
-        if (err == SGPU_E_CELL_RANGE) {
-            return sgpu_fail(ctx, err, "a group id is >= n_groups or maps to a cell >= num_cells (filter the pileup first)");
-        }
-        if (err != 0) {
-            if (first) {
-                return sgpu_fail(ctx, SGPU_E_COUNT_RANGE, "more than 127 reads of one cell at one locus: outside the int8 GEMM path, use the "
-                                 "scatter path (count planes untouched)");
-            }
-            if (poisoned) {
-                *poisoned = true; // the panels before this one have been added: the planes hold a partial sum
-            }
-            return sgpu_fail(ctx, SGPU_E_COUNT_RANGE, "more than 127 reads of one cell at one locus: outside the int8 GEMM path, use the scatter "
-                             "path (the counts object holds a partial sum: sgpu_counts_zero before using it again)");
-        }
+        *err = static_cast<int>(ctx->h_scratch[2] & 0xFFFFFFFFu);
+        return SGPU_OK;
+    }
 
-        WorkList wl;
-        wl.tiles = d_tiles;
-        wl.kbs = kbs_main + kt;
-        wl.ck_shift = pl.ck_shift;
-        wl.kb_neg0 = kbs_main;
-        wl.kb_negd = kt;
-        wl.wave_ctr = reinterpret_cast<unsigned int *>(errp + 1);
-        // whole tiles in full rounds of the grid; the rest (or everything, when there are few tiles) in
-        // K ranges so that every SM has work in the last round
-        const uint32_t units = sms / 2; // CTA pairs that take work items
-        wl.n_full = n_tiles >= 2 * units ? n_tiles / units * units : 0;
-        const uint32_t rest = n_tiles - wl.n_full;
-        uint32_t splits = 1;
-        if (rest) {
-            const uint32_t target = wl.n_full ? units : 2 * units;
-            splits = static_cast<uint32_t>(std::min<uint64_t>(wl.kbs, std::max<uint32_t>(1, target / rest)));
-        }
-        wl.per = (wl.kbs + splits - 1) / splits;
-        wl.splits = (wl.kbs + wl.per - 1) / wl.per; // no empty range
-        wl.n_work = wl.n_full + rest * wl.splits;
+    // the tensor kernel of the panel just staged: issued, or, for the last panel of a deferred call, held back for
+    // sgpu_tensor_flush (behind the next batch's link_window kernel, or at the first join)
+    int launch_or_hold(uint32_t kbs_main, uint32_t kt, bool last, int32_t *S, int32_t *D, bool *fresh) {
+        TensorJob earlier(ctx); // an earlier panel's job owns no blocks
+        TensorJob &j = last ? job : earlier;
+        j.planes = S;
         // the planes are zero right after sgpu_counts_zero: the first panel stores, later ones add in place
-        const int epi = *fresh ? EPI_STORE : EPI_RMW;
-        const unsigned grid = static_cast<unsigned>(std::min<uint64_t>(wl.n_work, units));
-        TensorLaunch tl;
-        tl.map = map;
-        tl.wl = wl;
-        tl.S = S_plane;
-        tl.D = D_plane;
-        tl.N = N;
-        tl.epi = epi;
-        tl.grid = grid;
-        tl.job.planes = S_plane;
-        SGPU_CUDA(ctx, get_event(&tl.job.t0));
-        SGPU_CUDA(ctx, get_event(&tl.job.t1));
+        j.args = TensorArgs{ map, tiles, kbs_main, kt, 0, 0, 0, 0, 0, reinterpret_cast<unsigned int *>(job.err + 1), S, D, N,
+                             *fresh ? EPI_STORE : EPI_RMW };
+        split_work(n_tiles, sms, j.args);
+        SGPU_CUDA(ctx, take_event(ctx, &j.t0));
+        SGPU_CUDA(ctx, take_event(ctx, &j.t1));
         *fresh = false;
         if (last && defer) {
-            // prepared, not issued: sgpu_tensor_flush (behind the next batch's link_window kernel, or at the first join)
-            TensorLaunch *pending = new TensorLaunch(tl);
-            if (get_event(&pending->staged) != cudaSuccess || cudaEventRecord(pending->staged, st) != cudaSuccess) {
-                delete pending;
+            if (take_event(ctx, &j.staged) != cudaSuccess || cudaEventRecord(j.staged, st) != cudaSuccess) {
                 return sgpu_fail(ctx, SGPU_E_CUDA, "event for the deferred tensor kernel");
             }
-            pending->job.U = owner.U;
-            pending->job.err = owner.err;
-            owner.U = nullptr;
-            owner.err = nullptr;
-            ctx->pending_gemm = pending;
-        } else {
-            if (defer) {
-                SGPU_CUDA(ctx, cudaStreamWaitEvent(gs, ev_s1, 0)); // staged (and everything before it on ctx->stream: the zeroed planes)
-                SGPU_TRY(sgpu_cache_preference(ctx, true));        // what is launched from now on may run beside this kernel
-            }
-            if (last) { // the job of the last panel owns the panel
-                tl.job.U = owner.U;
-                tl.job.err = owner.err;
-            }
-            owner.launched = true;
-            if (last) { // the job list owns them now (also if the launch fails: the job is in the list by then)
-                owner.U = nullptr;
-                owner.err = nullptr;
-            }
-            SGPU_TRY(issue_tensor_launch(ctx, gs, tl));
-            if (!last && defer) {
-                SGPU_CUDA(ctx, cudaStreamWaitEvent(st, ctx->tensor_jobs.back().t1, 0)); // the next panel is staged into the same buffer
-            }
+            ctx->tensor.held.emplace(std::move(j));
+            return SGPU_OK;
         }
-        first = false;
+        if (defer) {
+            SGPU_CUDA(ctx, cudaStreamWaitEvent(gs, s1, 0)); // staged (and everything before it on ctx->stream: the zeroed planes)
+            SGPU_TRY(sgpu_cache_preference(ctx, true));     // what is launched from now on may run beside this kernel
+        }
+        if (!last) {
+            readers = gs; // before the launch: a launch error may still leave the kernel queued
+        }
+        SGPU_TRY(issue(ctx, gs, std::move(j)));
+        if (!last && defer) {
+            SGPU_CUDA(ctx, cudaStreamWaitEvent(st, ctx->tensor.jobs.back().t1, 0)); // the next panel is staged into the same buffer
+        }
+        return SGPU_OK;
+    }
+};
+
+} // namespace
+
+// The GEMM path on any CSR of (cell group, letter) entries: loci [0, n_main) are counted, the loci listed
+// in tail_loci are subtracted as Z Z^T. Used for the pileup itself and for the derived pileup of locus
+// pairs of the second-order correction (multilocus.cu).
+int sgpu_gemm_run(sgpu_ctx *ctx, const GemmInput &in, uint32_t N, int32_t *S_plane, int32_t *D_plane, bool *fresh, bool *poisoned) {
+    const uint64_t P = in.n_main;
+    if (P == 0 || in.n_entries == 0 || N < 2) {
+        return SGPU_OK;
+    }
+    if (N > ST_MAX_STRIPES * (ST_MAX_CELLS & ~3u) - 256) { // stripes of the staging tiles; cells are 16-bit in the partition's group map
+        return sgpu_fail(ctx, SGPU_E_ARG, "the GEMM path supports at most %u cells", ST_MAX_STRIPES * (ST_MAX_CELLS & ~3u) - 256);
+    }
+    GemmRun r(ctx, in, N);
+    const uint64_t panel = panel_loci(r.n_pad, P);
+    // the tail k-blocks (Z and -Z) ride along with the first panel
+    const uint32_t kbs_tail = static_cast<uint32_t>((in.n_tail_loci + LOCI_PER_KB - 1) / LOCI_PER_KB);
+    SGPU_TRACE(ctx, "gemm: enter");
+
+    // tensor kernels of earlier batches: issue the one still held back, retire the finished ones; never more than two
+    // operand panels in flight
+    SGPU_TRY(sgpu_tensor_flush(ctx, false));
+    SGPU_TRY(sgpu_tensor_poll(ctx, false));
+    while (ctx->tensor.jobs.size() >= 2) {
+        SGPU_CUDA(ctx, cudaEventSynchronize(ctx->tensor.jobs.front().t1));
+        SGPU_TRY(sgpu_tensor_poll(ctx, false));
+    }
+    SGPU_TRY(r.prepare(panel / LOCI_PER_KB + 2ull * kbs_tail));
+    SGPU_TRY(r.partition());
+    for (uint64_t l0 = 0; l0 < P; l0 += panel) {
+        const uint64_t nl = std::min<uint64_t>(P - l0, panel);
+        const uint32_t kbs_main = static_cast<uint32_t>((nl + LOCI_PER_KB - 1) / LOCI_PER_KB);
+        const uint32_t kt = l0 == 0 ? kbs_tail : 0;
+        int err = 0;
+        SGPU_TRY(r.stage(l0, nl, kbs_main, kt, &err));
+        SGPU_TRY(range_status(ctx, err, l0 == 0, poisoned));
+        SGPU_TRY(r.launch_or_hold(kbs_main, kt, l0 + nl == P, S_plane, D_plane, fresh));
         SGPU_TRACE(ctx, "gemm: syrk");
     }
-    if (!defer) { // the caller goes on with the result on ctx->stream: nothing stays in flight
-        SGPU_CUDA(ctx, cudaStreamSynchronize(st));
+    if (!r.defer) { // the caller goes on with the result on ctx->stream: nothing stays in flight
+        SGPU_CUDA(ctx, cudaStreamSynchronize(r.st));
         SGPU_TRY(sgpu_tensor_poll(ctx, true));
     }
     return SGPU_OK;
-}
-
-// Jobs whose end event has been reached: kernel time into the context's statistics, events back to the pool, operand
-// panel back to the cache (whoever gets it next is ordered behind this call on ctx->stream, and the kernel is done).
-int sgpu_tensor_poll(sgpu_ctx *ctx, bool wait_all) {
-    if (wait_all) {
-        SGPU_TRY(sgpu_tensor_flush(ctx, false));
-    }
-    while (!ctx->tensor_jobs.empty()) {
-        sgpu_ctx::TensorJob &j = ctx->tensor_jobs.front();
-        cudaError_t q = wait_all ? cudaEventSynchronize(j.t1) : cudaEventQuery(j.t1);
-        if (q == cudaErrorNotReady) {
-            break; // jobs finish in order
-        }
-        if (q != cudaSuccess) {
-            return sgpu_fail(ctx, SGPU_E_CUDA, "tensor kernel failed: %s", cudaGetErrorString(q));
-        }
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, j.t0, j.t1) == cudaSuccess) {
-            ctx->ms_syrk += ms;
-            ++ctx->n_syrk;
-        }
-        ctx->event_pool.push_back(j.t0);
-        ctx->event_pool.push_back(j.t1);
-        sgpu_dev_free(ctx, j.U);
-        sgpu_dev_free(ctx, j.err);
-        ctx->tensor_jobs.pop_front();
-    }
-    return SGPU_OK;
-}
-
-int sgpu_tensor_join(sgpu_ctx *ctx, const void *planes) {
-    const TensorLaunch *pending = static_cast<const TensorLaunch *>(ctx->pending_gemm);
-    if (pending && (planes == nullptr || pending->job.planes == planes)) {
-        SGPU_TRY(sgpu_tensor_flush(ctx, false));
-    }
-    for (auto it = ctx->tensor_jobs.rbegin(); it != ctx->tensor_jobs.rend(); ++it) {
-        if (planes == nullptr || it->planes == planes) { // jobs finish in order: the last one of these planes covers the earlier ones
-            SGPU_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, it->t1, 0));
-            break;
-        }
-    }
-    return sgpu_cache_preference(ctx, false); // what the caller launches next runs alone (or at most beside another object's kernel)
 }
